@@ -54,6 +54,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip per_config / dropin_e2e (N = 1 extras)")
     ap.add_argument("--no-parity", action="store_true", help="skip the untimed per-rank parity check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of the last step's baseband "
+                                                          "(what the caller of the timed path receives) as DIR/*.npy")
     ap.add_argument("--deadline", type=int, default=-1, help="seconds after which a run without a result reports where it stopped and exits "
                                                              "(default: 420 for N > 1, 1500 for N = 1; 0 = never)")
     return ap.parse_args()
@@ -234,6 +236,23 @@ def run_reference_arm(args):
 
 
 # --------------------------------------------------------------------------------------------------
+DUMP_SAMPLES = 1 << 21      # 16 MB of float32 I/Q + 16 MB of float64 indices
+
+
+def dump_outputs(path, out):
+    """Write the timed path's output `out` (complex64 [channels, samples per channel]) for output-by-output comparison
+    of two builds: baseband.npy = float32 [n, 2] (I, Q) at the flat indices in baseband_index.npy (float64), a sample
+    drawn with a fixed seed (the whole array when it is small enough)."""
+    flat = out.reshape(-1)
+    if flat.size <= DUMP_SAMPLES:
+        idx = np.arange(flat.size)
+    else:
+        idx = np.sort(np.random.default_rng(20261020).choice(flat.size, DUMP_SAMPLES, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "baseband.npy"), flat[idx].view(np.float32).reshape(-1, 2))
+    np.save(os.path.join(path, "baseband_index.npy"), idx.astype(np.float64))
+
+
 def mer_db(got, want):
     err = np.sum(np.abs(got.astype(np.complex128) - want) ** 2)
     sig = np.sum(np.abs(want.astype(np.complex128)) ** 2)
@@ -712,6 +731,17 @@ def run_ours(args):
     launches = T.kernel_launches() - launches0
     clk = clocks.stop()
     chain.enable_timing(False)
+    # after the clock sampler stops: the copy and the files belong to no timed step
+    if args.dump_outputs and rank == 0:
+        stage("dump outputs")
+        if G is None:
+            last = d_out[:nch].cpu().numpy()
+        else:                            # the ordered reassembly of every rank's channels in the root's last slot
+            torch.cuda.synchronize()
+            last = np.empty((args.channels, nfr * S), np.complex64)
+            T.copy_to_host(last, G.wait(step_no[0] - 1, cp))
+            torch.cuda.synchronize()
+        dump_outputs(args.dump_outputs, last)
     total_samples = args.channels * nfr * S
     value = total_samples / (ms_per_step * 1e-3) / 1e6
 

@@ -1,5 +1,6 @@
 """GPU parity tests: the CUDA path, called through the C ABI (ctypes), against the compiled unmodified
-reference (oracle/_ref) and the committed golden fixtures, on identical synthetic TS input.
+reference (oracle/_ref; where it is not built, the numpy oracle behind the same API -- see the reflib fixture) and
+the committed golden fixtures, on identical synthetic TS input.
 
 Bars (BASELINE.json north_star): BBFRAME/FECFRAME bits bit-exact; cells bit-exact (the LUT reproduces the
 reference's float arithmetic, so better than the 1-ulp bar); frame-mapper output bit-exact; time-domain

@@ -146,7 +146,7 @@ def test_chain_generic_work_streams():
     assert np.array_equal(np.concatenate(got).view(np.uint32), want.view(np.uint32))
 
 
-def test_overfull_frame_warn_policy(reflib):
+def test_overfull_frame_warn_policy(compiled_ref):
     """An over-full T2 frame: refused by default, reproduced like the reference (warn, truncate) with the opt-in policy."""
     cfg = K.resolve(dict(K.CONFIGS["c1"], fecblocks=9))
     T.set_overfull_policy(False)
@@ -156,7 +156,7 @@ def test_overfull_frame_warn_policy(reflib):
     try:
         fm = T.framemapperfint_cc(*fm_args(cfg))
         assert fm.warnings == 1
-        rf = reflib.framemapper(*fm_args(cfg))
+        rf = compiled_ref.framemapper(*fm_args(cfg))
         assert rf.warnings == 1
         assert fm.output_multiple == rf.output_multiple
         # (the reference's forecast() asks for 0 items here: its divisor is the grown private frame length; the
@@ -175,7 +175,7 @@ def test_overfull_frame_warn_policy(reflib):
         assert ch.warnings == 1
         ts = K.make_ts(ch.ts_bytes(0, 2) + 512, seed=3)
         out = ch.run_host(ts[:ch.ts_bytes(0, 2)], 1, 2)[0]
-        rc = reflib.Chain(cfg)
+        rc = compiled_ref.Chain(cfg)
         S = ch.samples_per_frame
         for fr in range(2):
             want = rc.run_frame(ts)["samples"]

@@ -26,10 +26,11 @@ def test_oracle_chain_equals_reference(reflib, name):
 
 @pytest.mark.parametrize("name", ["c1", "c2", "c3", "c4"])
 def test_oracle_matches_golden(name):
-    """Golden fixtures were produced by the reference itself (tools/make_golden.py); one T2 frame here."""
+    """Golden fixtures were produced by the reference itself (tools/make_golden.py): both stored T2 frames (the second
+    one checks the state carried across frames)."""
     g = load_golden("chain_%s.json" % name)
     cfg = K.resolve(name)
-    nfr = 2 if name == "c1" else 1
+    nfr = 2
     n = g["frames"][0]["ts_used"]
     ts = K.make_ts(2 * n + 1000)
     assert sha(ts[:4096]) == g["ts_head_sha256"]
