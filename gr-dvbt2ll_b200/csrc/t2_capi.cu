@@ -659,10 +659,9 @@ struct FrameHandle : dvbt2ll_handle {
 
 // ================================================================================================
 struct OfdmDevice {
-  DevBuf d_code, d_pool, d_p1, d_sinc, d_tw, d_tw_split, d_scratch, d_sym_flags;
+  DevBuf d_code, d_pool, d_p1, d_sinc, d_tw, d_tw_split, d_sym_flags;
   int log2_m, split;
   long long pool_stride;
-  long long scratch_slot_elems;     // float2 elements per scratch slot (one slot per concurrently running batch)
   // c16: `code` holds staging slots (chain mode, 16-bit cells) and is re-encoded for the kernel's branch-free fill:
   //   data carrier         -> 2 * slot            (byte offset into the staging area, < 131072)
   //   small pool cell p<8  -> (p + 1) << 17       (zero / pilot amplitudes, kept in shared memory)
@@ -684,13 +683,7 @@ struct OfdmDevice {
     }
     CK(upload(d_p1, op.p1));
     const int N = op.dims.fft_n;
-    split = N > 16384 ? 2 : 1;
-    {
-      // experiment: 16K symbols as two 8K halves recombined through L2 (like 32K), which fits two CTAs per SM
-      const char *e = std::getenv("DVBT2LL_OFDM_SPLIT16K");
-      if (c16 && N == 16384 && e && e[0] == '1') split = 2;
-    }
-    scratch_slot_elems = 0;
+    split = N > 16384 ? 2 : 1;      // 32K: two 16K halves (even / odd bins), recombined in the kernel
     const int M = N / split;
     log2_m = 0;
     while ((1 << log2_m) < M) log2_m++;
@@ -727,16 +720,7 @@ struct OfdmDevice {
       CK(upload(d_sinc, sinc_pos));
     }
     CK(upload(d_tw, make_twiddles(M, M)));
-    if (split == 2) {
-      CK(upload(d_tw_split, make_twiddles(N, M)));
-      int dev = 0, sms = 148;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      // parking space of the int16-sink 32K path: one M-point region per resident CTA, two slots so that two batches
-      // can be in flight on two streams (dvbt2ll_chain_run_host)
-      scratch_slot_elems = (long long)(4 * sms + 8) * M;      // up to 4 resident CTAs per SM below 16K sub-transforms
-      CK(d_scratch.ensure((size_t)2 * scratch_slot_elems * sizeof(float2)));
-    }
+    if (split == 2) CK(upload(d_tw_split, make_twiddles(N, M)));
     return 0;
   }
   void fill(t2k::OfdmArgs &a, const t2::OfdmPlan &op, const t2::CellPool &pool) const
@@ -750,7 +734,7 @@ struct OfdmDevice {
     a.norm = op.normalization;
     a.cells16 = 0; a.run_desc = 0; a.run_ptr = 0; a.run_cnt = 0; a.desc_cap = 0; a.stage_bytes = 0; a.stage_cap = 0; a.lut = 0; a.lut_n = 0; a.lut_single = 0;
     a.sym_flags = d_sym_flags.as<int32_t>();
-    a.out_fmt = 0; a.sink_gain = 1.0f; a.scratch = d_scratch.as<float2>();
+    a.out_fmt = 0; a.sink_gain = 1.0f;
     a.cells_len = 0; a.out_len = 0; a.pool_len = pool_stride;
   }
 };
@@ -912,10 +896,10 @@ struct ChainHandle : dvbt2ll_handle {
     for (int s = 0; s < TIMING_SLOTS; s++) for (int i = 0; i < 5; i++) CK(cudaEventCreate(&ev[s][i]));
     return 0;
   }
-  // buf_frame: first T2-frame slot of the intermediate buffers to use, scratch_slot: which half of the 32K parking
-  // scratch (two batches may be in flight on two streams); hist_valid < 0: history is present iff first_frame > 0
+  // buf_frame: first T2-frame slot of the intermediate buffers to use; hist_valid < 0: history is present iff
+  // first_frame > 0
   int run(const void *d_ts, long long ts_pitch, int n_channels, int n_frames, long long first_frame, void *d_out, cudaStream_t s,
-          int buf_frame = 0, int scratch_slot = 0, int hist_valid = -1)
+          int buf_frame = 0, int hist_valid = -1)
   {
     const int frames = n_channels * n_frames;
     if (frames < 1) return 0;
@@ -976,7 +960,6 @@ struct ChainHandle : dvbt2ll_handle {
     oa.out = d_out; oa.out_stride = oplan.samples_per_frame;
     oa.cells_len = (long long)frames * cells16_stride(); oa.out_len = (long long)frames * oplan.samples_per_frame;
     oa.out_fmt = sink_fmt; oa.sink_gain = sink_gain; oa.norm = oplan.normalization * sink_gain;
-    if (oa.scratch && scratch_slot) oa.scratch += odev.scratch_slot_elems;
     oa.frames = frames; oa.frames_per_channel = n_frames;
     oa.frame_idx0 = (int)(first_frame % (tables.pool.l1post_variants > 0 ? tables.pool.l1post_variants : 1));
     t2k::launch_ofdm(oa, s);
@@ -1215,7 +1198,7 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
   if (!resident) CK(h->copy_host(din, in, in_bytes, cudaMemcpyHostToDevice, s));
   int used = 0;
   if (ch) {
-    r = ch->run(din, 0, 1, frames, ch->next_frame, d_out.p, s, 0, 0, 1);
+    r = ch->run(din, 0, 1, frames, ch->next_frame, d_out.p, s, 0, 1);
     if (r >= 0) { r = nout; used = (int)need; ch->next_frame += frames; }
   }
   else r = h->work_device(din, (int)need, d_out.p, nout, &used, s);
@@ -1532,7 +1515,7 @@ int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch
     CK(cudaMemcpy2DAsync(base + (size_t)c0 * P * dpitch - hist, (size_t)dpitch, (const uint8_t *)ts + (size_t)c0 * P * ts_pitch - hist,
                          (size_t)ts_pitch, (size_t)(per_ch + hist), (size_t)nc * P, cudaMemcpyHostToDevice, s));
     r = c->run(base + (size_t)c0 * P * dpitch, dpitch, nc, n_frames, first_frame, dout + (size_t)c0 * ch_out * ssz, s,
-               groups == 1 ? 0 : (gi & 1) * per * n_frames, gi & 1);
+               groups == 1 ? 0 : (gi & 1) * per * n_frames);
     if (r < 0) return r;
     CK(cudaMemcpyAsync((uint8_t *)out + (size_t)c0 * ch_out * ssz, dout + (size_t)c0 * ch_out * ssz, (size_t)nc * ch_out * ssz,
                        cudaMemcpyDeviceToHost, s));

@@ -1954,6 +1954,45 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
   }
 }
 
+// ---- tensor memory (TMEM, sm_100): the 32K path keeps thread-private values there between its two phases.  Every
+// tcgen05 instruction is warp-collective (.sync.aligned): all 32 lanes must execute it together.
+constexpr int OFDM_PARK_COLS = 256;       // 512 threads x 64 words over the 128 lanes
+
+// one warp: allocate NCOLS columns (power of two >= 32); the column base is written to the shared word at dst_s
+template <int NCOLS>
+__device__ __forceinline__ void tmem_alloc(uint32_t dst_s)
+{
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(dst_s), "n"(NCOLS) : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish() { asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory"); }
+template <int NCOLS>
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr)
+{
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(taddr), "n"(NCOLS) : "memory");
+}
+__device__ __forceinline__ void tmem_fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory"); }
+__device__ __forceinline__ void tmem_fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory"); }
+// four complex values to 8 consecutive columns of the thread's lane
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const float2 (&v)[4])
+{
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};\n"
+               ::"r"(taddr), "f"(v[0].x), "f"(v[0].y), "f"(v[1].x), "f"(v[1].y), "f"(v[2].x), "f"(v[2].y), "f"(v[3].x), "f"(v[3].y));
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory"); }
+// the registers of tmem_ld4 hold the values only after tmem_wait_ld4 on them: the wait names them as operands, so
+// the compiler cannot move a use of them above it
+__device__ __forceinline__ void tmem_ld4(uint32_t taddr, float2 (&v)[4])
+{
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
+               : "=f"(v[0].x), "=f"(v[0].y), "=f"(v[1].x), "=f"(v[1].y), "=f"(v[2].x), "=f"(v[2].y), "=f"(v[3].x), "=f"(v[3].y)
+               : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_wait_ld4(float2 (&v)[4])
+{
+  asm volatile("tcgen05.wait::ld.sync.aligned;\n"
+               : "+f"(v[0].x), "+f"(v[0].y), "+f"(v[1].x), "+f"(v[1].y), "+f"(v[2].x), "+f"(v[2].y), "+f"(v[3].x), "+f"(v[3].y));
+}
+
 template <int LOG2M, int T, bool C16, int FMT, int SPLIT>
 __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const OfdmArgs a)
 {
@@ -1990,6 +2029,25 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
       if (!a.lut_single) lut_im[i] = v.y;
     }
     __syncthreads();
+  }
+  static_assert(SPLIT == 1 || LOG2M == 14, "only 32K symbols are transformed as two halves");
+  // 32K: the even-bin half E[n] of a symbol waits for the odd-bin phase in tensor memory (TMEM), 256 columns of this
+  // CTA's allocation; see park_col below.  Warp 0 allocates, the column base goes through the first word of x (not
+  // yet in use; the first fill is behind a barrier) to the other threads.
+  uint32_t park_col = 0;
+  if constexpr (SPLIT == 2) {
+    uint32_t *tm_slot = reinterpret_cast<uint32_t *>(x);
+    if (threadIdx.x < 32) {
+      tmem_alloc<OFDM_PARK_COLS>((uint32_t)__cvta_generic_to_shared(tm_slot));
+      tmem_relinquish();
+    }
+    tmem_fence_before_sync();
+    __syncthreads();
+    tmem_fence_after_sync();
+    // a warp reaches only the 32 TMEM lanes of its quadrant (warp mod 4); the four warps of a quadrant take 64
+    // columns each: thread-private slots of 8 butterflies x 4 complex values (lane = thread, one column per word)
+    const uint32_t warp = threadIdx.x >> 5;
+    park_col = *tm_slot + ((32u * (warp & 3u)) << 16) + 64u * (warp >> 2);
   }
   constexpr int R0 = FillGeom<LOG2M, T>::R0;       // first radix, done inside the fill (1 = no first pass)
   constexpr int NLAST = M / 16;              // NPREV of the last radix-16 pass
@@ -2101,9 +2159,6 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
     sample_t *out = reinterpret_cast<sample_t *>(a.out) + (long long)f * a.out_stride;
     sample_t *sym = out + 2048 + (long long)l * (N + a.gi);
     BND(a.out_len == 0 || (long long)f * a.out_stride + 2048 + (long long)(l + 1) * (N + a.gi) <= a.out_len);
-    // parking space for the even-bin half of a 32K symbol: the first half of the symbol itself when the output is
-    // complex64 (the odd-bin phase overwrites it in place, the lines are still in L2), a per-CTA scratch slot otherwise
-    float2 *park = FMT == 0 ? reinterpret_cast<float2 *>(sym) + a.gi : a.scratch + (long long)blockIdx.x * M;
 
     if (l == 0)
       for (int i = threadIdx.x; i < 2048; i += T) {
@@ -2167,37 +2222,23 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
       if constexpr (REGTW) {
         // radix 4 over the whole sub-transform: butterfly i = tid + 512 j (j < 8) reads x[i + q M/4] and produces the
         // samples i + k M/4.  W_M^i = W_M^tid * exp(j 2 pi j / 32); for the 32K recombination W_N^(i + k M/4) =
-        // W_N^tid * exp(j 2 pi j / 64) * exp(j 2 pi k / 8).  The parked even-bin values of butterfly j + 1 are requested
-        // from L2 while butterfly j is computed.
+        // W_N^tid * exp(j 2 pi j / 64) * exp(j 2 pi k / 8).  32K: phase 0 parks its results E in TMEM (8 columns per
+        // butterfly, no global stores); phase 1 requests butterfly j's E at the head of butterfly j and waits for it just
+        // before the recombination.  The tcgen05 instructions stay outside the per-thread cyclic-prefix conditions.
         constexpr int NL = M / 4, NBT = NL / T;
         constexpr int XS = NL + NL / 16;                      // padx(q * NL) = q * XS
         sample_t *o = sym + a.gi + threadIdx.x;
         const bool odd_phase = SPLIT == 2 && phase == 1;
-        const float2 *pk = park + threadIdx.x;
-        // parked even-bin values: requested from L2 PARK_AHEAD butterflies before their use, kept in a ring of
-        // PARK_AHEAD + 1 register sets.  One ahead leaves ~10 % of the kernel's stall samples on the first use of e[];
-        // two or three ahead spill at the 128-register cap and are slower (0.601 -> 0.612 / 0.638 ms)
-#ifndef PARK_AHEAD
-#define PARK_AHEAD 1
-#endif
-        float2 e[PARK_AHEAD + 1][4];
-        if (odd_phase) {
-#pragma unroll
-          for (int jj = 0; jj < PARK_AHEAD; jj++)
-#pragma unroll
-            for (int k = 0; k < 4; k++) e[jj][k] = pk[jj * T + k * NL];
-        }
+        if (odd_phase) tmem_wait_st();                        // phase 0's stores have landed
 #pragma unroll
         for (int j = 0; j < NBT; j++) {
           const int i = threadIdx.x + j * T;
           const float2 *xb = x + padx(i);
+          float2 e[4];
+          if (odd_phase) tmem_ld4(park_col + 8u * j, e);
           float2 v[4];
 #pragma unroll
           for (int q = 0; q < 4; q++) v[q] = xb[q * XS];
-          if (odd_phase && j + PARK_AHEAD < NBT) {
-#pragma unroll
-            for (int k = 0; k < 4; k++) e[(j + PARK_AHEAD) % (PARK_AHEAD + 1)][k] = pk[(j + PARK_AHEAD) * T + k * NL];
-          }
           const float2 w1 = j ? cmul(tw_last, w32(j)) : tw_last;
           const float2 w2 = cmul(w1, w1), w3 = cmul(w2, w1);
           v[1] = cmul(v[1], w1); v[2] = cmul(v[2], w2); v[3] = cmul(v[3], w3);
@@ -2212,18 +2253,23 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
             }
           }
           else if (phase == 0) {
-            float2 *pw = park + threadIdx.x;
+            // even-bin half E[n], n = i + k M/4: read back only by this thread, in phase 1
+            float2 r[4];
 #pragma unroll
-            for (int k = 0; k < 4; k++) pw[j * T + k * NL] = __fmul2_rn(v[bitrev_c(k, 4)], make_float2(a.norm, a.norm));
+            for (int k = 0; k < 4; k++) r[k] = __fmul2_rn(v[bitrev_c(k, 4)], make_float2(a.norm, a.norm));
+            tmem_st4(park_col + 8u * j, r);
           }
           else {
             sample_t *ocp = sym + ((long long)threadIdx.x + M - cp_from);
             const float2 wi = j ? cmul(tw_rec, w64(j)) : tw_rec;
+            float2 r[4];
+#pragma unroll
+            for (int k = 0; k < 4; k++) r[k] = cmul(tw16(v[bitrev_c(k, 4)], 2 * k), wi);
+            tmem_wait_ld4(e);
 #pragma unroll
             for (int k = 0; k < 4; k++) {
-              const float2 r = cmul(tw16(v[bitrev_c(k, 4)], 2 * k), wi);
-              store_sample(o, j * T + k * NL, cadd(e[j % (PARK_AHEAD + 1)][k], r));
-              const float2 hi = csub(e[j % (PARK_AHEAD + 1)][k], r);
+              store_sample(o, j * T + k * NL, cadd(e[k], r[k]));
+              const float2 hi = csub(e[k], r[k]);
               store_sample(o, j * T + k * NL + M, hi);
               if (i + k * NL + M >= cp_from) store_sample(ocp, j * T + k * NL, hi);
             }
@@ -2246,50 +2292,25 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
         dft_reg<16>(v);
         // sample t = i + k NLAST: one 64-bit base per destination, compile-time offsets k NLAST
         sample_t *o = sym + a.gi + i;
-        if (SPLIT == 1) {
-          sample_t *ocp = sym + ((long long)i - cp_from);       // cyclic prefix: sample t >= N - gi also goes to t - (N - gi)
+        sample_t *ocp = sym + ((long long)i - cp_from);       // cyclic prefix: sample t >= N - gi also goes to t - (N - gi)
 #pragma unroll
-          for (int k = 0; k < 16; k++) {
-            float2 r = v[bitrev_c(k, 16)];
-            r = __fmul2_rn(r, make_float2(a.norm, a.norm));
-            store_sample(o, k * NLAST, r);
-            if (i + k * NLAST >= cp_from) store_sample(ocp, k * NLAST, r);
-          }
-        }
-        else if (phase == 0) {
-          float2 *pk = park + i;
-#pragma unroll
-          for (int k = 0; k < 16; k++) {
-            float2 r = v[bitrev_c(k, 16)];
-            r = __fmul2_rn(r, make_float2(a.norm, a.norm));
-            // even-bin half E[n]: parked (stays in L2); the odd-bin phase reads it back (same thread, same
-            // address) and writes both halves and the cyclic prefix exactly once
-            pk[k * NLAST] = r;
-          }
-        }
-        else {
-          // odd-bin half: out[n] = E[n] + W_N^n O[n], out[n + N/2] = E[n] - W_N^n O[n], n = i + k M/16,
-          // W_N^n = W_N^i * exp(j 2 pi k / 32); E is re-read in two batches of 8
-          const float2 *pk = park + i;
-          sample_t *ocp = sym + ((long long)i + M - cp_from);
-          const float2 wi = __fmul2_rn(__ldg(a.tw_split + i), make_float2(a.norm, a.norm));
-#pragma unroll
-          for (int h = 0; h < 2; h++) {
-            float2 e[8];
-#pragma unroll
-            for (int k = 0; k < 8; k++) e[k] = pk[(8 * h + k) * NLAST];
-#pragma unroll
-            for (int k = 0; k < 8; k++) {
-              const int kk = 8 * h + k;
-              const float2 r = cmul(cmul(v[bitrev_c(kk, 16)], w32(kk)), wi);
-              store_sample(o, kk * NLAST, cadd(e[k], r));
-              const float2 hi = csub(e[k], r);
-              store_sample(o, kk * NLAST + M, hi);
-              if (i + kk * NLAST + M >= cp_from) store_sample(ocp, kk * NLAST, hi);
-            }
-          }
+        for (int k = 0; k < 16; k++) {
+          float2 r = v[bitrev_c(k, 16)];
+          r = __fmul2_rn(r, make_float2(a.norm, a.norm));
+          store_sample(o, k * NLAST, r);
+          if (i + k * NLAST >= cp_from) store_sample(ocp, k * NLAST, r);
         }
       }
+    }
+  }
+  if constexpr (SPLIT == 2) {
+    // every thread's TMEM accesses are complete (each load was waited for) before warp 0 frees the columns; the
+    // kernel has no other way out
+    tmem_fence_before_sync();
+    __syncthreads();
+    if (threadIdx.x < 32) {
+      tmem_fence_after_sync();
+      tmem_dealloc<OFDM_PARK_COLS>(park_col);
     }
   }
 }
@@ -2322,13 +2343,10 @@ static void launch_ofdm_c(const OfdmArgs &a, cudaStream_t s)
     case 10: launch_ofdm_t<10, 256, C16, FMT, 1>(a, s); break;
     case 11: launch_ofdm_t<11, 256, C16, FMT, 1>(a, s); break;
     case 12: launch_ofdm_t<12, 256, C16, FMT, 1>(a, s); break;
-    case 13:
-      // 8K symbols, or 16K symbols as two 8K halves (two CTAs per SM instead of one: OfdmDevice::init decides)
-      if (a.split == 2) launch_ofdm_t<13, 512, C16, FMT, 2>(a, s);
-      else launch_ofdm_t<13, 512, C16, FMT, 1>(a, s);
-      break;
+    case 13: launch_ofdm_t<13, 512, C16, FMT, 1>(a, s); break;
     case 14:
-      // 512 threads with up to 128 registers each: two butterflies per thread and pass, interleaved by the compiler
+      // 512 threads with up to 128 registers each: two butterflies per thread and pass, interleaved by the compiler;
+      // 32K symbols (split = 2) as two 16K halves
       if (a.split == 2) launch_ofdm_t<14, 512, C16, FMT, 2>(a, s);
       else launch_ofdm_t<14, 512, C16, FMT, 1>(a, s);
       break;

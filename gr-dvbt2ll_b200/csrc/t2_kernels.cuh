@@ -140,7 +140,6 @@ struct OfdmArgs {
   void *out;           long long out_stride;     // samples per T2 frame (complex64, or short2 when out_fmt = 1)
   int out_fmt;               // 0 = complex64, 1 = interleaved 16-bit I/Q (x * 32767, saturated)
   float sink_gain;           // extra gain folded into `norm` and the P1 samples (1 = the reference block's output)
-  float2 *scratch;           // [grid][M] parking space for the even-bin half of 32K symbols
   const int32_t *code_pos;   // [num_symbols][split][M] carrier codes in shared-memory POSITION order
   const float2 *pool;        // special cells, one copy per L1-post variant (copy v holds the L1-post cells of frame index v)
   long long pool_stride;     // cells per copy
