@@ -370,21 +370,21 @@ struct BbHandle : dvbt2ll_handle {
     const int base = (noutput - 80 - (plan.fec.nbch - plan.fec.kbch)) / 8;
     return plan.mode == t2::INPUTMODE_NORMAL ? base : base + ((plan.fec.kbch - 80) / 8) / 187 + 1;
   }
-  uint32_t crc_mask[8];
   uint32_t crc_pos_mask[47][8];
   int dev_init()
   {
     std::vector<uint8_t> scr(plan.scramble);
     scr.resize((scr.size() + 7) & ~(size_t)3, 0);      // kernel XORs the scrambler word-wise
     CK(upload(d_scr, scr));
+    CK(upload(d_crc, std::vector<uint8_t>(plan.crc8_tab, plan.crc8_tab + 256)));   // byte table: the BB header's CRC-8
     // CRC-8 slicing-by-4 tables: S1 = byte table, S(k+1)[x] = S1[Sk[x]] (a byte followed by k zero bytes)
     std::vector<uint8_t> crc(1024);
     for (int x = 0; x < 256; x++) {
       uint8_t v = plan.crc8_tab[x];
       for (int k = 0; k < 4; k++) { crc[k * 256 + x] = v; v = plan.crc8_tab[v]; }
     }
-    CK(upload(d_crc, crc));
     // the same four-byte step as parity masks (GF(2)-linear in the 32 bits): byte i of the word is followed by 3 - i more
+    uint32_t crc_mask[8];
     for (int k = 0; k < 8; k++) {
       crc_mask[k] = 0;
       for (int i = 0; i < 4; i++)
@@ -437,7 +437,6 @@ struct BbHandle : dvbt2ll_handle {
     a.mode = plan.mode; a.inband = plan.inband ? 1 : 0; a.fecblocks = plan.fecblocks;
     a.chunk_bytes = plan.chunk_bytes; a.lead_zero_bytes = plan.lead_zero_bytes;
     a.scramble = d_scr.as<uint8_t>(); a.crc8_tab = d_crc.as<uint8_t>(); a.bch_tab = d_tab.as<uint32_t>();
-    for (int k = 0; k < 8; k++) a.crc8_mask[k] = crc_mask[k];
     std::memcpy(a.crc8_pos_mask, crc_pos_mask, sizeof(crc_pos_mask));
     a.bch_cols = d_cols.as<uint32_t>(); a.inband_bytes = d_ib.as<uint8_t>();
     a.out = d_out; a.out_pitch = out_pitch; a.sync_errors = h_err;
@@ -802,18 +801,12 @@ struct ChainHandle : dvbt2ll_handle {
   cudaStream_t stream2;
   int last_frames;
   long long next_frame;  // stream position of the generic work() / work_device() path (T2 frames consumed so far)
-  bool fuse_fec;         // LDPC and mapper as one kernel (DVBT2LL_FUSE_FEC=1).  Off by default: measured on B200 the fused
-                         // kernel takes 0.320 ms for 64 x c3 against 0.127 + 0.162 ms for the two kernels -- its phases are
-                         // short and separated by CTA barriers, the warp-per-FECFRAME LDPC kernel has none
-  bool taps;             // keep the packed LDPC codewords for dvbt2ll_chain_tap("fec") (parity tests)
   bool timing;
   enum { TIMING_SLOTS = 64 };
   cudaEvent_t ev[TIMING_SLOTS][5];     // per-run event sets so the timed loop never has to synchronise
   long long n_timed;
-  ChainHandle() : dvbt2ll_handle(CHAIN), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), last_frames(0), next_frame(0), fuse_fec(false), taps(false), timing(false)
+  ChainHandle() : dvbt2ll_handle(CHAIN), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), last_frames(0), next_frame(0), timing(false)
   {
-    const char *e = std::getenv("DVBT2LL_FUSE_FEC");
-    if (e && e[0] == '1') fuse_fec = true;
     n_timed = 0;
     for (int s = 0; s < TIMING_SLOTS; s++) for (int i = 0; i < 5; i++) ev[s][i] = 0;
   }
@@ -909,8 +902,8 @@ struct ChainHandle : dvbt2ll_handle {
     cudaEvent_t *tev = ev[n_timed % TIMING_SLOTS];
     if (timing) cudaEventRecord(tev[0], s);
     uint8_t *bch_buf = d_bch.as<uint8_t>() + (size_t)buf_frame * F() * bp;
-    if (!fuse_fec || taps) CK(d_fec.ensure((size_t)max_frames * F() * fp + 64));
-    uint8_t *fec_buf = d_fec.as<uint8_t>() ? d_fec.as<uint8_t>() + (size_t)buf_frame * F() * fp : 0;
+    CK(d_fec.ensure((size_t)max_frames * F() * fp + 64));
+    uint8_t *fec_buf = d_fec.as<uint8_t>() + (size_t)buf_frame * F() * fp;
     uint16_t *cell_buf = d_cells.as<uint16_t>() + (size_t)buf_frame * cells16_stride();
     // BB framing + BCH, PLP by PLP: row c * P + p of the TS holds PLP p of channel c; every PLP has its own stream
     // position (packet phase, in-band cycle = its FEC blocks per frame), and its codewords go to their place inside
@@ -938,17 +931,9 @@ struct ChainHandle : dvbt2ll_handle {
     ma.ci_inv = d_ci_inv.as<uint16_t>(); ma.fec_shift = d_fec_shift.as<int32_t>(); ma.fecblocks = F();   // cell-interleaved
     ma.ci_inv4 = d_ci_inv4.as<uint16_t>(); ma.ci_inv4_stride = ci4_stride;
     ma.out_len = (long long)frames * cells16_stride();
-    if (fuse_fec) {
-      // LDPC + bit interleaver / mapper in one kernel: the LDPC codeword stays in shared memory (the packed codewords
-      // reach HBM only when the parity-test tap is on)
-      if (timing) cudaEventRecord(tev[2], s);
-      t2k::launch_fec(la, ma, taps ? fec_buf : 0, fp, s);
-    }
-    else {
-      t2k::launch_ldpc(la, s);
-      if (timing) cudaEventRecord(tev[2], s);
-      t2k::launch_map(ma, s);
-    }
+    t2k::launch_ldpc(la, s);
+    if (timing) cudaEventRecord(tev[2], s);
+    t2k::launch_map(ma, s);
     if (timing) cudaEventRecord(tev[3], s);
     t2k::OfdmArgs oa;
     odev.fill(oa, oplan, tables.pool);
@@ -1534,10 +1519,7 @@ long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, lon
   const void *src; size_t bytes;
   std::string n(stage);
   if (n == "bch") { src = c->d_bch.p; bytes = nfec * align16(c->bb.plan.fec.nbch / 8); }
-  else if (n == "fec") {
-    if (c->fuse_fec && !c->taps) return fail(DVBT2LL_ERR_INVALID, "chain: the LDPC codewords stay on chip; call dvbt2ll_chain_enable_taps before the run");
-    src = c->d_fec.p; bytes = nfec * align16(c->bb.plan.fec.nldpc / 8);
-  }
+  else if (n == "fec") { src = c->d_fec.p; bytes = nfec * align16(c->bb.plan.fec.nldpc / 8); }
   else if (n == "cells") { src = c->d_cells.p; bytes = (size_t)c->last_frames * c->cells16_stride() * sizeof(uint16_t); }
   else return fail(DVBT2LL_ERR_INVALID, "chain: unknown tap");
   CK(cudaStreamSynchronize(c->stream));
@@ -1555,14 +1537,6 @@ int dvbt2ll_chain_set_sink(dvbt2ll_handle *h, int format, float gain)
   c->sink_gain = gain;
   return 0;
 }
-
-void dvbt2ll_chain_enable_taps(dvbt2ll_handle *h, int on)
-{
-  ChainHandle *c = as_chain(h);
-  if (c) c->taps = on != 0;
-}
-
-int dvbt2ll_chain_fused_fec(const dvbt2ll_handle *h) { ChainHandle *c = as_chain(h); return c ? (c->fuse_fec ? 1 : 0) : 0; }
 
 void dvbt2ll_chain_enable_timing(dvbt2ll_handle *h, int on)
 {

@@ -9,10 +9,11 @@
 //                                  memory), constellation LUT, cyclic Q delay, coalesced float2 stores
 //   k_gather   grid-stride       : frame mapper as one static gather
 //   k_ofdm     CTA per OFDM symbol: carrier fill (gather + pilots), in-place shared-memory DIT FFT
-//                                  (radix 16/8/4/2 in registers, XOR-swizzled), scale, CP, P1
+//                                  (radix 16/8/4/2 in registers, padded layout), scale, CP, P1
 //
-// None of the stages is a dense contraction, so no tensor-core path is used: the cell-domain
-// kernels are HBM/L2 bound, the bit-domain ones integer-pipe bound, the IFFT shared-memory bound.
+// None of the stages is a dense contraction, so no tensor-core MMA is used: the cell-domain kernels are
+// HBM/L2 bound, the bit-domain ones integer-pipe bound, the IFFT shared-memory bound.  The 32K k_ofdm
+// uses tensor memory as storage only (the parked even-bin half, see the TMEM helpers).
 #include "t2_kernels.cuh"
 
 #include <atomic>
@@ -100,17 +101,6 @@ __device__ __forceinline__ long long hem_ts_index(long long P, int c0)
   return t0 + 1 + pp + pp / 187;
 }
 
-// 4 bytes at an arbitrary byte address, via aligned 32-bit loads (little endian)
-__device__ __forceinline__ uint32_t load_u32_unaligned(const uint8_t *p)
-{
-  const uintptr_t ad = reinterpret_cast<uintptr_t>(p);
-  const uint32_t *w = reinterpret_cast<const uint32_t *>(ad & ~(uintptr_t)3);
-  const int sh = (int)(ad & 3) * 8;
-  const uint32_t lo = __ldg(w);
-  if (sh == 0) return lo;
-  return __funnelshift_r(lo, __ldg(w + 1), sh);
-}
-
 // W6 = false: remainder register of at most 160 bits (5 words): the sixth word is identically zero and skipped
 template <bool W6>
 __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
@@ -120,9 +110,6 @@ __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
   // (k = nibble position inside a 16-bit step: n x^(r + 4k) mod g) for lane l sits at ((k*16 + n)*NW + w)*32 + l,
   // i.e. always in bank l -- 32 lanes looking up 32 different rows never conflict (a byte-indexed table shared by
   // the warp costs ~3.3 wavefronts per access instead).
-  // (BCH_TAB_VECTOR: rows kept as one 16-byte vector + the remaining one or two words per lane, so a row costs two
-  // load instructions instead of NW -- 30 % fewer LDS, same wavefronts; measured 1 % slower (0.198 -> 0.200 ms for
-  // 64 x c3, 0.025 -> 0.027 for c1), so not the default)
   constexpr int NW = W6 ? 6 : 5;
   uint32_t *s_ntab = reinterpret_cast<uint32_t *>(smem_raw);  // 4 * 16 * NW * 32
   uint32_t *s_cols = s_ntab + 4 * 16 * NW * 32;               // 6 * 32 * 6
@@ -140,14 +127,7 @@ __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
 #pragma unroll
     for (int u = 0; u < 8; u++) {
       const int i = i0 + u * blockDim.x;
-#ifndef BCH_TAB_VECTOR
       const int w = (i >> 5) % NW, kn = (i >> 5) / NW, k = kn >> 4, n = kn & 15;
-#else
-      // vector rows: words 0..3 of (row kn, lane l) at (kn*32 + l)*4 + w, the rest at 8192 + (kn*32 + l)*(NW-4) + (w-4)
-      constexpr int NB = NW - 4;
-      const int jb = i - 8192;
-      const int w = i < 8192 ? (i & 3) : 4 + jb % NB, kn = i < 8192 ? (i >> 7) : jb / (NB * 32), k = kn >> 4, n = kn & 15;
-#endif
       // from the byte tables T0 = b x^r, T1 = b x^(r+8): nibble n at position k is byte (n << 4*(k&1)) of table k>>1
       v[u] = i < 4 * 16 * NW * 32 ? __ldg(a.bch_tab + ((k >> 1) * 256 + (n << (4 * (k & 1)))) * 6 + w) : 0u;
     }
@@ -203,15 +183,6 @@ __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
       }
       if (lane < 2) buf[10 + lane] = src[lane];
       const int w_end = (10 + Dj) >> 2;                    // words [3, w_end) lie completely inside the payload
-#ifdef BB_STAGE_OLD
-      for (int w0 = 3 + lane; w0 < w_end; w0 += 128) {     // four loads in flight per lane
-        uint32_t d[4];
-#pragma unroll
-        for (int u = 0; u < 4; u++) if (w0 + 32 * u < w_end) d[u] = load_u32_unaligned(src + 4 * (w0 + 32 * u) - 10);
-#pragma unroll
-        for (int u = 0; u < 4; u++) if (w0 + 32 * u < w_end) bufw[w0 + 32 * u] = d[u];
-      }
-#else
       {
         // buffer word w = payload bytes 4 w - 10 .. 4 w - 7: the payload's misalignment is the same for every word of the
         // frame, so a word is a funnel shift of two ALIGNED global words.  All eight loads of a batch are issued
@@ -235,7 +206,6 @@ __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
             if (w0 + 32 * u <= last) bufw[3 + w0 + 32 * u] = __funnelshift_r(lo[u], hi[u], sh);
         }
       }
-#endif
       for (int i = 4 * w_end - 10 + lane; i < Dj; i += 32) buf[10 + i] = src[i];
       // the 187 bytes before the frame (previous packet's tail) for the first CRC-8; missing history reads as 0,
       // which leaves a zero CRC state unchanged
@@ -325,7 +295,6 @@ __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
       const int e = s + a.chunk_bytes;
       if (s < 0) s = 0;
       int i = s;
-#ifndef BCH_TAB_VECTOR
       const uint32_t *nt = s_ntab + lane;
       constexpr int ROW = NW * 32;              // words between rows of a table
       // one message byte: two nibble rows
@@ -351,43 +320,6 @@ __global__ void __launch_bounds__(BB_MAX_WARPS * 32) k_bb_bch(const BbArgs a)
         r4 = ((r4 << 16) | (W6 ? r5 >> 16 : 0u)) ^ t3[128] ^ t2[128] ^ t1[128] ^ t0[128];
         if (W6) r5 = (r5 << 16) ^ t3[NW * 32 - 32] ^ t2[NW * 32 - 32] ^ t1[NW * 32 - 32] ^ t0[NW * 32 - 32];
       };
-#else
-      constexpr int NB = NW - 4;
-      const uint4 *ntv = reinterpret_cast<const uint4 *>(s_ntab) + lane;              // row kn: ntv[kn * 32]
-      const uint32_t *ntb = s_ntab + 8192 + lane * NB;                                // row kn: ntb[kn * 32 * NB (+ 1)]
-      // one message byte: two nibble rows
-      auto step8 = [&](uint32_t byte) {
-        const uint32_t x = (r0 >> 24) ^ byte;
-        const uint32_t k1 = 16u + (x >> 4), k0 = x & 15u;
-        const uint4 a1 = ntv[k1 * 32], a0 = ntv[k0 * 32];
-        const uint32_t b1 = ntb[k1 * (32 * NB)], b0 = ntb[k0 * (32 * NB)];
-        r0 = ((r0 << 8) | (r1 >> 24)) ^ a1.x ^ a0.x;
-        r1 = ((r1 << 8) | (r2 >> 24)) ^ a1.y ^ a0.y;
-        r2 = ((r2 << 8) | (r3 >> 24)) ^ a1.z ^ a0.z;
-        r3 = ((r3 << 8) | (r4 >> 24)) ^ a1.w ^ a0.w;
-        r4 = ((r4 << 8) | (W6 ? r5 >> 24 : 0u)) ^ b1 ^ b0;
-        if (W6) r5 = (r5 << 8) ^ ntb[k1 * (32 * NB) + (NB - 1)] ^ ntb[k0 * (32 * NB) + (NB - 1)];
-      };
-      // two message bytes (big-endian halfword): four nibble rows, all independent of each other
-      auto step16 = [&](uint32_t half) {
-        const uint32_t x = (r0 >> 16) ^ half;
-        const uint32_t k3 = 48u + (x >> 12), k2 = 32u + ((x >> 8) & 15u), k1 = 16u + ((x >> 4) & 15u), k0 = x & 15u;
-        const uint4 a3 = ntv[k3 * 32], a2 = ntv[k2 * 32], a1 = ntv[k1 * 32], a0 = ntv[k0 * 32];
-        uint32_t b3, b2, b1, b0, d3 = 0, d2 = 0, d1 = 0, d0 = 0;
-        if (W6) {
-          const uint2 q3 = *reinterpret_cast<const uint2 *>(ntb + k3 * (32 * NB)), q2 = *reinterpret_cast<const uint2 *>(ntb + k2 * (32 * NB)),
-                      q1 = *reinterpret_cast<const uint2 *>(ntb + k1 * (32 * NB)), q0 = *reinterpret_cast<const uint2 *>(ntb + k0 * (32 * NB));
-          b3 = q3.x; b2 = q2.x; b1 = q1.x; b0 = q0.x; d3 = q3.y; d2 = q2.y; d1 = q1.y; d0 = q0.y;
-        }
-        else { b3 = ntb[k3 * (32 * NB)]; b2 = ntb[k2 * (32 * NB)]; b1 = ntb[k1 * (32 * NB)]; b0 = ntb[k0 * (32 * NB)]; }
-        r0 = ((r0 << 16) | (r1 >> 16)) ^ a3.x ^ a2.x ^ a1.x ^ a0.x;
-        r1 = ((r1 << 16) | (r2 >> 16)) ^ a3.y ^ a2.y ^ a1.y ^ a0.y;
-        r2 = ((r2 << 16) | (r3 >> 16)) ^ a3.z ^ a2.z ^ a1.z ^ a0.z;
-        r3 = ((r3 << 16) | (r4 >> 16)) ^ a3.w ^ a2.w ^ a1.w ^ a0.w;
-        r4 = ((r4 << 16) | (W6 ? r5 >> 16 : 0u)) ^ b3 ^ b2 ^ b1 ^ b0;
-        if (W6) r5 = (r5 << 16) ^ d3 ^ d2 ^ d1 ^ d0;
-      };
-#endif
       // head: single bytes up to a word boundary of the frame buffer (the same 0..3 bytes for every lane: the chunk
       // length is a multiple of 4); body: one conflict-free 32-bit load per four message bytes; tail: single bytes
       for (; (i & 3) && i < e; i++) step8(buf[i]);
@@ -517,9 +449,6 @@ __global__ void __launch_bounds__(LDPC_WARPS * 32, 8) k_ldpc(const LdpcArgs a, i
     {
       uint32_t *ow = reinterpret_cast<uint32_t *>(out);
       const int nw = info_bytes >> 2;
-#ifdef LDPC_LOADS_OLD
-      for (int i = lane; i < nw; i += 32) ow[i] = __ldg(cw + i);
-#else
       for (int i = lane; i < nw; i += 256) {           // eight loads in flight per lane (their latency was 13 % of the stall samples)
         uint32_t v[8];
 #pragma unroll
@@ -527,20 +456,11 @@ __global__ void __launch_bounds__(LDPC_WARPS * 32, 8) k_ldpc(const LdpcArgs a, i
 #pragma unroll
         for (int u = 0; u < 8; u++) if (i + 32 * u < nw) ow[i + 32 * u] = v[u];
       }
-#endif
       for (int b = (nw << 2) + lane; b < info_bytes; b += 32) out[b] = __ldg(in + b);
     }
     // ---- wrap-extended groups: 13 words = circular bits [0, 416) of each 360-bit group.  A group is 45 bytes, so
     // word w is the big-endian 32-bit value at byte 45 g + 4 w (w <= 10), bytes {44, 0, 1, 2} (w = 11) or bytes 3..6
     // (w = 12): unaligned loads by byte permute (bytes past the group only land in positions that are masked off)
-#ifdef LDPC_LOADS_OLD
-    for (int idx = lane; idx < G * 13; idx += 32) {
-      const int g = idx / 13, w = idx - g * 13;
-      uint32_t v = be32_at(cw, 45 * g + (w == 12 ? 3 : 4 * w));
-      if (w == 11) v = (v & 0xFF000000u) | (be32_at(cw, 45 * g) >> 8);
-      ext[idx] = v;
-    }
-#else
     for (int idx0 = lane; idx0 < G * 13; idx0 += 128) {      // four words (twelve loads) in flight per lane
       uint32_t v[4], h[4];
       int wsel[4];
@@ -556,7 +476,6 @@ __global__ void __launch_bounds__(LDPC_WARPS * 32, 8) k_ldpc(const LdpcArgs a, i
       for (int u = 0; u < 4; u++)
         if (idx0 + 32 * u < G * 13) ext[idx0 + 32 * u] = wsel[u] == 11 ? (v[u] & 0xFF000000u) | (h[u] >> 8) : v[u];
     }
-#endif
     __syncwarp();
     // ---- pre-accumulator parity rows: R_t = XOR of rotated info groups
     if (a.lane_per_row) {
@@ -590,7 +509,6 @@ __global__ void __launch_bounds__(LDPC_WARPS * 32, 8) k_ldpc(const LdpcArgs a, i
       uint32_t acc = 0;
       const int e1 = a.row_ptr[t + 1];
       int e = a.row_ptr[t];
-#ifndef LDPC_LOADS_OLD
       for (; e + 4 <= e1; e += 4) {                          // four table entries and their windows in flight
         uint32_t en[4];
 #pragma unroll
@@ -603,7 +521,6 @@ __global__ void __launch_bounds__(LDPC_WARPS * 32, 8) k_ldpc(const LdpcArgs a, i
           acc ^= window32(ext + (en[u] & 0xffffu) * 13, p);
         }
       }
-#endif
       for (; e < e1; e++) {
         const uint32_t en = __ldg(a.entries + e);
         int p = 32 * w - (int)(en >> 16);
@@ -695,7 +612,9 @@ void launch_ldpc(const LdpcArgs &a, cudaStream_t s)
 // 32 consecutive codeword bits u[rows*c + (d - twist[c]) mod rows] -- one funnel-shifted window of the
 // packed codeword per column.  The windows are loaded in OUTPUT-bit order (demux folded into which
 // column feeds which row), a 32x32 bit-matrix transpose in registers turns them into 32 cell-pair words,
-// and the cells go to shared memory as bytes.  QPSK (no twist / demux) uses the generic bit_src table.
+// and the cells go to shared memory as bytes; the column count is a template parameter (k_map_n).  QPSK (no twist /
+// demux: k_map, k_map_qtr) maps the cells whose bits sit in place in the codeword through a byte table, the parity
+// cells by in-register bit transposes (k_map_qtr) or, like any other cell, bit by bit through the bit_src table.
 constexpr int MAP_THREADS = 128;
 
 template <int J>
@@ -722,36 +641,17 @@ __device__ __forceinline__ void transpose32(uint32_t (&A)[32])
   transpose32_stage<1>(A);
 }
 
-// Geometry of the column-twist path kept in shared memory: per output bit of the demux word, the first codeword bit
-// of the column that feeds it and that column's twist; plus the constellation table
-__device__ __forceinline__ void map_setup(const MapArgs &a, float2 *lut, int *s_base, int *s_twist)
-{
-  // (the constellation table is only read by the complex64 output of the drop-in block: the chain's 16-bit codes skip it)
-  if (!a.out16)
-    for (int i = threadIdx.x; i < (1 << a.mod); i += blockDim.x) lut[i] = a.lut[i];
-  if (threadIdx.x < 16) {
-    const int rho = threadIdx.x;
-    int col = 0;
-#pragma unroll
-    for (int k = 0; k < 16; k++) if (k == rho) col = a.col_of_bit[k];
-    int tw = 0;
-#pragma unroll
-    for (int k = 0; k < 16; k++) if (k == col) tw = a.twist_of_col[k];
-    s_base[rho] = a.ncol ? (a.nldpc / a.ncol) * col : 0;
-    s_twist[rho] = tw;
-  }
-}
-
 // Bit interleaver + demux + cell codes + output of FECFRAME f whose packed "u"-order codeword sits in shared memory
 // (raw byte order, zero slack words behind it).  The caller has synchronised the CTA on `u`; ends without a barrier.
 // QTR: the instantiation that carries the QPSK transposed-parity path (its 32-register tile would otherwise raise the
 // register count of every mapper launch)
-// NCOL > 0: the column count of the twist matrix as a compile-time constant -- which rows of the bit tile are empty is
-// then known to the compiler (the transposes shrink for 8 and 12 columns) and the per-bit geometry comes from the
-// kernel-parameter constant bank (a.base_of_bit / a.twist_of_bit, compile-time indices) instead of shared memory.
+// NCOL: the column count of the twist matrix (8, 12 or 16) as a compile-time constant, 0 for QPSK (no twist matrix) --
+// which rows of the bit tile are empty is then known to the compiler (the transposes shrink for 8 and 12 columns) and
+// the per-bit geometry comes from the kernel-parameter constant bank (a.base_of_bit / a.twist_of_bit, compile-time
+// indices).
 template <bool QTR, int NCOL = 0>
 __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const uint32_t *u, const float2 *lut, uint16_t *cw,
-                                         const int *s_base, const int *s_twist, const int shift)
+                                         const int shift)
 {
   const int mod = a.mod, Nc = a.cell_size;
   // single-table constellation (MapPlan::im_from_re): the byte that supplies the imaginary part is kept as w~
@@ -759,9 +659,8 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
   const uint32_t tI = a.im_mask_i * 0x01010101u, tQ = a.im_mask_q * 0x01010101u, tF = a.im_flip * 0x01010101u;
   auto tilde4 = [&](uint32_t w) -> uint32_t { return tilde ? ((((w << 1) & tI) | ((w >> 1) & tQ)) ^ tF) : w; };   // four packed cell words
   auto tilde1 = [&](uint32_t w) -> uint32_t { return tilde4(w) & 0xFFu; };
-  const int ncol = NCOL ? NCOL : a.ncol;
-  if (ncol) {
-    const int rows = a.nldpc / ncol;
+  if constexpr (NCOL != 0) {
+    const int rows = a.nldpc / NCOL;
     const int groups = (rows + 31) >> 5;
     for (int g = threadIdx.x; g < groups; g += blockDim.x) {
       const int d0 = g << 5;
@@ -770,11 +669,11 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
       for (int y = 0; y < 32; y++) A[y] = 0;
 #pragma unroll
       for (int y = 16; y < 32; y++) {
-        const int rho = y - (32 - ncol);       // output bit (0 = MSB of the ncol-bit demux word) held by row y
+        const int rho = y - (32 - NCOL);       // output bit (0 = MSB of the NCOL-bit demux word) held by row y
         if (rho >= 0) {
-          int s0 = d0 - (NCOL ? a.twist_of_bit[NCOL ? y - (32 - NCOL) : 0] : s_twist[rho]);
+          int s0 = d0 - a.twist_of_bit[rho];
           if (s0 < 0) s0 += rows;
-          const int base = NCOL ? a.base_of_bit[NCOL ? y - (32 - NCOL) : 0] : s_base[rho];
+          const int base = a.base_of_bit[rho];
           const int n1 = rows - s0;
           uint32_t w = window32_be(u, base + s0);
           if (n1 < 32) w = (w & ~(0xFFFFFFFFu >> n1)) | (window32_be(u, base) >> n1);
@@ -783,8 +682,8 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
       }
       transpose32(A);
       // transpose32 uses (row, MSB-first column) coordinates: window bit i (from the MSB) of row y moves to
-      // bit y (from the MSB) of A[i], so A[i] is the ncol-bit word of row d0 + i of the twist matrix.
-      // Emit cells (two per word when ncol = 2 mod, else one) as packed bytes.
+      // bit y (from the MSB) of A[i], so A[i] is the NCOL-bit word of row d0 + i of the twist matrix.
+      // Emit cells (two per word when NCOL = 2 mod, else one) as packed bytes.
       // Four consecutive cells as bytes w = [c0 c1 c2 c3] (c0 lowest), then their codes by byte permutes: with
       // the Q delay [c0 | prev << 8, c1 | c0 << 8], [c2 | c1 << 8, c3 | c2 << 8] (prev = c3 of the previous
       // four; the first cell of the thread is patched below), without it [c0 | c0 << 8, ...].
@@ -792,7 +691,7 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
       // X = the four words supplying the imaginary parts (as w~): the previous cell's under the Q delay, else the own
       const int xs = a.cyclic_delay ? 8 : 0;
       uint32_t wprev = 0;
-      if (ncol == 2 * mod) {
+      if (NCOL == 2 * mod) {
         uint32_t *dst = reinterpret_cast<uint32_t *>(cw + 2 * d0 + 2 * g);      // 64 cells + 1 pad word per thread
 #pragma unroll
         for (int i = 0; i < 32; i += 2) {
@@ -819,7 +718,7 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
     if (a.cyclic_delay) {
       // first cell of every thread's run: the imaginary part comes from the last cell of the previous run
       __syncthreads();
-      const int run = ncol == 2 * mod ? 64 : 32;
+      const int run = NCOL == 2 * mod ? 64 : 32;
       for (int c = threadIdx.x * run; c < Nc; c += blockDim.x * run) {
         const int pc = c == 0 ? Nc - 1 : c - 1;
         reinterpret_cast<uint8_t *>(cw)[2 * (c + 2 * (c >> 6)) + 1] = (uint8_t)tilde1(cw[pc + 2 * (pc >> 6)]);
@@ -831,7 +730,6 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
     const uint8_t *ub = reinterpret_cast<const uint8_t *>(u);
     // cells whose bits sit in place in the codeword (the info part; everything for the parity-interleaved codes): a
     // 32-bit word is sixteen cells, each byte's four codes come from one 8-byte table entry
-#ifndef MAP_QPSK_GENERIC
     const int lin = a.qpsk_lin_cells;
     for (int wi = threadIdx.x; wi < (lin >> 4); wi += blockDim.x) {
       const uint32_t W = u[wi];                      // raw byte order: byte k of the stream is bits 8k..8k+7
@@ -843,9 +741,6 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
         dst[2 * k + 1] = cd.y;
       }
     }
-#else
-    const int lin = 0;
-#endif
     // cells [lin, gen_end) go bit by bit through bit_src; with the transposed parity path that is only the few info
     // cells behind the last whole table word
     const int gen_end = QTR && a.qpsk_par_q > 0 ? (a.qpsk_nbch >> 1) : Nc;
@@ -974,7 +869,6 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
         // (c2: mapper 0.071 -> 0.064 ms); with eight CTAs per SM the same batching is 5 % SLOWER (c3: 0.137 -> 0.144), so
         // the QAM instantiation keeps the two-deep unrolled loop
         int g = threadIdx.x;
-#ifndef MAP_PERM_BATCH_OLD
         if (QTR)
         for (; g + 3 * MAP_THREADS < ngrp; g += 4 * MAP_THREADS) {
           uint2 ci[4];
@@ -983,7 +877,6 @@ __device__ __forceinline__ void map_body(const MapArgs &a, const int f, const ui
 #pragma unroll
           for (int k4 = 0; k4 < 4; k4++) emit4(g + k4 * MAP_THREADS, ci[k4]);
         }
-#endif
 #pragma unroll 2
         for (; g < ngrp; g += MAP_THREADS) emit4(g, __ldg(ci4 + g));
         // ragged ends: up to 3 cells before and after the aligned part
@@ -1062,7 +955,6 @@ __device__ __forceinline__ void k_map_impl(const MapArgs &a)
   // cell codes of the FECFRAME: own cell word | (word supplying the imaginary part << 8), i.e. the previous cell's
   // word under the cyclic Q delay, the cell's own otherwise.  Padded: cell c at index c + 2 (c / 64).
   uint16_t *cw = reinterpret_cast<uint16_t *>(lut + (1 << a.mod));
-  __shared__ int s_base[16], s_twist[16];
   // packed codeword into shared memory as raw bytes with 16-byte asynchronous copies (frames are 16-byte pitched)
   const int n16 = (nwords + 3) >> 2;
   auto fetch = [&](int f) {
@@ -1074,7 +966,9 @@ __device__ __forceinline__ void k_map_impl(const MapArgs &a)
   };
   // the CTA's first codeword is requested before the tables are set up: one exposed global round trip instead of two
   if ((int)blockIdx.x < a.frames) fetch(blockIdx.x);
-  map_setup(a, lut, s_base, s_twist);
+  // (the constellation table is only read by the complex64 output of the drop-in block: the chain's 16-bit codes skip it)
+  if (!a.out16)
+    for (int i = threadIdx.x; i < (1 << a.mod); i += blockDim.x) lut[i] = a.lut[i];
 
   for (int f = blockIdx.x; f < a.frames; f += gridDim.x) {
     const int shift = a.fec_shift ? __ldg(a.fec_shift + f % a.fecblocks) : 0;     // requested early: used by the last stage
@@ -1085,155 +979,16 @@ __device__ __forceinline__ void k_map_impl(const MapArgs &a)
     asm volatile("cp.async.wait_group 0;\n" ::);
     if (threadIdx.x < 4) u[4 * n16 + threadIdx.x] = 0u;
     __syncthreads();
-    map_body<QTR, NCOL>(a, f, u, lut, cw, s_base, s_twist, shift);
+    map_body<QTR, NCOL>(a, f, u, lut, cw, shift);
   }
 }
+// QPSK (no twist matrix)
 __global__ void __launch_bounds__(MAP_THREADS) k_map(const MapArgs a) { k_map_impl<false>(a); }
 // 8, 12 or 16 twist-matrix columns as a compile-time constant (16QAM / short 256QAM, 64QAM, normal 256QAM)
 template <int NCOL>
 __global__ void __launch_bounds__(MAP_THREADS) k_map_n(const MapArgs a) { k_map_impl<false, NCOL>(a); }
 // QPSK with the transposed parity path: three CTAs per SM fit beside the 32400 cell codes of a normal FECFRAME
 __global__ void __launch_bounds__(MAP_THREADS, 3) k_map_qtr(const MapArgs a) { k_map_impl<true>(a); }
-
-// ================================================================================================
-// K2+K3 fused (chain mode): LDPC parity and bit interleaver / mapper of one FECFRAME per CTA.  The BCH codeword comes
-// in by asynchronous copies, the parity rows are computed by the whole CTA, laid behind the info bits in shared
-// memory in "u" order, and the mapper stages run from there: the LDPC codeword never travels through HBM.
-// ================================================================================================
-// big-endian 32-bit value at byte offset `off` of a byte stream held as raw (little-endian loaded) words in shared memory
-__device__ __forceinline__ uint32_t be32_at_smem(const uint32_t *w, int off)
-{
-  const int k = off >> 2;
-  return __byte_perm(w[k], w[k + 1], 0x0123u + 0x1111u * (unsigned)(off & 3));
-}
-
-#ifndef FEC_MIN_BLOCKS
-#define FEC_MIN_BLOCKS 6
-#endif
-__global__ void __launch_bounds__(MAP_THREADS, FEC_MIN_BLOCKS) k_fec(const LdpcArgs l, const MapArgs a, uint8_t *fec_tap, int fec_tap_pitch)
-{
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  const int nwords = (a.nldpc + 31) / 32;
-  uint32_t *u = reinterpret_cast<uint32_t *>(smem_raw);
-  float2 *lut = reinterpret_cast<float2 *>(u + map_u_words(a.nldpc));
-  uint16_t *cw = reinterpret_cast<uint16_t *>(lut + (1 << a.mod));
-  const int q = l.q, G = l.groups;
-  uint32_t *ext = reinterpret_cast<uint32_t *>(cw + ((map_cw_halfwords(a.cell_size) + 1) & ~1));   // [groups][13]
-  uint32_t *rows = ext + G * 13;                                                                     // [q][12] (+ 12 spare)
-  uint32_t *s_E = rows + q * 12 + 12;                                                                // [12] + one zero word
-  __shared__ int s_base[16], s_twist[16];
-  map_setup(a, lut, s_base, s_twist);
-  const int info_bytes = l.nbch / 8;
-  const int tid = threadIdx.x, lane = tid & 31;
-
-  for (int f = blockIdx.x; f < l.frames; f += gridDim.x) {
-    const uint8_t *in = l.in + (long long)f * l.in_pitch;
-    const int shift = a.fec_shift ? __ldg(a.fec_shift + f % a.fecblocks) : 0;
-    __syncthreads();
-    {
-      // the BCH codeword (= the info bits of the LDPC codeword) as raw bytes, 16-byte asynchronous copies
-      const int n16 = (info_bytes + 15) >> 4;
-      const unsigned dst0 = (unsigned)__cvta_generic_to_shared(u);
-      for (int i = tid; i < n16; i += MAP_THREADS)
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(dst0 + 16u * i), "l"(in + 16 * i));
-      asm volatile("cp.async.commit_group;\n" ::);
-      asm volatile("cp.async.wait_group 0;\n" ::);
-    }
-    __syncthreads();
-    // ---- wrap-extended groups: 13 words = circular bits [0, 416) of each 360-bit group (see k_ldpc)
-    for (int idx = tid; idx < G * 13; idx += MAP_THREADS) {
-      const int g = idx / 13, w = idx - g * 13;
-      uint32_t v = be32_at_smem(u, 45 * g + (w == 12 ? 3 : 4 * w));
-      if (w == 11) v = (v & 0xFF000000u) | (be32_at_smem(u, 45 * g) >> 8);
-      ext[idx] = v;
-    }
-    __syncthreads();
-    // ---- pre-accumulator parity rows: R_t = XOR of rotated info groups
-    for (int idx = tid; idx < q * 12; idx += MAP_THREADS) {
-      const int t = idx / 12, w = idx - t * 12;
-      uint32_t acc = 0;
-      const int e1 = l.row_ptr[t + 1];
-      for (int e = l.row_ptr[t]; e < e1; e++) {
-        const uint32_t en = __ldg(l.entries + e);
-        int p = 32 * w - (int)(en >> 16);
-        if (p < 0) p += 360;
-        acc ^= window32(ext + (en & 0xffffu) * 13, p);
-      }
-      if (w == 11) acc &= 0xFF000000u;
-      rows[idx] = acc;
-    }
-    if (tid < 13) { rows[q * 12 + (tid < 12 ? tid : 0)] = 0u; s_E[12] = 0u; }
-    __syncthreads();
-    // ---- accumulator, part 1: T_t = XOR_{t' <= t} R_t' (prefix over rows, per word): ten row segments scanned side
-    // by side by 120 threads, then offset by the totals of the segments before them
-    const int seg_rows = (q + 9) / 10;
-    const int sw = tid % 12, sg = tid / 12;
-    const int t0 = sg * seg_rows, t1 = min(q, t0 + seg_rows);
-    if (tid < 120) {
-      uint32_t run = 0;
-      for (int t = t0; t < t1; t++) { run ^= rows[t * 12 + sw]; rows[t * 12 + sw] = run; }
-    }
-    __syncthreads();
-    uint32_t offs = 0;
-    if (tid < 120)
-      for (int s2 = 0; s2 < sg; s2++) {
-        const int last = min(q, (s2 + 1) * seg_rows) - 1;
-        if (last >= s2 * seg_rows) offs ^= rows[last * 12 + sw];
-      }
-    __syncthreads();
-    if (tid < 120 && offs)
-      for (int t = t0; t < t1; t++) rows[t * 12 + sw] ^= offs;
-    __syncthreads();
-    // ---- part 2: E = exclusive prefix-XOR along the 360 bit positions of T_{q-1} (first warp)
-    if (tid < 32) {
-      uint32_t x = lane < 12 ? rows[(q - 1) * 12 + lane] : 0;
-      x ^= x >> 1; x ^= x >> 2; x ^= x >> 4; x ^= x >> 8; x ^= x >> 16;   // inclusive, MSB first
-      uint32_t par = x & 1u, carry = par;
-#pragma unroll
-      for (int d = 1; d < 16; d <<= 1) {
-        const uint32_t o = __shfl_up_sync(0xffffffffu, carry, d);
-        if (lane >= d) carry ^= o;
-      }
-      carry ^= par;     // exclusive over words
-      uint32_t E = (x >> 1) ^ (carry ? 0xFFFFFFFFu : 0u);
-      if (lane == 11) E &= 0xFF000000u;
-      if (lane < 12) s_E[lane] = E;
-    }
-    __syncthreads();
-    // ---- parity rows (T_t ^ E) laid end to end behind the info bits, in raw byte order
-    if ((info_bytes & 3) == 0) {
-      uint32_t *pw = u + (info_bytes >> 2);
-      const int nwp = (q * 360) >> 5;
-      for (int j = tid; j < nwp; j += MAP_THREADS) {
-        const int P = j << 5;
-        const int t = P / 360, o = P - t * 360;
-        uint32_t v = window32(rows + t * 12, o) ^ window32(s_E, o);
-        const int n1 = 360 - o;                        // bits left in row t
-        if (n1 < 32) v = (v & ~(0xFFFFFFFFu >> n1)) | ((rows[(t + 1) * 12] ^ s_E[0]) >> n1);
-        pw[j] = bswap32(v);
-      }
-      uint8_t *ub = reinterpret_cast<uint8_t *>(u);
-      for (int b = (nwp << 2) + tid; b < q * 45; b += MAP_THREADS) {
-        const int t = b / 45, bb = b - t * 45;
-        ub[info_bytes + b] = (uint8_t)((rows[t * 12 + (bb >> 2)] ^ s_E[bb >> 2]) >> (24 - 8 * (bb & 3)));
-      }
-    }
-    else {
-      uint8_t *ub = reinterpret_cast<uint8_t *>(u);
-      for (int b = tid; b < q * 45; b += MAP_THREADS) {
-        const int t = b / 45, bb = b - t * 45;
-        ub[info_bytes + b] = (uint8_t)((rows[t * 12 + (bb >> 2)] ^ s_E[bb >> 2]) >> (24 - 8 * (bb & 3)));
-      }
-    }
-    if (tid < 4) u[4 * ((nwords + 3) >> 2) + tid] = 0u;
-    __syncthreads();
-    if (fec_tap) {        // parity-test tap of the codeword (not part of the product path)
-      uint32_t *o = reinterpret_cast<uint32_t *>(fec_tap + (long long)f * fec_tap_pitch);
-      for (int i = tid; i < (a.nldpc / 8 + 3) / 4; i += MAP_THREADS) o[i] = u[i];
-    }
-    map_body<false>(a, f, u, lut, cw, s_base, s_twist, shift);
-  }
-}
 
 void launch_map(const MapArgs &a, cudaStream_t s)
 {
@@ -1244,12 +999,7 @@ void launch_map(const MapArgs &a, cudaStream_t s)
   static bool attr[MAX_DEVICES], attr_q[MAX_DEVICES];
   allow_smem(k_map, 100 * 1024, attr);      // QPSK normal: 32400 cell codes
   allow_smem(k_map_qtr, 100 * 1024, attr_q);
-#ifdef MAP_QPSK_NO_TRANSPOSE
-  const bool qtr = false;
-#else
   const bool qtr = a.qpsk_par_q > 0 && a.mod == 2 && a.ncol == 0 && (a.cell_size & 3) == 0;
-#endif
-#ifndef MAP_NO_NCOL_TEMPLATE
   if (!qtr && (a.ncol == 8 || a.ncol == 12 || a.ncol == 16)) {
     MapArgs b = a;
     const int rows = a.nldpc / a.ncol;
@@ -1265,20 +1015,8 @@ void launch_map(const MapArgs &a, cudaStream_t s)
     count_launch();
     return;
   }
-#endif
   if (qtr) k_map_qtr<<<blocks, MAP_THREADS, smem, s>>>(a);
   else k_map<<<blocks, MAP_THREADS, smem, s>>>(a);
-  count_launch();
-}
-
-void launch_fec(const LdpcArgs &l, const MapArgs &a, uint8_t *fec_tap, int fec_tap_pitch, cudaStream_t s)
-{
-  if (l.frames < 1) return;
-  const size_t smem = (size_t)map_u_words(a.nldpc) * 4 + (size_t)(1 << a.mod) * 8 + 2 * (size_t)((map_cw_halfwords(a.cell_size) + 1) & ~1) +
-                      (size_t)(l.groups * 13 + l.q * 12 + 12 + 16) * 4;
-  static bool attr[MAX_DEVICES];
-  allow_smem(k_fec, 160 * 1024, attr);
-  k_fec<<<l.frames, MAP_THREADS, smem, s>>>(l, a, fec_tap, fec_tap_pitch);      // one FECFRAME per CTA
   count_launch();
 }
 
@@ -1573,10 +1311,7 @@ __global__ void __launch_bounds__(256) k_gather(const GatherArgs a)
 void launch_gather(const GatherArgs &a, cudaStream_t s)
 {
   if (a.frames < 1 || a.n < 1) return;
-#ifndef GATHER_FPB
-#define GATHER_FPB 4
-#endif
-  constexpr int FPB = GATHER_FPB;
+  constexpr int FPB = 4;
   const int npair = a.n >> 1;
   int gx = (npair + 255) / 256;
   if (gx < 1) gx = 1;
@@ -1603,8 +1338,8 @@ void launch_gather(const GatherArgs &a, cudaStream_t s)
 // elements for every access pattern used, with compile-time address offsets inside a butterfly.
 //
 // N = 32K does not fit (256 KB): it is split by bin parity (decimation in time at the top level):
-// phase 0 transforms the even bins and stores E[n] to out[n] and out[n + N/2]; phase 1 transforms the
-// odd bins and adds / subtracts W_N^n O[n] in place (the same thread re-reads what it wrote, from L2).
+// phase 0 transforms the even bins and parks E[n] in tensor memory, in the slots of the thread that
+// produced it; phase 1 transforms the odd bins and stores E[n] +/- W_N^n O[n] to out[n] and out[n + N/2].
 // Each carrier is gathered exactly once and every global store is a full, contiguous line.
 
 // Shared-memory layout of the transform: point p lives at float2 index padx(p) = p + p / 16 (one spare slot per 16).
@@ -1673,19 +1408,17 @@ __device__ __forceinline__ void apply_twiddles(float2 (&v)[R], float2 w1)
 }
 
 // one in-place DIT pass of radix 16 over M points; NPREV = length of the already transformed sub-blocks
-// PRE: the twiddle base W^i of the thread's butterflies (i = threadIdx.x mod NPREV, the same for every u when T is a
-// multiple of NPREV) was loaded once by the caller and is passed in `wpre`
-template <int M, int NPREV, int T, bool PRE = false>
-__device__ __forceinline__ void fft_pass16(float2 *x, const float2 *__restrict__ tw, float2 wpre = make_float2(1.f, 0.f))
+// w1: the twiddle base W^i of the thread's butterflies (i = threadIdx.x mod NPREV, the same for every u because T is a
+// multiple of NPREV), loaded once by the caller
+template <int M, int NPREV, int T>
+__device__ __forceinline__ void fft_pass16(float2 *x, float2 w1)
 {
   constexpr int NB = M / 16;
-  constexpr int TW_STEP = M / (NPREV * 16);
-  static_assert(!PRE || T % NPREV == 0, "preloaded twiddle needs a thread-constant butterfly index");
+  static_assert(T % NPREV == 0, "the twiddle base needs a thread-constant butterfly index");
 #pragma unroll (NB / T == 2 ? 2 : 1)
   for (int u = threadIdx.x; u < NB; u += T) {
     const int i = u & (NPREV - 1);
     float2 *xb = x + padx((u - i) * 16 + i);
-    const float2 w1 = PRE ? wpre : __ldg(tw + i * TW_STEP);
     float2 v[16];
 #pragma unroll
     for (int qd = 0; qd < 16; qd++) v[qd] = xb[padx(qd * NPREV)];
@@ -1766,11 +1499,7 @@ __device__ __forceinline__ float2 w64(int k)
 // loads -- stored [quad][group][4] so that each load is contiguous across the warp
 int ofdm_table_index(int p, int log2_m)
 {
-#ifdef OFDM_4K_PLAIN_FILL
-  if (log2_m != 14) return p;
-#else
   if (log2_m != 14 && log2_m != 12) return p;       // the transforms whose fill carries a radix-16 first pass
-#endif
   const int g = p >> 4, q = (p >> 2) & 3, r = p & 3;
   return ((q << (log2_m - 4)) + g) * 4 + r;
 }
@@ -1823,12 +1552,8 @@ __device__ __forceinline__ void store_sample(short2 *p, int idx, float2 v)
 template <int LOG2M, int T>
 struct FillGeom {
   static constexpr int M = 1 << LOG2M;
-#ifdef OFDM_4K_PLAIN_FILL
-  static constexpr int R0 = LOG2M == 14 ? 16 : 1 << (LOG2M & 3);   // first radix (1 = no first pass)
-#else
   // 4K = 16 * 16 * 16: its first radix-16 pass (no twiddles) rides in the fill as well, like the 16K sub-transform's
   static constexpr int R0 = (LOG2M == 14 || LOG2M == 12) ? 16 : 1 << (LOG2M & 3);   // first radix (1 = no first pass)
-#endif
   static constexpr int GROUPS = M / R0;             // first-pass butterflies
   static constexpr int INFL = LOG2M == 14 ? 16 : 8; // positions in flight per thread (16 where 128 registers are available)
   static constexpr int GPB0 = R0 >= INFL ? 1 : INFL / R0; // groups gathered per batch
@@ -1887,9 +1612,7 @@ struct FillSmem {
 // the codes of batch n + 1 are fetched while batch n is processed.
 template <int LOG2M, int T, bool C16, bool POOL, bool SINC>
 __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__ code, const float *__restrict__ sinc,
-                                          int (&c)[FillGeom<LOG2M, T>::GPB][FillGeom<LOG2M, T>::R0],
-                                          const uint8_t *stage, const float *lut_re, const float *lut_im, int lut_rep_shift,
-                                          const uint8_t *spool_m8, const float2 *__restrict__ cells,
+                                          int (&c)[FillGeom<LOG2M, T>::GPB][FillGeom<LOG2M, T>::R0], const float2 *__restrict__ cells,
                                           const float2 *__restrict__ pool, const FillSmem fs, int stage_cap_dbg = 0)
 {
   typedef FillGeom<LOG2M, T> G;
@@ -1907,7 +1630,6 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
           // small pool cell (null, pilots): (p + 1) << 17 -> spool[p]; big pool cell: sign bit set (POOL symbols only)
           const unsigned off = POOL && cc < 0 ? 0u : (unsigned)cc & 0x1FFFFu;
           BND(cc < 0 || cc >= 0x20000 || off + 2 <= 2u * (unsigned)stage_cap_dbg);
-#ifndef OFDM_FILL_GENERIC
           // explicit 32-bit shared-window addresses (one base register + the lane's table column): the generic-pointer
           // form made the compiler rebuild the window base and the lane offset for every carrier (≈ 10 instructions)
           unsigned sc;
@@ -1918,15 +1640,6 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
           asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.x) : "r"(fs.lut_lane_s + ((sc & 255u) << fs.esh)));
           asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.y) : "r"(fs.lut_lane_s + fs.im_ofs + ((sc >> 8) << fs.esh)));
           if (cc >= 0x20000) asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(val.x), "=f"(val.y) : "r"(fs.spool_m8_s + ((unsigned)cc >> 14)));
-#else
-          const unsigned sc = *reinterpret_cast<const uint16_t *>(stage + off);
-          // the LUTs are replicated 2^lut_rep_shift times (entry e, copy c at e * copies + c) and a lane reads copy
-          // lane mod copies: with 16 copies only lanes l and l + 16 can collide (2 wavefronts instead of ~3.4)
-          const unsigned esh = 2 + lut_rep_shift, emask = 255u << esh, lane_off = (threadIdx.x & ((1u << lut_rep_shift) - 1u)) << 2;
-          float2 val = make_float2(*reinterpret_cast<const float *>(reinterpret_cast<const uint8_t *>(lut_re) + (((sc << esh) & emask) | lane_off)),
-                                   *reinterpret_cast<const float *>(reinterpret_cast<const uint8_t *>(lut_im) + ((((sc >> 8) << esh) & emask) | lane_off)));
-          if (cc >= 0x20000) val = *reinterpret_cast<const float2 *>(spool_m8 + ((unsigned)cc >> 14));
-#endif
           if (POOL && cc < 0) val = __ldg(pool + (cc & 0x7FFFFFFF));
           v[b][r] = val;
         }
@@ -2076,15 +1789,12 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
   // smaller transforms with at most one butterfly per thread and pass (M / 16 <= T): the thread's twiddle base of every
   // pass is the same for every symbol -- loaded once here instead of at the head of each pass, where the load's
   // latency was exposed (13 % of the 8K kernel's stall samples)
-  constexpr bool PRETW = !REGTW && (M / 16 <= T);
+  static_assert(REGTW || M / 16 <= T, "one butterfly per thread and pass: the twiddle bases are loaded once");
   constexpr int NP1 = R0, NP2 = R0 * 16 < NLAST ? R0 * 16 : 1;       // NPREV of the middle passes (see below)
-  (void)NP1; (void)NP2;
-  if (PRETW) {
-#ifndef OFDM_NO_PRETW
+  if (!REGTW) {
     tw_p1 = __ldg(a.tw + (threadIdx.x & (NP1 - 1)) * (M / (NP1 * 16)));
     tw_p2 = __ldg(a.tw + (threadIdx.x & (NP2 - 1)) * (M / (NP2 * 16)));
     tw_last = (int)threadIdx.x < NLAST ? __ldg(a.tw + threadIdx.x) : make_float2(1.f, 0.f);
-#endif
   }
 
   // C16: the cells of symbol `u` go to the staging area by bulk asynchronous copies (TMA, cp.async.bulk): one copy
@@ -2179,19 +1889,18 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
     for (int phase = 0; phase < SPLIT; phase++) {
       const int32_t *code = a.code_pos + ((long long)l * SPLIT + phase) * M;
       const float *sinc = a.sinc_pos ? a.sinc_pos + (long long)phase * M : nullptr;
-      const uint8_t *spool_m8 = reinterpret_cast<const uint8_t *>(spool) - 8;
       if (phase) fill_load_codes<LOG2M, T>(code, threadIdx.x, c);
       __syncthreads();      // staging area landed (phase 0) / previous phase has finished reading x
       // every thread is past its reads of the descriptor buffer: the next symbol's list may come in
       if (C16 && phase == 0 && threadIdx.x == 0 && unit + (int)gridDim.x < units) desc_issue(cp1);
       // ---- 1. carrier fill (+ first pass)
       if (sinc) {
-        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, true>(x, code, sinc, c, stage, lut_re, lut_im, lut_rep_shift, spool_m8, cells, pool, fs, a.stage_cap);
-        else ofdm_fill<LOG2M, T, C16, false, true>(x, code, sinc, c, stage, lut_re, lut_im, lut_rep_shift, spool_m8, cells, pool, fs, a.stage_cap);
+        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, true>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
+        else ofdm_fill<LOG2M, T, C16, false, true>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
       }
       else {
-        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, false>(x, code, sinc, c, stage, lut_re, lut_im, lut_rep_shift, spool_m8, cells, pool, fs, a.stage_cap);
-        else ofdm_fill<LOG2M, T, C16, false, false>(x, code, sinc, c, stage, lut_re, lut_im, lut_rep_shift, spool_m8, cells, pool, fs, a.stage_cap);
+        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, false>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
+        else ofdm_fill<LOG2M, T, C16, false, false>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
       }
       __syncthreads();
       // every fill of the symbol has read its cells: the next symbol's cells may replace them (under the passes)
@@ -2201,22 +1910,12 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
       }
       // ---- 2. middle radix-16 passes
       if constexpr (REGTW) {
-#ifdef OFDM_PASS_TREE
-        fft_pass16<M, 16, T, REGTW>(x, a.tw, tw_p1); __syncthreads();
-        fft_pass16<M, 256, T, REGTW>(x, a.tw, tw_p2); __syncthreads();
-#else
         fft_pass16x2<M, 16, T>(x, tw_p1); __syncthreads();
         fft_pass16x2<M, 256, T>(x, tw_p2); __syncthreads();
-#endif
       }
       else {
-#ifndef OFDM_NO_PRETW
-        if (R0 * 16 < NLAST * 16 && R0 < NLAST) { fft_pass16<M, NP1, T, PRETW>(x, a.tw, tw_p1); __syncthreads(); }
-        if (R0 * 16 < NLAST) { fft_pass16<M, NP2, T, PRETW>(x, a.tw, tw_p2); __syncthreads(); }
-#else
-        if (R0 * 16 < NLAST * 16 && R0 < NLAST) { fft_pass16<M, R0, T>(x, a.tw); __syncthreads(); }
-        if (R0 * 16 < NLAST) { fft_pass16<M, (R0 * 16 < NLAST ? R0 * 16 : 1), T>(x, a.tw); __syncthreads(); }
-#endif
+        if (R0 * 16 < NLAST * 16 && R0 < NLAST) { fft_pass16<M, NP1, T>(x, tw_p1); __syncthreads(); }
+        if (R0 * 16 < NLAST) { fft_pass16<M, NP2, T>(x, tw_p2); __syncthreads(); }
       }
       // ---- 3. last pass fused with scale + store (+ cyclic prefix, + 32K recombination)
       if constexpr (REGTW) {
@@ -2280,15 +1979,10 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
 #pragma unroll 1
       for (int i = threadIdx.x; i < NLAST; i += T) {
         const float2 *xb = x + padx(i);
-#ifndef OFDM_NO_PRETW
-        const float2 w1 = PRETW ? tw_last : __ldg(a.tw + i);      // TW_STEP = M / (NLAST * 16) = 1
-#else
-        const float2 w1 = __ldg(a.tw + i);      // TW_STEP = M / (NLAST * 16) = 1
-#endif
         float2 v[16];
 #pragma unroll
         for (int qd = 0; qd < 16; qd++) v[qd] = xb[padx(qd * NLAST)];
-        apply_twiddles<16>(v, w1);
+        apply_twiddles<16>(v, tw_last);
         dft_reg<16>(v);
         // sample t = i + k NLAST: one 64-bit base per destination, compile-time offsets k NLAST
         sample_t *o = sym + a.gi + i;

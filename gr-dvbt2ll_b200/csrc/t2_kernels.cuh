@@ -18,9 +18,7 @@ struct BbArgs {
   int kbch, nbch, bch_r, payload_bytes, mode, inband, fecblocks;
   int chunk_bytes, lead_zero_bytes;
   const uint8_t *scramble;    // kbch / 8
-  const uint8_t *crc8_tab;    // 4 * 256: slicing-by-4 tables S1..S4 (S1 = the plain byte table)
-  uint32_t crc8_mask[8];      // bit k of the CRC-8 after the four bytes of little-endian word t (state XORed into the
-                              // first byte) = parity(t & crc8_mask[k])
+  const uint8_t *crc8_tab;    // 256: the CRC-8 byte table (BB header)
   // The CRC-8 of a 187-byte packet read as 47 little-endian words (one leading byte, zeroed by the masks) is linear in
   // the data: bit k = parity(XOR_j word_j & crc8_pos_mask[j][k]).  Kernel parameters live in the constant bank, so
   // with the loop unrolled every mask is an instruction operand: one AND-XOR per word and CRC bit, no look-ups.
@@ -92,9 +90,6 @@ struct MapArgs {
   long long in_len, out_len; // bytes behind in, cells behind out / out16 (debug build bounds checks; 0 = not checked)
 };
 void launch_map(const MapArgs &a, cudaStream_t s);
-// K2 + K3 fused, one FECFRAME per CTA: l.in = packed BCH codewords (l.out unused), a = mapper arguments (a.in unused);
-// fec_tap != NULL additionally stores the packed "u"-order LDPC codewords (parity tests only)
-void launch_fec(const LdpcArgs &l, const MapArgs &a, uint8_t *fec_tap, int fec_tap_pitch, cudaStream_t s);
 
 // ---- bit format helpers for the drop-in blocks (1 bit per byte <-> packed) ------------------------
 // pack: in = frames * nbits bytes (0/1) -> out packed with pitch

@@ -37,7 +37,6 @@ EXPORTED_SYMBOLS = [
     "dvbt2ll_copy_to_host", "dvbt2ll_copy_to_device", "dvbt2ll_device_alloc", "dvbt2ll_device_free",
     "dvbt2ll_device_count", "dvbt2ll_set_device", "dvbt2ll_device_synchronize",
     "dvbt2ll_stream_create", "dvbt2ll_stream_destroy", "dvbt2ll_stream_synchronize",
-    "dvbt2ll_chain_enable_taps", "dvbt2ll_chain_fused_fec",
     "dvbt2ll_chain_create_multiplp", "dvbt2ll_chain_num_plp", "dvbt2ll_chain_plp_ts_bytes",
     "dvbt2ll_chain_history_bytes", "dvbt2ll_ts_sync", "dvbt2ll_ts_fill",
 ]
@@ -131,9 +130,6 @@ def lib():
         L.dvbt2ll_stream_destroy.argtypes = [vp]
         L.dvbt2ll_stream_destroy.restype = None
         L.dvbt2ll_stream_synchronize.argtypes = [vp]
-        L.dvbt2ll_chain_enable_taps.argtypes = [vp, ci]
-        L.dvbt2ll_chain_enable_taps.restype = None
-        L.dvbt2ll_chain_fused_fec.argtypes = [vp]
         L.dvbt2ll_chain_create_multiplp.restype = vp
         L.dvbt2ll_chain_create_multiplp.argtypes = [C.POINTER(ChainParams), ci, C.POINTER(ci), ci, ci]
         L.dvbt2ll_chain_num_plp.argtypes = [vp]
@@ -470,14 +466,6 @@ class Chain(_Block):
         lib().dvbt2ll_chain_tap(self._h, stage.encode(), buf.ctypes.data, n)
         return buf.view(dtype)
 
-    def enable_taps(self, on=True):
-        """Keep the packed LDPC codewords of the next runs for tap("fec") (the fused kernel otherwise keeps them on chip)."""
-        lib().dvbt2ll_chain_enable_taps(self._h, 1 if on else 0)
-
-    @property
-    def fused_fec(self):
-        return bool(lib().dvbt2ll_chain_fused_fec(self._h))
-
     def enable_timing(self, on=True):
         lib().dvbt2ll_chain_enable_timing(self._h, 1 if on else 0)
 
@@ -486,11 +474,7 @@ class Chain(_Block):
         r = lib().dvbt2ll_chain_stage_ms(self._h, ms)
         if r < 0:
             raise RuntimeError(last_error())
-        d = dict(zip(("bb_bch", "ldpc", "map", "ofdm", "total"), [float(x) for x in ms]))
-        if self.fused_fec:            # one kernel: LDPC + bit interleaver / mapper
-            d["ldpc_map"] = d.pop("map")
-            d.pop("ldpc")
-        return d
+        return dict(zip(("bb_bch", "ldpc", "map", "ofdm", "total"), [float(x) for x in ms]))
 
 
 def ts_sync(ts):

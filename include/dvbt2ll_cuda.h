@@ -146,12 +146,6 @@ DVBT2LL_API_EXPORT int dvbt2ll_chain_set_sink(dvbt2ll_handle *h, int format, flo
  * word supplying the imaginary part << 8, frame stride padded to a multiple of 4 cells).  Copies to HOST; returns
  * bytes or negative error. */
 DVBT2LL_API_EXPORT long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, long long cap);
-/* With DVBT2LL_FUSE_FEC=1 the chain runs LDPC and the bit interleaver / mapper as one kernel and the packed LDPC
- * codewords never reach HBM; enable the taps before a run to have them stored for dvbt2ll_chain_tap("fec") as well. */
-DVBT2LL_API_EXPORT void dvbt2ll_chain_enable_taps(dvbt2ll_handle *h, int on);
-/* 1 when LDPC + mapper run as one kernel (DVBT2LL_FUSE_FEC=1 in the environment; two kernels by default): then
- * dvbt2ll_chain_stage_ms reports that kernel under "map" and 0 under "ldpc". */
-DVBT2LL_API_EXPORT int dvbt2ll_chain_fused_fec(const dvbt2ll_handle *h);
 /* Device time in ms of each stage kernel (bb_bch, ldpc, map, ofdm, total), averaged over the chain runs issued since
  * timing was enabled (at most the last 64); events are recorded per run, so the caller's timed loop needs no sync. */
 DVBT2LL_API_EXPORT int dvbt2ll_chain_stage_ms(dvbt2ll_handle *h, float *ms5);

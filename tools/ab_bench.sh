@@ -7,7 +7,7 @@ for round in 1 2; do
 import json,sys
 try:
     d=json.loads(sys.stdin.read()); s=d['roofline']['stage_ms']
-    print('$v', '$DVBT2LL_FUSE_FEC', round(d['ms_per_step'],4), {k:round(x,4) for k,x in s.items()})
+    print('$v', round(d['ms_per_step'],4), {k:round(x,4) for k,x in s.items()})
 except Exception as e:
     print('$v', 'FAILED', e)"
   done
