@@ -7,8 +7,10 @@
 // dvbt2ll_ts_fill) -- what a rate-adapting source does when the multiplex runs dry.  Frames are modulated in batches
 // of `batch` T2 frames per call (stream position carried by first_frame + the 187 history bytes in front of a batch).
 //
-// usage: t2_file_modulator [--config c1|c2|c3|c4] [--plp-blocks a,b,..] [--frames N] [--batch B] [--sc16 GAIN]
-//                          --out FILE  TS_FILE [TS_FILE ...]
+// usage: t2_file_modulator [--config c1|c2|c3|c4] [--plp-blocks a,b,..] [--plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]]...
+//                          [--frames N] [--batch B] [--sc16 GAIN] --out FILE  TS_FILE [TS_FILE ...]
+// --plp, once per PLP: its FEC blocks per T2 frame and, optionally, its own FEC type, code rate, constellation and
+// rotation (enum values of dvbt2ll_config.h; the config's where omitted).
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -52,6 +54,8 @@ int main(int argc, char **argv)
 {
   std::string cfg = "c1", out_path;
   std::vector<int> plp_blocks;
+  std::vector<dvbt2ll_plp_params> plps;
+  std::vector<int> plp_own;          // --plp entries that name their own parameters
   std::vector<const char *> inputs;
   int frames = -1, batch = 4, sc16 = 0;
   float gain = 1.0f;
@@ -65,16 +69,33 @@ int main(int argc, char **argv)
     else if (a == "--plp-blocks" && i + 1 < argc) {
       for (char *t = std::strtok(argv[++i], ","); t; t = std::strtok(0, ",")) plp_blocks.push_back(std::atoi(t));
     }
+    else if (a == "--plp" && i + 1 < argc) {
+      int v[5] = { 0, -1, -1, -1, -1 };
+      const int n = std::sscanf(argv[++i], "%d:%d:%d:%d:%d", &v[0], &v[1], &v[2], &v[3], &v[4]);
+      if (n != 1 && n != 5) { std::fprintf(stderr, "--plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]\n"); return 2; }
+      dvbt2ll_plp_params q = { v[0], v[1], v[2], v[3], v[4] };
+      plps.push_back(q);
+      plp_own.push_back(n == 5);
+    }
     else inputs.push_back(argv[i]);
   }
   dvbt2ll_chain_params prm;
-  if (!named_config(cfg, &prm) || out_path.empty() || inputs.empty() || batch < 1) {
-    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,..] [--frames N] [--batch B] [--sc16 GAIN] --out FILE TS_FILE...\n", argv[0]);
+  if (!named_config(cfg, &prm) || out_path.empty() || inputs.empty() || batch < 1 || (!plps.empty() && !plp_blocks.empty())) {
+    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--frames N] [--batch B] [--sc16 GAIN] --out FILE TS_FILE...\n", argv[0]);
     return 2;
   }
-  const int P = plp_blocks.empty() ? 1 : (int)plp_blocks.size();
+  bool own = false;
+  for (size_t p = 0; p < plps.size(); p++) {
+    if (plp_own[p]) { own = true; continue; }
+    plps[p].framesize = prm.framesize; plps[p].rate = prm.rate; plps[p].constellation = prm.constellation; plps[p].rotation = prm.rotation;
+  }
+  if (!own)
+    for (size_t p = 0; p < plps.size(); p++) plp_blocks.push_back(plps[p].fecblocks);
+  const int P = own ? (int)plps.size() : plp_blocks.empty() ? 1 : (int)plp_blocks.size();
   if ((int)inputs.size() != P) { std::fprintf(stderr, "one TS file per PLP expected (%d)\n", P); return 2; }
-  dvbt2ll_handle *h = P == 1 ? dvbt2ll_chain_create(&prm, batch, -1) : dvbt2ll_chain_create_multiplp(&prm, P, plp_blocks.data(), batch, -1);
+  if (P == 1 && !own && !plps.empty()) prm.fecblocks = plps[0].fecblocks;
+  dvbt2ll_handle *h = own ? dvbt2ll_chain_create_plps(&prm, P, plps.data(), batch, -1)
+                    : P == 1 ? dvbt2ll_chain_create(&prm, batch, -1) : dvbt2ll_chain_create_multiplp(&prm, P, plp_blocks.data(), batch, -1);
   if (!h) { std::fprintf(stderr, "chain: %s\n", dvbt2ll_last_error()); return 1; }
   if (sc16 && dvbt2ll_chain_set_sink(h, 1, gain) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }
 

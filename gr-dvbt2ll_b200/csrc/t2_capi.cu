@@ -661,11 +661,12 @@ struct OfdmDevice {
   DevBuf d_code, d_pool, d_p1, d_sinc, d_tw, d_tw_split, d_sym_flags;
   int log2_m, split;
   long long pool_stride;
-  // c16: `code` holds staging slots (chain mode, 16-bit cells) and is re-encoded for the kernel's branch-free fill:
-  //   data carrier         -> 2 * slot            (byte offset into the staging area, < 131072)
-  //   small pool cell p<8  -> (p + 1) << 17       (zero / pilot amplitudes, kept in shared memory)
-  //   other pool cell      -> 0x80000000 | index  (L1 signalling, dummy cells; symbols holding any are flagged)
-  int init(const std::vector<int32_t> &code, const t2::CellPool &pool, const t2::OfdmPlan &op, bool c16 = false)
+  // c16: `code` holds staging slots (chain mode, 16-bit cells) and is re-encoded as the chain-mode carrier codes of
+  // t2_kernels.cuh (2 * slot | (small pool cell + 1) << 17 | 0x80000000 + pool cell) for the kernel's branch-free fill;
+  // with tab_base (several constellation tables) a data carrier's code also carries the first table entry of its cell's
+  // PLP, tab_base[plp[carrier]] << OFDM_CODE_TAB_SHIFT
+  int init(const std::vector<int32_t> &code, const t2::CellPool &pool, const t2::OfdmPlan &op, bool c16 = false,
+           const std::vector<uint8_t> *plp = 0, const int *tab_base = 0)
   {
     // one copy of the pool per L1-post variant: in copy v the L1-post slot holds variant v, so the kernel
     // selects a pool base per frame instead of patching indices per cell
@@ -704,6 +705,7 @@ struct OfdmDevice {
             if (v >= 0) {
               if (v >= 65536) return fail(DVBT2LL_ERR_INVALID, "chain: staging slot out of range");
               v = 2 * v;
+              if (tab_base) v |= tab_base[(*plp)[(size_t)l * cps + k]] << t2k::OFDM_CODE_TAB_SHIFT;
             }
             else if (~v < 8) v = (~v + 1) << 17;
             else { v = (int32_t)(0x80000000u | (uint32_t)(~v)); sym_flags[l] = 1; }
@@ -735,6 +737,7 @@ struct OfdmDevice {
     a.sym_flags = d_sym_flags.as<int32_t>();
     a.out_fmt = 0; a.sink_gain = 1.0f;
     a.cells_len = 0; a.out_len = 0; a.pool_len = pool_stride;
+    a.lut_tables = 1;
   }
 };
 
@@ -785,10 +788,39 @@ struct OfdmHandle : dvbt2ll_handle {
 };
 
 // ================================================================================================
+// the same table shifted by 0..3 entries: four consecutive entries at any phase become one aligned 8-byte load
+std::vector<uint16_t> make_ci_inv4(const std::vector<uint16_t> &ci_inv, int *stride)
+{
+  const int nc = (int)ci_inv.size();
+  *stride = (nc + 8 + 3) & ~3;
+  std::vector<uint16_t> c4((size_t)4 * *stride, 0);
+  for (int k = 0; k < 4; k++)
+    for (int j = 0; j + k < nc; j++) {
+      const int c = ci_inv[j + k];
+      c4[(size_t)k * *stride + j] = (uint16_t)(c + 2 * (c >> 6));      // index in the kernel's padded code array
+    }
+  return c4;
+}
+
 struct ChainHandle : dvbt2ll_handle {
+  // the stages of PLP parameter set 0 (every PLP's, unless the PLPs have their own parameters)
   BbHandle bb;
   LdpcHandle ldpc;
   MapHandle map;
+  // PLPs with their own parameters (dvbt2ll_chain_create_plps) and more than one set of them (fplan.plp_sets > 1): the
+  // stages of sets 1.., one launch per PLP and stage; the BCH / FEC buffers are PLP-major (PLP p's region holds its
+  // codewords [channel][frame][block] at its own pitch), the 16-bit cells of PLP p start at fplan.plp_chain_off[p]
+  struct Set { BbHandle bb; LdpcHandle ldpc; MapHandle map; };
+  std::unique_ptr<Set> xset[t2::MAX_PLP];
+  DevBuf d_ci_inv_p[t2::MAX_PLP], d_ci_inv4_p[t2::MAX_PLP];
+  int ci4_stride_p[t2::MAX_PLP];
+  size_t bch_off[t2::MAX_PLP + 1], fec_off[t2::MAX_PLP + 1];   // byte offsets of the PLP regions
+  // constellation tables of the OFDM fill: one per distinct (constellation, rotation), the largest first; PLP p's
+  // starts at entry lut_base[p].  One table: the set-0 mapper's.
+  std::vector<t2::cfloat> luts;
+  int lut_tables, lut_base[t2::MAX_PLP], lut_single;
+  int lut_copies;      // copies of the table(s) k_ofdm kept in shared memory in the last run
+  DevBuf d_luts;
   t2::FramePlan fplan;
   t2::OfdmPlan oplan;
   t2::Chain16Tables tables;
@@ -805,7 +837,7 @@ struct ChainHandle : dvbt2ll_handle {
   enum { TIMING_SLOTS = 64 };
   cudaEvent_t ev[TIMING_SLOTS][5];     // per-run event sets so the timed loop never has to synchronise
   long long n_timed;
-  ChainHandle() : dvbt2ll_handle(CHAIN), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), last_frames(0), next_frame(0), timing(false)
+  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), last_frames(0), next_frame(0), timing(false)
   {
     n_timed = 0;
     for (int s = 0; s < TIMING_SLOTS; s++) for (int i = 0; i < 5; i++) ev[s][i] = 0;
@@ -822,11 +854,18 @@ struct ChainHandle : dvbt2ll_handle {
     if (device >= 0) CK(cudaSetDevice(device));
     return ensure_device();
   }
+  bool mixed() const { return fplan.plp_sets > 1; }
+  BbHandle &bb_of(int plp) { const int s = fplan.plp_set[plp]; return s ? xset[s]->bb : bb; }
+  const BbHandle &bb_of(int plp) const { const int s = fplan.plp_set[plp]; return s ? xset[s]->bb : bb; }
+  LdpcHandle &ldpc_of(int plp) { const int s = fplan.plp_set[plp]; return s ? xset[s]->ldpc : ldpc; }
+  MapHandle &map_of(int plp) { const int s = fplan.plp_set[plp]; return s ? xset[s]->map : map; }
+  int bch_pitch(int plp) const { return align16(bb_of(plp).plan.fec.nbch / 8); }
+  int fec_pitch(int plp) const { return align16(bb_of(plp).plan.fec.nldpc / 8); }
   int F() const { return fplan.prm.fecblocks; }
   int P() const { return fplan.num_plp; }
   int Fp(int plp) const { return fplan.plp_first_block[plp + 1] - fplan.plp_first_block[plp]; }
   // cells per T2 frame in the 16-bit cell memory, padded so every frame starts on a 16-byte boundary (bulk copies)
-  long long cells16_stride() const { return ((long long)F() * map.plan.cell_size + 7) & ~7LL; }
+  long long cells16_stride() const { return ((long long)fplan.plp_chain_off[P()] + 7) & ~7LL; }
   // TS byte index (per channel, stream starts on a packet boundary) at which T2 frame `frame` begins
   long long stream_pos(long long frame, int plp = 0) const
   {
@@ -834,7 +873,7 @@ struct ChainHandle : dvbt2ll_handle {
     const long long j0 = frame * fpl;
     long long nb0 = 0;
     if (bb.plan.inband) nb0 = (j0 + fpl - 1) / fpl;
-    const long long P = j0 * bb.plan.payload_bytes - 13 * nb0;          // payload bytes before the frame
+    const long long P = j0 * bb_of(plp).plan.payload_bytes - 13 * nb0;  // payload bytes before the frame
     if (bb.plan.mode == t2::INPUTMODE_NORMAL || P == 0) return P;
     const long long last = P - 1;                                       // high efficiency mode: sync bytes are skipped,
     return 1 + last + last / 187 + 1;                                   // packets = 1 sync + 187 payload bytes
@@ -858,19 +897,20 @@ struct ChainHandle : dvbt2ll_handle {
     if ((r = bb.dev_init())) return r;
     if ((r = ldpc.dev_init())) return r;
     if ((r = map.dev_init())) return r;
-    if ((r = odev.init(tables.code, tables.pool, oplan, true))) return r;
+    for (int s = 1; s < fplan.plp_sets; s++) {
+      Set &x = *xset[s];
+      x.bb.stream = 0; x.ldpc.stream = 0; x.map.stream = 0;
+      if ((r = x.bb.dev_init()) || (r = x.ldpc.dev_init()) || (r = x.map.dev_init())) return r;
+    }
+    if ((r = odev.init(tables.code, tables.pool, oplan, true, &tables.plp, lut_tables > 1 ? lut_base : 0))) return r;
     CK(upload(d_ci_inv, fplan.cell_perm_inv));
-    {
-      // the same table shifted by 0..3 entries: four consecutive entries at any phase become one aligned 8-byte load
-      const int nc = (int)fplan.cell_perm_inv.size();
-      ci4_stride = (nc + 8 + 3) & ~3;
-      std::vector<uint16_t> c4((size_t)4 * ci4_stride, 0);
-      for (int k = 0; k < 4; k++)
-        for (int j = 0; j + k < nc; j++) {
-          const int c = fplan.cell_perm_inv[j + k];
-          c4[(size_t)k * ci4_stride + j] = (uint16_t)(c + 2 * (c >> 6));      // index in the kernel's padded code array
-        }
-      CK(upload(d_ci_inv4, c4));
+    CK(upload(d_ci_inv4, make_ci_inv4(fplan.cell_perm_inv, &ci4_stride)));
+    if (mixed()) {
+      for (int pl = 0; pl < P(); pl++) {
+        CK(upload(d_ci_inv_p[pl], fplan.plp_cell_perm_inv[pl]));
+        CK(upload(d_ci_inv4_p[pl], make_ci_inv4(fplan.plp_cell_perm_inv[pl], &ci4_stride_p[pl])));
+      }
+      CK(upload(d_luts, luts));
     }
     CK(upload(d_fec_shift, fplan.fec_shift));
     CK(upload(d_run_desc, tables.run_desc));
@@ -881,7 +921,16 @@ struct ChainHandle : dvbt2ll_handle {
     if ((size_t)(1 << odev.log2_m) * 8 * 17 / 16 + (size_t)stage_cap * 2 + 2048 + 96 + (size_t)(tables.max_runs + 2) * 8 > 227 * 1024)
       return fail(DVBT2LL_ERR_INVALID, "chain: the cells of one OFDM symbol do not fit the shared-memory staging area");
     const size_t nfec = (size_t)max_frames * F();
-    CK(d_bch.ensure(nfec * align16(bb.plan.fec.nbch / 8) + 64));
+    bch_off[0] = fec_off[0] = 0;
+    for (int pl = 0; pl < P(); pl++) {
+      bch_off[pl + 1] = bch_off[pl] + (size_t)max_frames * Fp(pl) * bch_pitch(pl);
+      fec_off[pl + 1] = fec_off[pl] + (size_t)max_frames * Fp(pl) * fec_pitch(pl);
+    }
+    if (mixed()) {
+      CK(d_bch.ensure(bch_off[P()] + 64));
+      CK(d_fec.ensure(fec_off[P()] + 64));
+    }
+    else CK(d_bch.ensure(nfec * align16(bb.plan.fec.nbch / 8) + 64));
     CK(d_cells.ensure((size_t)max_frames * cells16_stride() * sizeof(uint16_t) + 64));   // 16-bit cell codes
     // the padding cells between frames and the slack behind the last one are never written by the mapper but travel
     // with the aligned bulk copies: give them a valid code once
@@ -902,9 +951,11 @@ struct ChainHandle : dvbt2ll_handle {
     cudaEvent_t *tev = ev[n_timed % TIMING_SLOTS];
     if (timing) cudaEventRecord(tev[0], s);
     uint8_t *bch_buf = d_bch.as<uint8_t>() + (size_t)buf_frame * F() * bp;
-    CK(d_fec.ensure((size_t)max_frames * F() * fp + 64));
+    if (!mixed()) CK(d_fec.ensure((size_t)max_frames * F() * fp + 64));      // (PLP-major buffers: sized at dev_init)
     uint8_t *fec_buf = d_fec.as<uint8_t>() + (size_t)buf_frame * F() * fp;
     uint16_t *cell_buf = d_cells.as<uint16_t>() + (size_t)buf_frame * cells16_stride();
+    if (mixed()) run_plps(d_ts, ts_pitch, n_channels, n_frames, first_frame, cell_buf, s, buf_frame, hist_valid, tev);
+    else {
     // BB framing + BCH, PLP by PLP: row c * P + p of the TS holds PLP p of channel c; every PLP has its own stream
     // position (packet phase, in-band cycle = its FEC blocks per frame), and its codewords go to their place inside
     // the frame's block list (streams begin on a packet boundary at frame 0)
@@ -935,6 +986,7 @@ struct ChainHandle : dvbt2ll_handle {
     if (timing) cudaEventRecord(tev[2], s);
     t2k::launch_map(ma, s);
     if (timing) cudaEventRecord(tev[3], s);
+    }
     t2k::OfdmArgs oa;
     odev.fill(oa, oplan, tables.pool);
     oa.cells = 0; oa.cells_stride = cells16_stride();
@@ -942,16 +994,56 @@ struct ChainHandle : dvbt2ll_handle {
     oa.run_cnt = d_run_cnt.as<int32_t>(); oa.desc_cap = (tables.max_runs + 2) & ~1;
     oa.stage_bytes = d_stage_bytes.as<int32_t>(); oa.stage_cap = stage_cap; oa.lut_single = map.plan.im_from_re;
     oa.lut = map.d_lut.as<float2>(); oa.lut_n = 1 << map.plan.mod;
+    if (mixed()) { oa.lut_single = lut_single; oa.lut = d_luts.as<float2>(); oa.lut_n = (int)luts.size(); oa.lut_tables = lut_tables; }
     oa.out = d_out; oa.out_stride = oplan.samples_per_frame;
     oa.cells_len = (long long)frames * cells16_stride(); oa.out_len = (long long)frames * oplan.samples_per_frame;
     oa.out_fmt = sink_fmt; oa.sink_gain = sink_gain; oa.norm = oplan.normalization * sink_gain;
     oa.frames = frames; oa.frames_per_channel = n_frames;
     oa.frame_idx0 = (int)(first_frame % (tables.pool.l1post_variants > 0 ? tables.pool.l1post_variants : 1));
-    t2k::launch_ofdm(oa, s);
+    lut_copies = t2k::launch_ofdm(oa, s);
     if (timing) { cudaEventRecord(tev[4], s); n_timed++; }
     CK(cudaGetLastError());
     if (buf_frame == 0) last_frames = frames;
     return frames;
+  }
+  // BB + BCH, LDPC and mapper of a chain whose PLPs have more than one parameter set: a launch per PLP and stage, each
+  // on the PLP's own contiguous regions of the BCH / FEC buffers and of the cell memory
+  void run_plps(const void *d_ts, long long ts_pitch, int n_channels, int n_frames, long long first_frame, uint16_t *cell_buf,
+                cudaStream_t s, int buf_frame, int hist_valid, cudaEvent_t *tev)
+  {
+    const int frames = n_channels * n_frames;
+    auto bch_buf = [&](int pl) { return d_bch.as<uint8_t>() + bch_off[pl] + (size_t)buf_frame * Fp(pl) * bch_pitch(pl); };
+    auto fec_buf = [&](int pl) { return d_fec.as<uint8_t>() + fec_off[pl] + (size_t)buf_frame * Fp(pl) * fec_pitch(pl); };
+    for (int pl = 0; pl < P(); pl++) {
+      const int fpl = Fp(pl);
+      const long long j0 = first_frame * fpl;
+      t2k::BbArgs ba;
+      bb_of(pl).fill_args(ba, (const uint8_t *)d_ts + (long long)pl * ts_pitch, ts_pitch * P(), n_channels, n_frames * fpl,
+                          (int)(stream_pos(first_frame, pl) % 188), bb.plan.inband ? (int)(j0 % fpl) : 0,
+                          hist_valid >= 0 ? hist_valid : (first_frame > 0 ? 1 : 0), bch_buf(pl), bch_pitch(pl));
+      ba.fecblocks = fpl;
+      ba.ts_len = ts_bytes(first_frame, n_frames, pl);
+      t2k::launch_bb_bch(ba, s);
+    }
+    if (timing) cudaEventRecord(tev[1], s);
+    for (int pl = 0; pl < P(); pl++) {
+      t2k::LdpcArgs la;
+      ldpc_of(pl).fill_args(la, bch_buf(pl), bch_pitch(pl), fec_buf(pl), fec_pitch(pl), frames * Fp(pl));
+      t2k::launch_ldpc(la, s);
+    }
+    if (timing) cudaEventRecord(tev[2], s);
+    for (int pl = 0; pl < P(); pl++) {
+      t2k::MapArgs ma;
+      map_of(pl).fill_args(ma, fec_buf(pl), fec_pitch(pl), 0, frames * Fp(pl));
+      ma.out16 = cell_buf + fplan.plp_chain_off[pl]; ma.out16_frame_stride = cells16_stride();
+      ma.ci_inv = d_ci_inv_p[pl].as<uint16_t>(); ma.fec_shift = d_fec_shift.as<int32_t>() + fplan.plp_first_block[pl];
+      ma.fecblocks = Fp(pl);
+      ma.ci_inv4 = d_ci_inv4_p[pl].as<uint16_t>(); ma.ci_inv4_stride = ci4_stride_p[pl];
+      ma.im_from_re = lut_single;      // the w~ codes only when the OFDM fill keeps the single-table form for every PLP
+      ma.out_len = (long long)frames * cells16_stride() - fplan.plp_chain_off[pl];
+      t2k::launch_map(ma, s);
+    }
+    if (timing) cudaEventRecord(tev[3], s);
   }
   int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
   {
@@ -992,6 +1084,20 @@ struct ChainHandle : dvbt2ll_handle {
       return copy_out(v, sizeof(int) * (3 + fplan.num_plp), out, cap);
     }
     if (n == "frame.fi_src") return copy_vec(fplan.fi_src, out, cap);
+    if (n == "frame.fec_shift") return copy_vec(fplan.fec_shift, out, cap);
+    if (n == "frame.plp_cells") {
+      // per PLP: cells per FECFRAME, first cell in the frame (PLP_START), first cell in the chain's cell memory
+      int v[3 * t2::MAX_PLP];
+      for (int i = 0; i < P(); i++) { v[3 * i] = fplan.plp_cell_size[i]; v[3 * i + 1] = fplan.plp_first_cell[i]; v[3 * i + 2] = fplan.plp_chain_off[i]; }
+      return copy_out(v, sizeof(int) * 3 * P(), out, cap);
+    }
+    if (n == "chain.luts") {
+      // constellation tables of the OFDM fill: { tables, single-table form, copies in shared memory in the last run
+      // (0 before any), first entry of each PLP's table }
+      int v[3 + t2::MAX_PLP] = { lut_tables, mixed() ? lut_single : map.plan.im_from_re, lut_copies };
+      for (int i = 0; i < P(); i++) v[3 + i] = mixed() ? lut_base[i] : 0;
+      return copy_out(v, sizeof(int) * (3 + P()), out, cap);
+    }
     long long r;
     if ((r = bb.plan_get(name, out, cap)) >= 0) return r;
     if ((r = ldpc.plan_get(name, out, cap)) >= 0) return r;
@@ -1409,6 +1515,74 @@ static dvbt2ll_handle *chain_create(const dvbt2ll_chain_params *c, int num_plp, 
   return h;
 }
 
+dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, int max_frames,
+                                          int device)
+{
+  if (!c || !plp || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
+  if (num_plp < 1 || num_plp > t2::MAX_PLP) { fail(DVBT2LL_ERR_INVALID, "chain: number of PLPs out of range"); return 0; }
+  int fecblocks = 0;
+  for (int p = 0; p < num_plp; p++) {
+    if (plp[p].fecblocks < 1 || plp[p].fecblocks > 1023) { fail(DVBT2LL_ERR_INVALID, "chain: FEC blocks of a PLP out of range"); return 0; }
+    fecblocks += plp[p].fecblocks;
+  }
+  std::unique_ptr<ChainHandle> h(new ChainHandle());
+  std::string err;
+  h->max_frames = max_frames; h->device = device;
+  // the frame's own FEC / modulation fields are PLP 0's (they name the parameter set of the stages bb / ldpc / map)
+  t2::FrameParams fp = { plp[0].framesize, plp[0].rate, plp[0].constellation, plp[0].rotation, fecblocks, c->tiblocks,
+                         c->carriermode, c->fftsize, c->guardinterval, c->l1constellation, c->pilotpattern, c->t2frames,
+                         c->numdatasyms, c->paprmode, c->version, c->preamble, c->inputmode, c->reservedbiasbits,
+                         c->l1scrambled, c->inband };
+  fp.num_plp = num_plp;
+  fp.plp_modcod = 1;
+  for (int p = 0; p < num_plp; p++) {
+    fp.plp_fecblocks[p] = plp[p].fecblocks;
+    fp.plp_framesize[p] = plp[p].framesize; fp.plp_rate[p] = plp[p].rate;
+    fp.plp_constellation[p] = plp[p].constellation; fp.plp_rotation[p] = plp[p].rotation;
+  }
+  t2::OfdmParams op = { c->carriermode, c->fftsize, c->pilotpattern, c->guardinterval, c->numdatasyms, c->paprmode,
+                        c->version, c->preamble, c->misogroup, c->equalization, c->bandwidth, c->vlength };
+  bool ok = t2::build_frame_plan(fp, &h->fplan, &err);
+  // the stages of every parameter set, built from its first PLP: the same checks as a single-PLP chain's
+  for (int s = 0; ok && s < h->fplan.plp_sets; s++) {
+    int p = 0;
+    while (h->fplan.plp_set[p] != s) p++;
+    if (s) h->xset[s].reset(new ChainHandle::Set());
+    BbHandle &bb = s ? h->xset[s]->bb : h->bb;
+    LdpcHandle &ldpc = s ? h->xset[s]->ldpc : h->ldpc;
+    MapHandle &map = s ? h->xset[s]->map : h->map;
+    ok = ok && t2::build_bb_plan(plp[p].framesize, plp[p].rate, c->inputmode, c->inband, fecblocks, c->tsrate, &bb.plan, &err);
+    ok = ok && t2::build_ldpc_plan(plp[p].framesize, plp[p].rate, &ldpc.plan, &err);
+    ok = ok && t2::build_map_plan(plp[p].framesize, plp[p].rate, plp[p].constellation, plp[p].rotation, &map.plan, &err);
+  }
+  ok = ok && t2::build_ofdm_plan(op, &h->oplan, &err);
+  ok = ok && t2::compose_chain16(h->fplan, h->oplan, &h->tables, &err);
+  if (!ok) { fail(DVBT2LL_ERR_INVALID, err); return 0; }
+  if (h->mixed()) {
+    // one table per distinct (constellation, rotation), the largest first: the non-data carriers' look-ups (entry =
+    // any cell code, see OFDM_CODE_TAB_SHIFT) stay inside it
+    std::vector<int> order;
+    for (int p = 0; p < num_plp; p++) order.push_back(p);
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return plp[x].constellation > plp[y].constellation; });
+    h->lut_tables = 0;
+    h->lut_single = 1;
+    for (size_t i = 0; i < order.size(); i++) {
+      const int p = order[i];
+      const t2::MapPlan &mp = h->map_of(p).plan;
+      h->lut_single &= mp.im_from_re;
+      size_t j = 0;
+      while (j < i && !(plp[order[j]].constellation == plp[p].constellation && plp[order[j]].rotation == plp[p].rotation)) j++;
+      if (j < i) { h->lut_base[p] = h->lut_base[order[j]]; continue; }
+      h->lut_base[p] = (int)h->luts.size();
+      h->luts.insert(h->luts.end(), mp.lut.begin(), mp.lut.end());
+      h->lut_tables++;
+    }
+    h->luts.resize((h->luts.size() + 15) & ~(size_t)15);      // the small pool behind the tables stays 64-byte aligned
+    if (h->luts.size() - 1 > t2k::OFDM_CODE_TAB_MAX) { fail(DVBT2LL_ERR_INVALID, "chain: constellation tables too large"); return 0; }
+  }
+  return h.release();
+}
+
 dvbt2ll_handle *dvbt2ll_chain_create(const dvbt2ll_chain_params *c, int max_frames, int device)
 {
   return chain_create(c, 1, 0, max_frames, device);
@@ -1518,6 +1692,29 @@ long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, lon
   const size_t nfec = (size_t)c->last_frames * c->F();
   const void *src; size_t bytes;
   std::string n(stage);
+  if ((n.compare(0, 4, "bch.") == 0 || n.compare(0, 4, "fec.") == 0) && n.size() > 4) {
+    // PLP p's codewords [channel][frame][block] at its own pitch: its region of the PLP-major buffers, or gathered from
+    // the frame-major ones
+    char *end = 0;
+    const long p = std::strtol(n.c_str() + 4, &end, 10);
+    if (*end || p < 0 || p >= c->P()) return fail(DVBT2LL_ERR_INVALID, "chain: unknown tap");
+    const bool fec = n[0] == 'f';
+    const size_t pitch = fec ? c->fec_pitch((int)p) : c->bch_pitch((int)p), fp = c->Fp((int)p);
+    const DevBuf &buf = fec ? c->d_fec : c->d_bch;
+    bytes = (size_t)c->last_frames * fp * pitch;
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaDeviceSynchronize());
+    if (!out || cap <= 0) return (long long)bytes;
+    std::vector<uint8_t> h(bytes);
+    if (c->mixed()) CK(cudaMemcpy(h.data(), buf.as<uint8_t>() + (fec ? c->fec_off[p] : c->bch_off[p]), bytes, cudaMemcpyDeviceToHost));
+    else
+      for (int f = 0; f < c->last_frames; f++)
+        CK(cudaMemcpy(h.data() + (size_t)f * fp * pitch, buf.as<uint8_t>() + ((size_t)f * c->F() + c->fplan.plp_first_block[p]) * pitch,
+                      fp * pitch, cudaMemcpyDeviceToHost));
+    std::memcpy(out, h.data(), (size_t)cap < bytes ? (size_t)cap : bytes);
+    return (long long)bytes;
+  }
+  if ((n == "bch" || n == "fec") && c->mixed()) return fail(DVBT2LL_ERR_INVALID, "chain: the PLPs have their own FEC parameters: use the taps bch.<plp> / fec.<plp>");
   if (n == "bch") { src = c->d_bch.p; bytes = nfec * align16(c->bb.plan.fec.nbch / 8); }
   else if (n == "fec") { src = c->d_fec.p; bytes = nfec * align16(c->bb.plan.fec.nldpc / 8); }
   else if (n == "cells") { src = c->d_cells.p; bytes = (size_t)c->last_frames * c->cells16_stride() * sizeof(uint16_t); }

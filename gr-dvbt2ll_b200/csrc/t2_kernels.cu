@@ -1610,10 +1610,11 @@ struct FillSmem {
 // from the big pool (L1 signalling / dummy cells); SINC: inverse-sinc equalisation factors are applied.
 // `c` holds the codes of the thread's first batch (loaded by the caller ahead of the barrier that precedes the fill);
 // the codes of batch n + 1 are fetched while batch n is processed.
-template <int LOG2M, int T, bool C16, bool POOL, bool SINC>
+// MT: the carrier codes carry the first entry of their constellation table (several tables, see OFDM_CODE_TAB_SHIFT).
+template <int LOG2M, int T, bool C16, bool POOL, bool SINC, bool MT = false>
 __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__ code, const float *__restrict__ sinc,
                                           int (&c)[FillGeom<LOG2M, T>::GPB][FillGeom<LOG2M, T>::R0], const float2 *__restrict__ cells,
-                                          const float2 *__restrict__ pool, const FillSmem fs, int stage_cap_dbg = 0)
+                                          const float2 *__restrict__ pool, const FillSmem fs, int stage_cap_dbg = 0, int lut_n_dbg = 0)
 {
   typedef FillGeom<LOG2M, T> G;
   constexpr int R0 = G::R0, GPB = G::GPB;
@@ -1629,7 +1630,8 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
           // data cell: 16-bit code from the staging area through the LUT (a dummy read of offset 0 for the others);
           // small pool cell (null, pilots): (p + 1) << 17 -> spool[p]; big pool cell: sign bit set (POOL symbols only)
           const unsigned off = POOL && cc < 0 ? 0u : (unsigned)cc & 0x1FFFFu;
-          BND(cc < 0 || cc >= 0x20000 || off + 2 <= 2u * (unsigned)stage_cap_dbg);
+          // small pool cell: bits 17..20 only (with table bits a data code can exceed 0x20000 as well)
+          BND(cc < 0 || (MT ? (unsigned)cc - 0x20000u < OFDM_CODE_SMALL_POOL : cc >= 0x20000) || off + 2 <= 2u * (unsigned)stage_cap_dbg);
           // explicit 32-bit shared-window addresses (one base register + the lane's table column): the generic-pointer
           // form made the compiler rebuild the window base and the lane offset for every carrier (≈ 10 instructions)
           unsigned sc;
@@ -1637,9 +1639,18 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
           // the tables are replicated 2^rep_shift times (entry e, copy c at (e << esh) + 4 c) and a lane reads copy
           // lane mod copies: with 32 copies no two lanes share a bank, with 16 only lanes l and l + 16 can collide
           float2 val;
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.x) : "r"(fs.lut_lane_s + ((sc & 255u) << fs.esh)));
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.y) : "r"(fs.lut_lane_s + fs.im_ofs + ((sc >> 8) << fs.esh)));
-          if (cc >= 0x20000) asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(val.x), "=f"(val.y) : "r"(fs.spool_m8_s + ((unsigned)cc >> 14)));
+          if constexpr (MT) {
+            // the cell's own table starts at entry tb; pool and pilot carriers read the first (largest) table
+            const unsigned tb = POOL && cc < 0 ? 0u : (unsigned)cc >> OFDM_CODE_TAB_SHIFT;
+            BND(tb + (sc & 255u) < (unsigned)lut_n_dbg && tb + (sc >> 8) < (unsigned)lut_n_dbg);
+            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.x) : "r"(fs.lut_lane_s + ((tb + (sc & 255u)) << fs.esh)));
+            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.y) : "r"(fs.lut_lane_s + fs.im_ofs + ((tb + (sc >> 8)) << fs.esh)));
+          }
+          else {
+            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.x) : "r"(fs.lut_lane_s + ((sc & 255u) << fs.esh)));
+            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.y) : "r"(fs.lut_lane_s + fs.im_ofs + ((sc >> 8) << fs.esh)));
+          }
+          if (MT ? (unsigned)cc - 0x20000u < OFDM_CODE_SMALL_POOL : cc >= 0x20000) asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(val.x), "=f"(val.y) : "r"(fs.spool_m8_s + ((unsigned)cc >> 14)));
           if (POOL && cc < 0) val = __ldg(pool + (cc & 0x7FFFFFFF));
           v[b][r] = val;
         }
@@ -1706,9 +1717,14 @@ __device__ __forceinline__ void tmem_wait_ld4(float2 (&v)[4])
                : "+f"(v[0].x), "+f"(v[0].y), "+f"(v[1].x), "+f"(v[1].y), "+f"(v[2].x), "+f"(v[2].y), "+f"(v[3].x), "+f"(v[3].y));
 }
 
+// FMT: sink format (bit 0, SinkT) | OFDM_FMT_MT: chain mode with several constellation tables, the carrier codes carry
+// their table's first entry (OFDM_CODE_TAB_SHIFT)
+constexpr int OFDM_FMT_MT = 2;
 template <int LOG2M, int T, bool C16, int FMT, int SPLIT>
 __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const OfdmArgs a)
 {
+  constexpr bool MT = (FMT & OFDM_FMT_MT) != 0;
+  static_assert(!MT || C16, "several constellation tables only in chain mode");
   extern __shared__ __align__(16) uint8_t smem_raw[];
   float2 *x = reinterpret_cast<float2 *>(smem_raw);
   constexpr int M = 1 << LOG2M;
@@ -1725,7 +1741,10 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
   const uint32_t desc_s = mbar_s + 16;
   if (C16) {
     // the constellation table goes through the (still unused) transform buffer: one L2 round trip, then replication
-    if (threadIdx.x < a.lut_n) x[threadIdx.x] = __ldg(a.lut + threadIdx.x);
+    if constexpr (MT) {
+      for (int i = threadIdx.x; i < a.lut_n; i += T) x[i] = __ldg(a.lut + i);     // the tables together can exceed T entries
+    }
+    else if (threadIdx.x < a.lut_n) x[threadIdx.x] = __ldg(a.lut + threadIdx.x);
     if (threadIdx.x < 8) spool[threadIdx.x] = __ldg(a.pool + threadIdx.x);
     // carriers that are not data cells do a dummy read of staging slot 0 and look its code up: until a symbol with
     // data cells has been staged that slot must hold a valid code (the tables only have lut_n entries)
@@ -1865,7 +1884,7 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
     const float2 *cells = a.cells + (long long)f * a.cells_stride;
     const float2 *pool = a.pool + (long long)variant * a.pool_stride;
     // output addressing in samples relative to a.out (element size depends on the sink format)
-    typedef typename SinkT<FMT>::type sample_t;
+    typedef typename SinkT<FMT & 1>::type sample_t;
     sample_t *out = reinterpret_cast<sample_t *>(a.out) + (long long)f * a.out_stride;
     sample_t *sym = out + 2048 + (long long)l * (N + a.gi);
     BND(a.out_len == 0 || (long long)f * a.out_stride + 2048 + (long long)(l + 1) * (N + a.gi) <= a.out_len);
@@ -1895,12 +1914,12 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
       if (C16 && phase == 0 && threadIdx.x == 0 && unit + (int)gridDim.x < units) desc_issue(cp1);
       // ---- 1. carrier fill (+ first pass)
       if (sinc) {
-        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, true>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
-        else ofdm_fill<LOG2M, T, C16, false, true>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
+        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, true, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
+        else ofdm_fill<LOG2M, T, C16, false, true, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
       }
       else {
-        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, false>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
-        else ofdm_fill<LOG2M, T, C16, false, false>(x, code, sinc, c, cells, pool, fs, a.stage_cap);
+        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, false, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
+        else ofdm_fill<LOG2M, T, C16, false, false, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
       }
       __syncthreads();
       // every fill of the symbol has read its cells: the next symbol's cells may replace them (under the passes)
@@ -2048,9 +2067,9 @@ static void launch_ofdm_c(const OfdmArgs &a, cudaStream_t s)
   }
 }
 
-void launch_ofdm(const OfdmArgs &a0, cudaStream_t s)
+int launch_ofdm(const OfdmArgs &a0, cudaStream_t s)
 {
-  if (a0.frames * a0.num_symbols < 1) return;
+  if (a0.frames * a0.num_symbols < 1) return 1;
   OfdmArgs a = a0;
   // up to 32 copies of the constellation table(s) (conflict-free: copy = lane), as many as shared memory allows (chain mode)
   // (without lowering the number of CTAs per SM that fit without replication; 2 resident CTAs at most are useful below 16K)
@@ -2064,11 +2083,16 @@ void launch_ofdm(const OfdmArgs &a0, cudaStream_t s)
     for (int sh = 5; sh > 0; sh--)
       if (base + (one << sh) + 1024 <= sm_bytes / ctas) { a.lut_rep_shift = sh; break; }
   }
-  if (a.cells16) {
+  if (a.cells16 && a.lut_tables > 1) {
+    if (a.out_fmt) launch_ofdm_c<true, 1 | OFDM_FMT_MT>(a, s);
+    else launch_ofdm_c<true, 0 | OFDM_FMT_MT>(a, s);
+  }
+  else if (a.cells16) {
     if (a.out_fmt) launch_ofdm_c<true, 1>(a, s);
     else launch_ofdm_c<true, 0>(a, s);
   }
   else launch_ofdm_c<false, 0>(a, s);      // the drop-in block always emits complex64
+  return 1 << a.lut_rep_shift;
 }
 
 } // namespace t2k

@@ -117,8 +117,8 @@ void launch_gather(const GatherArgs &a, cudaStream_t s);
 // ---- K5: carrier fill + IFFT + normalisation + guard interval + P1 --------------------------------
 struct OfdmArgs {
   const float2 *cells; long long cells_stride;   // per T2 frame (stride in cells for both cell formats)
-  // chain mode with 16-bit cells: cells16 != NULL selects it; then `code_pos` holds the encoding described at
-  // OfdmDevice::init (2 * staging slot | (small pool cell + 1) << 17 | 0x80000000 + pool cell)
+  // chain mode with 16-bit cells: cells16 != NULL selects it; then `code_pos` holds the carrier codes below
+  // (OFDM_CODE_*, written by OfdmDevice::init)
   const uint16_t *cells16;   // [frame][fecblocks * cell_size] cell-interleaved 16-bit codes; frames start 16-byte aligned
   // bulk copies (cp.async.bulk) that stage a symbol's cells in shared memory: run i = { source 16-byte unit from the
   // frame's first cell, (staging 16-byte unit << 16) | length in units }, symbols back to back
@@ -151,8 +151,22 @@ struct OfdmArgs {
   // extents for the debug build bounds checks (0 = not checked): cells behind cells / cells16, samples behind out,
   // cells in one copy of the pool
   long long cells_len, out_len, pool_len;
+  // > 1: `lut` holds that many constellation tables back to back (lut_n entries in all, the largest table first) and the
+  // data carrier codes carry their table's first entry (OFDM_CODE_TAB_SHIFT); the k_ofdm instantiations with OFDM_FMT_MT run
+  int lut_tables;
 };
-void launch_ofdm(const OfdmArgs &a, cudaStream_t s);
+// Chain-mode carrier codes of k_ofdm (code_pos), one 32-bit word per carrier:
+//   data carrier         -> 2 * staging slot                       bits 1..16 (byte offset into the staging area)
+//                           | first table entry << 21              bits 21..30, only with several tables (lut_tables > 1)
+//   small pool cell p<8  -> (p + 1) << 17                          bits 17..20 (zero / pilot amplitudes, in shared memory)
+//   other pool cell      -> 0x80000000 | pool index                (L1 signalling, dummy cells; their symbols are flagged)
+// Non-data carriers look up entry (staging slot 0's code) of the first table, which is the largest: any cell code
+// stays inside it.
+constexpr int OFDM_CODE_TAB_SHIFT = 21;
+constexpr unsigned OFDM_CODE_TAB_MAX = 1023;      // largest first-entry index the table bits hold
+constexpr unsigned OFDM_CODE_SMALL_POOL = 0x1E0000u;   // bits of a small pool cell
+// returns the number of constellation-table copies kept in shared memory (chain mode; 1 otherwise)
+int launch_ofdm(const OfdmArgs &a, cudaStream_t s);
 // shared-memory position (before swizzle) at which the carrier-fill stage must store bin m of an
 // M = 2^log2_m point sub-transform (mixed-radix digit reversal matching the kernel's pass schedule)
 int ofdm_position_of_bin(int m, int log2_m);

@@ -158,18 +158,32 @@ struct FrameParams {
   // (fecblocks = their sum), laid one after the other in the frame.  num_plp = 0 or 1 is the reference's case.
   int num_plp;
   int plp_fecblocks[MAX_PLP];
+  // plp_modcod = 1: PLP p has its own FEC type, code rate, constellation and rotation (L1-post PLP_FEC_TYPE, PLP_COD,
+  // PLP_MOD, PLP_ROTATION); otherwise every PLP takes framesize / rate / constellation / rotation above.  A frame whose
+  // PLPs do not fit is then always refused (there is no reference behaviour to reproduce).
+  int plp_modcod;
+  int plp_framesize[MAX_PLP], plp_rate[MAX_PLP], plp_constellation[MAX_PLP], plp_rotation[MAX_PLP];
 };
 struct FramePlan {
   FrameParams prm;
   OfdmDims dims;
-  int cell_size, stream_items, mapped_items;
+  int cell_size, stream_items, mapped_items;   // cell_size: PLP 0's cells per FECFRAME
   int eta_mod, n_post, n_punc, dummy_cells;
   bool overfull;                       // reference warns "too many FEC blocks in T2 frame"
   int num_plp;                         // >= 1
   int plp_first_block[MAX_PLP + 1];    // first FEC block of each PLP inside the T2 frame's block list
+  int plp_cell_size[MAX_PLP];          // cells per FECFRAME of each PLP
+  int plp_first_cell[MAX_PLP + 1];     // first cell of each PLP in the frame's data cells (L1-post PLP_START)
+  // Chain mode: PLP p's 16-bit cells start at plp_chain_off[p] of the frame's cell memory.  PLPs of one parameter set
+  // follow each other (plp_chain_off = plp_first_cell); with more than one set (plp_sets > 1, one mapper launch per
+  // PLP) every PLP starts on an 8-cell (16-byte) boundary.  plp_chain_off[num_plp] = cells of a frame in that memory.
+  int plp_chain_off[MAX_PLP + 1];
+  int plp_sets;                        // distinct (framesize, rate, constellation, rotation) among the PLPs
+  int plp_set[MAX_PLP];                // the set of each PLP (0 = PLP 0's)
+  std::vector<std::vector<uint16_t> > plp_cell_perm_inv;   // [num_plp] inverse cell permutation of each PLP
   int l1post_sig_bits;                 // K_sig of L1-post (350 for one PLP)
   std::vector<int32_t> cell_perm;      // cell interleaver permutation (reference :1087-1107)
-  std::vector<int32_t> fec_shift;      // per FEC block cyclic shift (reference :1981-1992)
+  std::vector<int32_t> fec_shift;      // per FEC block cyclic shift (reference :1981-1992), with its PLP's cell count
   std::vector<int32_t> ti_src;         // time-interleaver read-out position -> input cell index (cell int. composed)
   std::vector<int32_t> ci_dst;         // input cell index -> index in cell-interleaved memory
   std::vector<uint16_t> cell_perm_inv; // inverse of cell_perm
@@ -234,6 +248,7 @@ struct Chain16Tables {
   int max_runs;                     // longest list
   std::vector<int32_t> stage_bytes; // [num_symbols] bytes the symbol's copies deliver (mbarrier transaction count)
   int max_slots;                    // largest number of staging slots (cells) of any symbol
+  std::vector<uint8_t> plp;         // [num_symbols * c_ps]: the PLP whose cell a data carrier takes (0 for the others)
   CellPool pool;
 };
 bool compose_chain16(const FramePlan &fp, const OfdmPlan &op, Chain16Tables *out, std::string *err);

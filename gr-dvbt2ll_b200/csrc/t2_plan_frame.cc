@@ -204,17 +204,23 @@ void build_l1pre(const FrameParams &prm, int l1_post_size, int l1_post_info_size
   for (int i = 3240; i < 16200; i++) if (!punct[i]) bpsk(cw[i]);
 }
 
-void build_l1post(const FrameParams &prm, const int *plp_blocks, int num_plp, int cell_size, int frame_idx, int n_post, int n_punc,
+// what L1-post signals of one PLP
+struct PlpL1 { int blocks, cell_size, framesize, rate, constellation, rotation; };
+
+int plp_cod_of(int rate)
+{
+  switch (rate) {
+    case C1_3: return 6; case C2_5: return 7; case C1_2: return 0; case C3_5: return 1;
+    case C2_3: return 2; case C3_4: return 3; case C4_5: return 4; case C5_6: return 5;
+  }
+  return 0;
+}
+
+void build_l1post(const FrameParams &prm, const PlpL1 *plps, int num_plp, int frame_idx, int n_post, int n_punc,
                   int eta, std::vector<cfloat> &cells)
 {
   const bool v131 = prm.version == VERSION_131;
   const bool bias = prm.reservedbiasbits && v131;
-  int plp_cod = 0;
-  switch (prm.rate) {
-    case C1_3: plp_cod = 6; break; case C2_5: plp_cod = 7; break; case C1_2: plp_cod = 0; break;
-    case C3_5: plp_cod = 1; break; case C2_3: plp_cod = 2; break; case C3_4: plp_cod = 3; break;
-    case C4_5: plp_cod = 4; break; case C5_6: plp_cod = 5; break;
-  }
   BitWriter w;
   w.put(1, 15);                                  // SUB_SLICES_PER_FRAME
   w.put(num_plp, 8);                             // NUM_PLP
@@ -230,11 +236,11 @@ void build_l1post(const FrameParams &prm, const int *plp_blocks, int num_plp, in
     w.put(0, 3);                                 // FIRST_RF_IDX
     w.put(0, 8);                                 // FIRST_FRAME_IDX
     w.put(1, 8);                                 // PLP_GROUP_ID
-    w.put(plp_cod, 3);
-    w.put(prm.constellation, 3);
-    w.put(prm.rotation, 1);
-    w.put(prm.framesize, 2);                     // PLP_FEC_TYPE
-    w.put(plp_blocks[pl], 10);                   // PLP_NUM_BLOCKS_MAX
+    w.put(plp_cod_of(plps[pl].rate), 3);         // PLP_COD
+    w.put(plps[pl].constellation, 3);            // PLP_MOD
+    w.put(plps[pl].rotation, 1);                 // PLP_ROTATION
+    w.put(plps[pl].framesize, 2);                // PLP_FEC_TYPE
+    w.put(plps[pl].blocks, 10);                  // PLP_NUM_BLOCKS_MAX
     w.put(1, 8);                                 // FRAME_INTERVAL
     w.put(prm.tiblocks, 8);                      // TIME_IL_LENGTH
     w.put(0, 1);                                 // TIME_IL_TYPE
@@ -258,9 +264,9 @@ void build_l1post(const FrameParams &prm, const int *plp_blocks, int num_plp, in
     for (int pl = 0; pl < num_plp; pl++) {       // dynamic part, 48 bits per PLP
       w.put(pl, 8);                              // PLP_ID (dynamic; the reference leaves its single one uninitialised = 0)
       w.put(start, 22);                          // PLP_START
-      w.put(plp_blocks[pl], 10);                 // PLP_NUM_BLOCKS
+      w.put(plps[pl].blocks, 10);                // PLP_NUM_BLOCKS
       w.put(bias ? 0xff : 0, 8);                 // RESERVED_4
-      start += plp_blocks[pl] * cell_size;
+      start += plps[pl].blocks * plps[pl].cell_size;
     }
   }
   w.put(bias ? 0xff : 0, 8);                     // RESERVED_5
@@ -382,18 +388,42 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
   if (!ofdm_dims(prm.carriermode, prm.fftsize, prm.pilotpattern, prm.guardinterval, prm.numdatasyms,
                  prm.paprmode, prm.preamble, &p->dims, err)) return false;
   const OfdmDims &d = p->dims;
-  // PLPs: the reference's single one, or several type-1 PLPs of the same parameters one after the other
+  // PLPs: the reference's single one, or several type-1 PLPs one after the other, each with the frame's parameters or
+  // (plp_modcod) its own
   const int P = p->num_plp = prm.num_plp > 1 ? prm.num_plp : 1;
   if (P > MAX_PLP) { if (err) *err = "framemapperfint_cc: too many PLPs"; return false; }
   int plp_blocks[MAX_PLP];
+  PlpL1 plps[MAX_PLP];
   p->plp_first_block[0] = 0;
+  p->plp_first_cell[0] = 0;
+  p->plp_sets = 0;
   for (int pl = 0; pl < P; pl++) {
     plp_blocks[pl] = P == 1 ? prm.fecblocks : prm.plp_fecblocks[pl];
     if (plp_blocks[pl] < 1 || plp_blocks[pl] > 1023) { if (err) *err = "framemapperfint_cc: FEC blocks of a PLP out of range"; return false; }
     p->plp_first_block[pl + 1] = p->plp_first_block[pl] + plp_blocks[pl];
+    PlpL1 &q = plps[pl];
+    q.blocks = plp_blocks[pl];
+    q.framesize = prm.plp_modcod ? prm.plp_framesize[pl] : prm.framesize;
+    q.rate = prm.plp_modcod ? prm.plp_rate[pl] : prm.rate;
+    q.constellation = prm.plp_modcod ? prm.plp_constellation[pl] : prm.constellation;
+    q.rotation = prm.plp_modcod ? prm.plp_rotation[pl] : prm.rotation;
+    FecSpec qs;
+    if (!fec_spec(q.framesize, q.rate, &qs)) { if (err) *err = "framemapperfint_cc: unsupported (framesize, rate) of a PLP"; return false; }
+    q.cell_size = p->plp_cell_size[pl] = cells_per_fecframe(q.framesize, q.constellation);
+    if (!q.cell_size) { if (err) *err = "framemapperfint_cc: unknown constellation of a PLP"; return false; }
+    p->plp_first_cell[pl + 1] = p->plp_first_cell[pl] + q.blocks * q.cell_size;
+    int s = 0;
+    while (s < pl && !(plps[s].framesize == q.framesize && plps[s].rate == q.rate && plps[s].constellation == q.constellation &&
+                       plps[s].rotation == q.rotation)) s++;
+    p->plp_set[pl] = s < pl ? p->plp_set[s] : p->plp_sets++;
   }
   if (p->plp_first_block[P] != prm.fecblocks) { if (err) *err = "framemapperfint_cc: fecblocks is not the sum over the PLPs"; return false; }
-  const int Nc = p->cell_size, F = prm.fecblocks;
+  p->plp_chain_off[0] = 0;
+  for (int pl = 0; pl < P; pl++) {
+    const int end = p->plp_chain_off[pl] + plp_blocks[pl] * plps[pl].cell_size;
+    p->plp_chain_off[pl + 1] = p->plp_sets > 1 ? (end + 7) & ~7 : end;
+  }
+  const int F = prm.fecblocks;
   static const int etas[4] = { 1, 2, 4, 6 };
   const int eta = p->eta_mod = etas[prm.l1constellation];
 
@@ -407,17 +437,18 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
   p->n_punc = n_punc_temp - (p->n_post - n_post_temp);
   const int l1post_cells = p->n_post / eta;
 
-  p->stream_items = Nc * F;
+  p->stream_items = p->plp_first_cell[P];
   p->mapped_items = d.active_items;
   const int fixed = 1840 + l1post_cells + (d.n_fc - d.c_fc);
   p->overfull = p->mapped_items < p->stream_items + fixed;
   // Length of the linear frame before truncation.  Reference :1138-1141: an over-full frame only logs a warning,
   // grows its private frame buffers to stream_items + fixed "to avoid segfault" and carries on; the frequency
   // interleaver then reads the physical frame only, so the cells that do not fit are dropped.  By default creation
-  // fails with the reference's message; with the opt-in policy the same truncated frame is produced.
+  // fails with the reference's message; with the opt-in policy the same truncated frame is produced.  PLPs with their
+  // own parameters have no reference behaviour to reproduce: such a frame is always refused.
   int linear_items = p->mapped_items;
   if (p->overfull) {
-    if (!overfull_warn_policy()) {
+    if (!overfull_warn_policy() || prm.plp_modcod) {
       if (err) *err = "Frame Mapper, too many FEC blocks in T2 frame.";
       return false;
     }
@@ -425,38 +456,46 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
   }
   p->dummy_cells = linear_items - p->stream_items - fixed;
 
-  // ---- cell interleaver permutation (EN 302 755 6.4; reference :999-1107)
+  // ---- cell interleaver permutation (EN 302 755 6.4; reference :999-1107), one per PLP
   {
-    int deg;
-    static const int degs_n[4] = { 15, 14, 14, 13 }, degs_s[4] = { 13, 12, 12, 11 };
-    deg = (prm.framesize == FECFRAME_NORMAL ? degs_n : degs_s)[prm.constellation];
-    static const int t11[] = { 0, 3 }, t12[] = { 0, 2 }, t13[] = { 0, 1, 4, 6 }, t14[] = { 0, 1, 4, 5, 9, 11 }, t15[] = { 0, 1, 2, 12 };
-    const int *taps; int nt;
-    switch (deg) {
-      case 11: taps = t11; nt = 2; break; case 12: taps = t12; nt = 2; break; case 13: taps = t13; nt = 4; break;
-      case 14: taps = t14; nt = 6; break; default: taps = t15; nt = 4; break;
-    }
-    p->cell_perm.clear();
-    unsigned reg = 0;
-    const unsigned mask = (1u << (deg - 1)) - 1;
-    for (int i = 0; i < (1 << deg); i++) {
-      if (i < 2) reg = 0;
-      else if (i == 2) reg = 1;
-      else {
-        unsigned fb = 0;
-        for (int k = 0; k < nt; k++) fb ^= (reg >> taps[k]) & 1u;
-        reg = ((reg & mask) >> 1) | (fb << (deg - 2));
+    std::vector<std::vector<int32_t> > perm(P);
+    int deg[MAX_PLP];
+    p->plp_cell_perm_inv.assign(P, std::vector<uint16_t>());
+    for (int pl = 0; pl < P; pl++) {
+      const int Nc = plps[pl].cell_size;
+      static const int degs_n[4] = { 15, 14, 14, 13 }, degs_s[4] = { 13, 12, 12, 11 };
+      deg[pl] = (plps[pl].framesize == FECFRAME_NORMAL ? degs_n : degs_s)[plps[pl].constellation];
+      static const int t11[] = { 0, 3 }, t12[] = { 0, 2 }, t13[] = { 0, 1, 4, 6 }, t14[] = { 0, 1, 4, 5, 9, 11 }, t15[] = { 0, 1, 2, 12 };
+      const int *taps; int nt;
+      switch (deg[pl]) {
+        case 11: taps = t11; nt = 2; break; case 12: taps = t12; nt = 2; break; case 13: taps = t13; nt = 4; break;
+        case 14: taps = t14; nt = 6; break; default: taps = t15; nt = 4; break;
       }
-      reg |= (unsigned)(i & 1) << (deg - 1);
-      if ((int)reg < Nc) p->cell_perm.push_back((int32_t)reg);
+      unsigned reg = 0;
+      const unsigned mask = (1u << (deg[pl] - 1)) - 1;
+      for (int i = 0; i < (1 << deg[pl]); i++) {
+        if (i < 2) reg = 0;
+        else if (i == 2) reg = 1;
+        else {
+          unsigned fb = 0;
+          for (int k = 0; k < nt; k++) fb ^= (reg >> taps[k]) & 1u;
+          reg = ((reg & mask) >> 1) | (fb << (deg[pl] - 2));
+        }
+        reg |= (unsigned)(i & 1) << (deg[pl] - 1);
+        if ((int)reg < Nc) perm[pl].push_back((int32_t)reg);
+      }
+      if ((int)perm[pl].size() != Nc) { if (err) *err = "internal: cell permutation size"; return false; }
+      p->plp_cell_perm_inv[pl].assign(Nc, 0);
+      for (int w = 0; w < Nc; w++) p->plp_cell_perm_inv[pl][perm[pl][w]] = (uint16_t)w;
     }
-    if ((int)p->cell_perm.size() != Nc) { if (err) *err = "internal: cell permutation size"; return false; }
+    p->cell_perm = perm[0];
+    p->cell_perm_inv = p->plp_cell_perm_inv[0];
 
     // TI block split (reference :1108-1119) and per-FEC-block shifts (restart per TI block, :1974-1992), PLP by PLP
     p->fec_shift.clear();
-    std::vector<int> ti_block_sizes;
+    std::vector<int> ti_block_sizes, ti_block_rows;
     for (int pl = 0; pl < P; pl++) {
-      const int Fp = plp_blocks[pl];
+      const int Fp = plp_blocks[pl], Nc = plps[pl].cell_size;
       int small, big, nbig, nsmall;
       if (prm.tiblocks == 0) { small = big = 1; nbig = 0; nsmall = Fp; }
       else {
@@ -468,12 +507,13 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
       for (int s = 0; s < nsmall + nbig; s++) {
         const int k = s < nsmall ? small : big;
         ti_block_sizes.push_back(k);
+        ti_block_rows.push_back(Nc / 5);
         unsigned n = 0;
         for (int r = 0; r < k; r++) {
           int shift = Nc;
           while (shift >= Nc) {
             unsigned t = n, sh = 0;
-            for (int b = 0; b < deg; b++) { sh |= t & 1u; sh <<= 1; t >>= 1; }
+            for (int b = 0; b < deg[pl]; b++) { sh |= t & 1u; sh <<= 1; t >>= 1; }
             shift = (int)sh;
             n++;
           }
@@ -484,25 +524,27 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
     if ((int)p->fec_shift.size() != F) { if (err) *err = "framemapperfint_cc: fecblocks/tiblocks combination leaves FEC blocks unassigned"; return false; }
 
     // cell-interleaved memory index <-> input index
-    std::vector<int32_t> ci_src((size_t)F * Nc);
-    p->ci_dst.assign((size_t)F * Nc, 0);
-    for (int r = 0; r < F; r++)
-      for (int w = 0; w < Nc; w++) {
-        const int x = r * Nc + (p->cell_perm[w] + p->fec_shift[r]) % Nc;
-        ci_src[x] = r * Nc + w;
-        p->ci_dst[(size_t)r * Nc + w] = x;
+    std::vector<int32_t> ci_src((size_t)p->stream_items);
+    p->ci_dst.assign((size_t)p->stream_items, 0);
+    for (int pl = 0; pl < P; pl++) {
+      const int Nc = plps[pl].cell_size;
+      for (int r = p->plp_first_block[pl]; r < p->plp_first_block[pl + 1]; r++) {
+        const int base = p->plp_first_cell[pl] + (r - p->plp_first_block[pl]) * Nc;
+        for (int w = 0; w < Nc; w++) {
+          const int x = base + (perm[pl][w] + p->fec_shift[r]) % Nc;
+          ci_src[x] = base + w;
+          p->ci_dst[(size_t)base + w] = x;
+        }
       }
-    p->cell_perm_inv.assign(Nc, 0);
-    for (int w = 0; w < Nc; w++) p->cell_perm_inv[p->cell_perm[w]] = (uint16_t)w;
+    }
 
     // time interleaver read-out (EN 302 755 6.5; reference :1999-2028)
-    p->ti_src.assign((size_t)F * Nc, 0);
+    p->ti_src.assign((size_t)p->stream_items, 0);
     if (prm.tiblocks == 0) p->ti_src = ci_src;
     else {
       size_t o = 0;
-      const int rows = Nc / 5;
       for (size_t s = 0; s < ti_block_sizes.size(); s++) {
-        const int cols = 5 * ti_block_sizes[s];
+        const int cols = 5 * ti_block_sizes[s], rows = ti_block_rows[s];
         for (int j = 0; j < rows; j++)
           for (int c = 0; c < cols; c++) p->ti_src[o + (size_t)cols * j + c] = ci_src[o + (size_t)rows * c + j];
         o += (size_t)rows * cols;
@@ -525,7 +567,7 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
   pool.l1post_variants = prm.t2frames;
   for (int v = 0; v < prm.t2frames; v++) {
     std::vector<cfloat> c;
-    build_l1post(prm, plp_blocks, P, Nc, v, p->n_post, p->n_punc, eta, c);
+    build_l1post(prm, plps, P, v, p->n_post, p->n_punc, eta, c);
     if ((int)c.size() != l1post_cells) { if (err) *err = "internal: L1-post size"; return false; }
     pool.cells.insert(pool.cells.end(), c.begin(), c.end());
   }

@@ -332,6 +332,12 @@ bool compose_chain16(const FramePlan &fp, const OfdmPlan &op, Chain16Tables *out
   out->run_cnt.assign(L, 0);
   out->max_slots = 0;
   out->max_runs = 0;
+  out->plp.assign(op.code.size(), 0);
+  // cell-interleaved index -> (PLP, address in the chain's cell memory: the PLP's region, see FramePlan::plp_chain_off)
+  std::vector<uint8_t> plp_of((size_t)fp.stream_items);
+  for (int pl = 0; pl < fp.num_plp; pl++)
+    std::fill(plp_of.begin() + fp.plp_first_cell[pl], plp_of.begin() + fp.plp_first_cell[pl + 1], (uint8_t)pl);
+  auto addr = [&](int32_t x) { return x - fp.plp_first_cell[plp_of[x]] + fp.plp_chain_off[plp_of[x]]; };
   for (int l = 0; l < L; l++) {
     const int s0 = op.sym_data_start[l], s1 = op.sym_data_start[l + 1];     // frame positions of this symbol
     // staging layout: the symbol's source cells sorted by source address, copied run by run with bulk
@@ -342,7 +348,7 @@ bool compose_chain16(const FramePlan &fp, const OfdmPlan &op, Chain16Tables *out
     std::vector<std::pair<int32_t, int32_t> > ps;      // (source cell, frame-order position - s0)
     for (int pos = s0; pos < s1; pos++) {
       const int32_t f = fp.framed[pos];
-      if (f >= 0) ps.push_back(std::make_pair(fp.ci_dst[f], pos - s0));
+      if (f >= 0) ps.push_back(std::make_pair(addr(fp.ci_dst[f]), pos - s0));
     }
     std::sort(ps.begin(), ps.end());
     std::vector<int32_t> slot_of_pos(s1 - s0, -1);
@@ -383,6 +389,7 @@ bool compose_chain16(const FramePlan &fp, const OfdmPlan &op, Chain16Tables *out
         const int32_t pos = fp.fi_src[c];
         const int32_t f = fp.framed[pos];
         v = f >= 0 ? slot_of_pos[pos - s0] : -(1 + base + (-(f + 1)));
+        if (f >= 0) out->plp[(size_t)l * cps + k] = plp_of[fp.ci_dst[f]];
       }
       out->code[(size_t)l * cps + k] = v;
     }

@@ -38,7 +38,7 @@ EXPORTED_SYMBOLS = [
     "dvbt2ll_device_count", "dvbt2ll_set_device", "dvbt2ll_device_synchronize",
     "dvbt2ll_stream_create", "dvbt2ll_stream_destroy", "dvbt2ll_stream_synchronize",
     "dvbt2ll_chain_create_multiplp", "dvbt2ll_chain_num_plp", "dvbt2ll_chain_plp_ts_bytes",
-    "dvbt2ll_chain_history_bytes", "dvbt2ll_ts_sync", "dvbt2ll_ts_fill",
+    "dvbt2ll_chain_history_bytes", "dvbt2ll_ts_sync", "dvbt2ll_ts_fill", "dvbt2ll_chain_create_plps",
 ]
 GATHER_BLOB_BYTES = 256
 
@@ -49,6 +49,18 @@ class ChainParams(C.Structure):
         "guardinterval", "l1constellation", "pilotpattern", "t2frames", "numdatasyms", "paprmode", "version",
         "preamble", "inputmode", "reservedbiasbits", "l1scrambled", "inband", "misogroup", "equalization",
         "bandwidth", "vlength", "tsrate")]
+
+
+class PlpParams(C.Structure):
+    _fields_ = [(n, C.c_int) for n in ("fecblocks", "framesize", "rate", "constellation", "rotation")]
+
+
+PLP_KEYS = ("framesize", "rate", "constellation", "rotation")
+
+
+def plp_params(cfg):
+    """cfg["plps"] with every PLP's missing framesize / rate / constellation / rotation taken from the cfg."""
+    return [dict({k: int(cfg[k]) for k in PLP_KEYS}, **{k: int(v) for k, v in p.items()}) for p in cfg["plps"]]
 
 
 def lib():
@@ -133,6 +145,8 @@ def lib():
         L.dvbt2ll_chain_create_multiplp.restype = vp
         L.dvbt2ll_chain_create_multiplp.argtypes = [C.POINTER(ChainParams), ci, C.POINTER(ci), ci, ci]
         L.dvbt2ll_chain_num_plp.argtypes = [vp]
+        L.dvbt2ll_chain_create_plps.restype = vp
+        L.dvbt2ll_chain_create_plps.argtypes = [C.POINTER(ChainParams), ci, C.POINTER(PlpParams), ci, ci]
         L.dvbt2ll_chain_plp_ts_bytes.restype = cll
         L.dvbt2ll_chain_plp_ts_bytes.argtypes = [vp, ci, cll, ci]
         L.dvbt2ll_chain_history_bytes.restype = cll
@@ -383,7 +397,11 @@ class Chain(_Block):
         self.cfg = cfg
         p = ChainParams(**{n: int(cfg[n]) for n, _ in ChainParams._fields_})
         plps = cfg.get("plp_fecblocks")
-        if plps and len(plps) > 1:          # several PLPs of the same parameters (beyond the single-PLP reference)
+        if cfg.get("plps"):                 # PLPs with their own FEC type, code rate, constellation and rotation
+            pp = plp_params(cfg)
+            arr = (PlpParams * len(pp))(*[PlpParams(**q) for q in pp])
+            h = lib().dvbt2ll_chain_create_plps(C.byref(p), len(pp), arr, int(max_frames), int(device))
+        elif plps and len(plps) > 1:        # several PLPs of the same parameters (beyond the single-PLP reference)
             arr = (C.c_int * len(plps))(*[int(x) for x in plps])
             h = lib().dvbt2ll_chain_create_multiplp(C.byref(p), len(plps), arr, int(max_frames), int(device))
         else:
@@ -459,6 +477,7 @@ class Chain(_Block):
         return r
 
     def tap(self, stage, dtype=np.uint8):
+        """Stage output of the most recent run: "bch", "fec", "cells", or one PLP's codewords "bch.<p>" / "fec.<p>"."""
         n = lib().dvbt2ll_chain_tap(self._h, stage.encode(), None, 0)
         if n < 0:
             raise RuntimeError(last_error())

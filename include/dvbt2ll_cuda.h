@@ -113,6 +113,18 @@ DVBT2LL_API_EXPORT dvbt2ll_handle *dvbt2ll_chain_create(const dvbt2ll_chain_para
  * num_plp = 1 is dvbt2ll_chain_create. */
 DVBT2LL_API_EXPORT dvbt2ll_handle *dvbt2ll_chain_create_multiplp(const dvbt2ll_chain_params *p, int num_plp,
                                                                  const int *plp_fecblocks, int max_frames, int device);
+/* PLPs with their own robustness: num_plp (1..16) type-1 data PLPs, PLP i with its own FEC type, code rate,
+ * constellation and rotation (enum values of dvbt2ll_config.h, validated as dvbt2ll_chain_create validates them) and
+ * plp[i].fecblocks (1..1023) FEC blocks per T2 frame; p->framesize / rate / constellation / rotation / fecblocks are
+ * ignored.  L1-post signals PLP_COD, PLP_MOD, PLP_ROTATION and PLP_FEC_TYPE per PLP, PLP_START advances by each PLP's
+ * cells.  Time interleaving (tiblocks) stays shared.  Everything else as dvbt2ll_chain_create_multiplp (TS row =
+ * channel * num_plp + plp, one stream per PLP).  A frame whose PLPs do not fit is always refused, whatever
+ * dvbt2ll_set_overfull_policy says.  Returns NULL and sets dvbt2ll_last_error on any failure. */
+typedef struct dvbt2ll_plp_params {
+  int fecblocks, framesize, rate, constellation, rotation;
+} dvbt2ll_plp_params;
+DVBT2LL_API_EXPORT dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *p, int num_plp,
+                                                             const dvbt2ll_plp_params *plp, int max_frames, int device);
 DVBT2LL_API_EXPORT int dvbt2ll_chain_num_plp(const dvbt2ll_handle *h);
 /* Stream bytes that must precede the first TS byte of first_frame in every row handed to dvbt2ll_chain_run_*:
  * 187 in normal input mode once the stream has started (CRC-8 of the packet in flight), else 0. */
@@ -143,7 +155,11 @@ DVBT2LL_API_EXPORT int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts,
 DVBT2LL_API_EXPORT int dvbt2ll_chain_set_sink(dvbt2ll_handle *h, int format, float gain);
 /* Stage taps of the most recent chain run, for parity tests: "bch" (packed bits), "fec" (packed, parity
  * in interleaved-row order), "cells" (uint16 cell codes in cell-interleaved order: own constellation word |
- * word supplying the imaginary part << 8, frame stride padded to a multiple of 4 cells).  Copies to HOST; returns
+ * word supplying the imaginary part << 8, frame stride padded to a multiple of 4 cells).  "bch.<p>" / "fec.<p>": PLP
+ * p's codewords only, [channel][frame][block] at the pitch of its code.  With dvbt2ll_chain_create_plps and more than
+ * one (framesize, rate, constellation, rotation) among the PLPs, "bch" and "fec" are refused, and in "cells" PLP p's
+ * cells start at an 8-cell boundary of each frame (dvbt2ll_plan_get "frame.plp_cells": per PLP cells per FECFRAME,
+ * first cell in the frame, first cell in this memory).  Copies to HOST; returns
  * bytes or negative error. */
 DVBT2LL_API_EXPORT long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, long long cap);
 /* Device time in ms of each stage kernel (bb_bch, ldpc, map, ofdm, total), averaged over the chain runs issued since
