@@ -8,9 +8,12 @@
 // of `batch` T2 frames per call (stream position carried by first_frame + the 187 history bytes in front of a batch).
 //
 // usage: t2_file_modulator [--config c1|c2|c3|c4] [--plp-blocks a,b,..] [--plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]]...
-//                          [--frames N] [--batch B] [--sc16 GAIN] --out FILE  TS_FILE [TS_FILE ...]
+//                          [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] --out FILE  TS_FILE [TS_FILE ...]
 // --plp, once per PLP: its FEC blocks per T2 frame and, optionally, its own FEC type, code rate, constellation and
 // rotation (enum values of dvbt2ll_config.h; the config's where omitted).
+// --papr-tr: paprmode = PAPR_TR and tone-reservation PAPR reduction on the reserved carriers (dvbt2ll_chain_set_papr_tr).
+// The reserved carriers take cells away: a config whose FEC blocks no longer fit is refused as over-full; lower its
+// block count with --plp BLOCKS (c1: 7, c3: 200, c4: 119; c2 fits as it is).
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -59,6 +62,8 @@ int main(int argc, char **argv)
   std::vector<const char *> inputs;
   int frames = -1, batch = 4, sc16 = 0;
   float gain = 1.0f;
+  int tr_iter = 0;
+  float tr_vclip = 0.f, tr_tone_max = 0.f;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
     if (a == "--config" && i + 1 < argc) cfg = argv[++i];
@@ -66,6 +71,12 @@ int main(int argc, char **argv)
     else if (a == "--frames" && i + 1 < argc) frames = std::atoi(argv[++i]);
     else if (a == "--batch" && i + 1 < argc) batch = std::atoi(argv[++i]);
     else if (a == "--sc16" && i + 1 < argc) { sc16 = 1; gain = (float)std::atof(argv[++i]); }
+    else if (a == "--papr-tr" && i + 1 < argc) {
+      if (std::sscanf(argv[++i], "%d:%f:%f", &tr_iter, &tr_vclip, &tr_tone_max) != 3) {
+        std::fprintf(stderr, "--papr-tr ITER:VCLIP:TONEMAX\n");
+        return 2;
+      }
+    }
     else if (a == "--plp-blocks" && i + 1 < argc) {
       for (char *t = std::strtok(argv[++i], ","); t; t = std::strtok(0, ",")) plp_blocks.push_back(std::atoi(t));
     }
@@ -81,7 +92,7 @@ int main(int argc, char **argv)
   }
   dvbt2ll_chain_params prm;
   if (!named_config(cfg, &prm) || out_path.empty() || inputs.empty() || batch < 1 || (!plps.empty() && !plp_blocks.empty())) {
-    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--frames N] [--batch B] [--sc16 GAIN] --out FILE TS_FILE...\n", argv[0]);
+    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] --out FILE TS_FILE...\n", argv[0]);
     return 2;
   }
   bool own = false;
@@ -94,10 +105,12 @@ int main(int argc, char **argv)
   const int P = own ? (int)plps.size() : plp_blocks.empty() ? 1 : (int)plp_blocks.size();
   if ((int)inputs.size() != P) { std::fprintf(stderr, "one TS file per PLP expected (%d)\n", P); return 2; }
   if (P == 1 && !own && !plps.empty()) prm.fecblocks = plps[0].fecblocks;
+  if (tr_iter) prm.paprmode = 2;      // PAPR_TR
   dvbt2ll_handle *h = own ? dvbt2ll_chain_create_plps(&prm, P, plps.data(), batch, -1)
                     : P == 1 ? dvbt2ll_chain_create(&prm, batch, -1) : dvbt2ll_chain_create_multiplp(&prm, P, plp_blocks.data(), batch, -1);
   if (!h) { std::fprintf(stderr, "chain: %s\n", dvbt2ll_last_error()); return 1; }
   if (sc16 && dvbt2ll_chain_set_sink(h, 1, gain) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }
+  if (tr_iter && dvbt2ll_chain_set_papr_tr(h, tr_iter, tr_vclip, tr_tone_max) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }
 
   // ---- ingest: sync acquisition per file; whole T2 frames available = limited by the shortest PLP (then null filled)
   std::vector<std::vector<unsigned char> > ts(P);

@@ -831,13 +831,20 @@ struct ChainHandle : dvbt2ll_handle {
   int sink_fmt;          // 0 complex64 (what pilotgenp1insert_cc emits), 1 interleaved int16 I/Q
   float sink_gain;       // the flowgraph's multiply_const stage folded into the last kernel
   cudaStream_t stream2;
+  // tone-reservation PAPR reduction (dvbt2ll_chain_set_papr_tr): k_papr_tr after k_ofdm when tr_iter > 0
+  int tr_iter;
+  float tr_vclip, tr_tone_max;
+  bool tr_built, tr_uploaded;
+  t2::PaprTrPlan tr;
+  DevBuf d_tr_set, d_tr_bins, d_tr_kernel, d_tr_tw, d_tr_stats, d_tr_scratch;
+  int tr_frames;         // frames whose counts the last run left in d_tr_stats (the "papr" tap)
   int last_frames;
   long long next_frame;  // stream position of the generic work() / work_device() path (T2 frames consumed so far)
   bool timing;
   enum { TIMING_SLOTS = 64 };
   cudaEvent_t ev[TIMING_SLOTS][5];     // per-run event sets so the timed loop never has to synchronise
   long long n_timed;
-  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), last_frames(0), next_frame(0), timing(false)
+  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), tr_iter(0), tr_vclip(0.f), tr_tone_max(0.f), tr_built(false), tr_uploaded(false), tr_frames(0), last_frames(0), next_frame(0), timing(false)
   {
     n_timed = 0;
     for (int s = 0; s < TIMING_SLOTS; s++) for (int i = 0; i < 5; i++) ev[s][i] = 0;
@@ -939,9 +946,9 @@ struct ChainHandle : dvbt2ll_handle {
     return 0;
   }
   // buf_frame: first T2-frame slot of the intermediate buffers to use; hist_valid < 0: history is present iff
-  // first_frame > 0
+  // first_frame > 0; tr_frame0: position of the batch's first frame in the tone-reservation counts (d_tr_stats)
   int run(const void *d_ts, long long ts_pitch, int n_channels, int n_frames, long long first_frame, void *d_out, cudaStream_t s,
-          int buf_frame = 0, int hist_valid = -1)
+          int buf_frame = 0, int hist_valid = -1, int tr_frame0 = 0)
   {
     const int frames = n_channels * n_frames;
     if (frames < 1) return 0;
@@ -987,6 +994,20 @@ struct ChainHandle : dvbt2ll_handle {
     t2k::launch_map(ma, s);
     if (timing) cudaEventRecord(tev[3], s);
     }
+    // tone reservation: in place on d_out when the sink is complex64 at gain 1; otherwise k_ofdm writes complex64 at
+    // gain 1 to a scratch (the buffer slots of buf_frame) and k_papr_tr applies the sink
+    const bool tr_on = tr_iter > 0, tr_inplace = tr_on && sink_fmt == 0 && sink_gain == 1.0f;
+    const long long spf = oplan.samples_per_frame;
+    void *ofdm_out = d_out;
+    if (tr_on) {
+      int r = tr_upload();
+      if (r) return r;
+      CK(d_tr_stats.ensure((size_t)(tr_frame0 + frames) * oplan.dims.num_symbols * sizeof(int16_t)));
+      if (!tr_inplace) {
+        CK(d_tr_scratch.ensure((size_t)max_frames * spf * sizeof(float2)));
+        ofdm_out = d_tr_scratch.as<float2>() + (size_t)buf_frame * spf;
+      }
+    }
     t2k::OfdmArgs oa;
     odev.fill(oa, oplan, tables.pool);
     oa.cells = 0; oa.cells_stride = cells16_stride();
@@ -995,16 +1016,42 @@ struct ChainHandle : dvbt2ll_handle {
     oa.stage_bytes = d_stage_bytes.as<int32_t>(); oa.stage_cap = stage_cap; oa.lut_single = map.plan.im_from_re;
     oa.lut = map.d_lut.as<float2>(); oa.lut_n = 1 << map.plan.mod;
     if (mixed()) { oa.lut_single = lut_single; oa.lut = d_luts.as<float2>(); oa.lut_n = (int)luts.size(); oa.lut_tables = lut_tables; }
-    oa.out = d_out; oa.out_stride = oplan.samples_per_frame;
+    oa.out = ofdm_out; oa.out_stride = oplan.samples_per_frame;
     oa.cells_len = (long long)frames * cells16_stride(); oa.out_len = (long long)frames * oplan.samples_per_frame;
     oa.out_fmt = sink_fmt; oa.sink_gain = sink_gain; oa.norm = oplan.normalization * sink_gain;
+    if (ofdm_out != d_out) { oa.out_fmt = 0; oa.sink_gain = 1.0f; oa.norm = oplan.normalization; }
     oa.frames = frames; oa.frames_per_channel = n_frames;
     oa.frame_idx0 = (int)(first_frame % (tables.pool.l1post_variants > 0 ? tables.pool.l1post_variants : 1));
     lut_copies = t2k::launch_ofdm(oa, s);
+    if (tr_on) {
+      t2k::PaprArgs pa;
+      pa.in = (const float2 *)ofdm_out; pa.out = d_out;
+      pa.out_fmt = sink_fmt; pa.gain = sink_gain; pa.inplace = tr_inplace ? 1 : 0;
+      pa.spf = spf; pa.fft_n = oplan.dims.fft_n; pa.gi = oplan.dims.gi; pa.num_symbols = oplan.dims.num_symbols; pa.frames = frames;
+      pa.iterations = tr_iter; pa.vclip = tr_vclip; pa.tone_max = tr_tone_max;
+      pa.tone_scale = (float)(1.0 / ((double)oplan.normalization * tr.tones));
+      pa.tones = tr.tones; pa.sets = tr.sets;
+      pa.sym_set = d_tr_set.as<int32_t>(); pa.bins = d_tr_bins.as<int32_t>();
+      pa.kernel = d_tr_kernel.as<float2>(); pa.tone_tw = d_tr_tw.as<float2>();
+      pa.stats = d_tr_stats.as<int16_t>() + (size_t)tr_frame0 * oplan.dims.num_symbols;
+      pa.in_len = pa.out_len = (long long)frames * spf;
+      t2k::launch_papr_tr(pa, s);
+      tr_frames = tr_frame0 + frames;
+    }
     if (timing) { cudaEventRecord(tev[4], s); n_timed++; }
     CK(cudaGetLastError());
     if (buf_frame == 0) last_frames = frames;
     return frames;
+  }
+  int tr_upload()
+  {
+    if (tr_uploaded) return 0;
+    CK(upload(d_tr_set, tr.sym_set));
+    CK(upload(d_tr_bins, tr.bins));
+    CK(upload(d_tr_kernel, tr.kernel));
+    CK(upload(d_tr_tw, tr.tone_tw));
+    tr_uploaded = true;
+    return 0;
   }
   // BB + BCH, LDPC and mapper of a chain whose PLPs have more than one parameter set: a launch per PLP and stage, each
   // on the PLP's own contiguous regions of the BCH / FEC buffers and of the cell memory
@@ -1084,6 +1131,9 @@ struct ChainHandle : dvbt2ll_handle {
       return copy_out(v, sizeof(int) * (3 + fplan.num_plp), out, cap);
     }
     if (n == "frame.fi_src") return copy_vec(fplan.fi_src, out, cap);
+    if (tr_built && n == "ofdm.tr_set") return copy_vec(tr.sym_set, out, cap);
+    if (tr_built && n == "ofdm.tr_bins") return copy_vec(tr.bins, out, cap);
+    if (tr_built && n == "ofdm.tr_kernel") return copy_vec(tr.kernel, out, cap);
     if (n == "frame.fec_shift") return copy_vec(fplan.fec_shift, out, cap);
     if (n == "frame.plp_cells") {
       // per PLP: cells per FECFRAME, first cell in the frame (PLP_START), first cell in the chain's cell memory
@@ -1663,6 +1713,8 @@ int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch
   // by 187 history bytes.  Channels are processed in groups on two streams so that the H2D copy and the
   // kernels of one group overlap the D2H copy of the previous one (the D2H copy dominates).
   if (!c->stream2) CK(cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking));
+  // every group writes its own part of the tone-reservation counts: size them for the whole call before the first
+  if (c->tr_iter > 0) CK(c->d_tr_stats.ensure((size_t)n_channels * n_frames * c->oplan.dims.num_symbols * sizeof(int16_t)));
   int groups = n_channels >= 8 ? 8 : n_channels;
   while (groups > 1 && 2 * ((n_channels + groups - 1) / groups) * n_frames > c->max_frames) groups--;
   const int per = (n_channels + groups - 1) / groups;
@@ -1674,7 +1726,7 @@ int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch
     CK(cudaMemcpy2DAsync(base + (size_t)c0 * P * dpitch - hist, (size_t)dpitch, (const uint8_t *)ts + (size_t)c0 * P * ts_pitch - hist,
                          (size_t)ts_pitch, (size_t)(per_ch + hist), (size_t)nc * P, cudaMemcpyHostToDevice, s));
     r = c->run(base + (size_t)c0 * P * dpitch, dpitch, nc, n_frames, first_frame, dout + (size_t)c0 * ch_out * ssz, s,
-               groups == 1 ? 0 : (gi & 1) * per * n_frames);
+               groups == 1 ? 0 : (gi & 1) * per * n_frames, -1, c0 * n_frames);
     if (r < 0) return r;
     CK(cudaMemcpyAsync((uint8_t *)out + (size_t)c0 * ch_out * ssz, dout + (size_t)c0 * ch_out * ssz, (size_t)nc * ch_out * ssz,
                        cudaMemcpyDeviceToHost, s));
@@ -1718,6 +1770,10 @@ long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, lon
   if (n == "bch") { src = c->d_bch.p; bytes = nfec * align16(c->bb.plan.fec.nbch / 8); }
   else if (n == "fec") { src = c->d_fec.p; bytes = nfec * align16(c->bb.plan.fec.nldpc / 8); }
   else if (n == "cells") { src = c->d_cells.p; bytes = (size_t)c->last_frames * c->cells16_stride() * sizeof(uint16_t); }
+  else if (n == "papr") {
+    if (c->tr_iter < 1 || c->tr_frames < 1) return fail(DVBT2LL_ERR_INVALID, "chain: the tone-reservation stage is off");
+    src = c->d_tr_stats.p; bytes = (size_t)c->tr_frames * c->oplan.dims.num_symbols * sizeof(int16_t);
+  }
   else return fail(DVBT2LL_ERR_INVALID, "chain: unknown tap");
   CK(cudaStreamSynchronize(c->stream));
   CK(cudaDeviceSynchronize());
@@ -1732,6 +1788,24 @@ int dvbt2ll_chain_set_sink(dvbt2ll_handle *h, int format, float gain)
   if (format != 0 && format != 1) return fail(DVBT2LL_ERR_INVALID, "chain: sink format must be 0 (complex64) or 1 (int16 I/Q)");
   c->sink_fmt = format;
   c->sink_gain = gain;
+  return 0;
+}
+
+int dvbt2ll_chain_set_papr_tr(dvbt2ll_handle *h, int iterations, float vclip, float tone_max)
+{
+  ChainHandle *c = as_chain(h);
+  if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
+  const int pm = c->oplan.prm.paprmode;
+  if (pm != t2::PAPR_TR && pm != t2::PAPR_BOTH) return fail(DVBT2LL_ERR_INVALID, "chain: tone reservation needs paprmode TR or BOTH");
+  if (iterations < 0 || iterations > 64) return fail(DVBT2LL_ERR_INVALID, "chain: tone-reservation iterations must be 0 (off) .. 64");
+  if (!(std::isfinite(vclip) && vclip > 0.f) || !(std::isfinite(tone_max) && tone_max > 0.f))
+    return fail(DVBT2LL_ERR_INVALID, "chain: tone-reservation vclip and tone_max must be finite and > 0");
+  if (!c->tr_built) {
+    std::string err;
+    if (!t2::build_papr_tr_plan(c->oplan, &c->tr, &err)) return fail(DVBT2LL_ERR_INVALID, err);
+    c->tr_built = true;
+  }
+  c->tr_iter = iterations; c->tr_vclip = vclip; c->tr_tone_max = tone_max;
   return 0;
 }
 

@@ -2095,4 +2095,209 @@ int launch_ofdm(const OfdmArgs &a0, cudaStream_t s)
   return 1 << a.lut_rep_shift;
 }
 
+// ================================================================================================
+// K6  tone-reservation PAPR reduction (peak cancellation on the reserved carriers, see PaprArgs)
+// ================================================================================================
+// One cluster of CL CTAs per (frame, symbol); CTA r keeps samples [r N/CL, (r+1) N/CL) of c in shared memory for the
+// whole iteration loop (32K: CL = 2, a 16K half each -- 256 KB do not fit one CTA).  Each iteration is one sweep over
+// the samples that applies the previous update and tracks the new maximum as the 64-bit key
+// float_bits(|c|^2) << 32 | (0xFFFFFFFF - n): the lowest index wins a tie, whatever the order of the reduction.  Warp
+// maxima meet by shared-memory atomics in their CTA; with CL = 2 each CTA then stores its maximum into its partner's slot
+// (DSMEM: a plain store -- there is no 64-bit max on the cluster's shared memory) and the key is the larger of the two.
+// Keys rotate over three slots so that a slot is cleared one iteration before it is filled again.  Every CTA takes the same decisions from the same data: the
+// reserved-carrier values R are kept (identically) in each.
+constexpr int PAPR_MAX_THREADS = 1024;
+
+// (not .aligned: the arrive follows a load whose address depends on the owner of c_m)
+__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release;\n" ::: "memory"); }
+__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire;\n" ::: "memory"); }
+__device__ __forceinline__ uint32_t cluster_rank()
+{
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
+  return r;
+}
+// generic address of the same shared-memory variable in CTA `rank` of the cluster
+template <class P>
+__device__ __forceinline__ P *cluster_map(P *p, uint32_t rank)
+{
+  uint64_t r;
+  asm volatile("mapa.u64 %0, %1, %2;\n" : "=l"(r) : "l"(reinterpret_cast<uint64_t>(p)), "r"(rank));
+  return reinterpret_cast<P *>(r);
+}
+
+template <int CL>
+__device__ __forceinline__ void papr_sync()
+{
+  if constexpr (CL == 1) __syncthreads();
+  else { cluster_arrive(); cluster_wait(); }
+}
+
+// slot[0]: this CTA's maximum; slot[1] (CL = 2): the partner's, stored there by the partner.  Visible to every CTA of
+// the cluster after the next papr_sync.
+template <int CL>
+__device__ __forceinline__ void papr_key_max(unsigned long long key, unsigned long long *slot, unsigned long long *rslot)
+{
+#pragma unroll
+  for (int o = 16; o; o >>= 1) key = max(key, __shfl_xor_sync(0xFFFFFFFFu, key, o));
+  if ((threadIdx.x & 31) == 0) atomicMax(slot, key);
+  if constexpr (CL == 2) {
+    __syncthreads();
+    if (threadIdx.x == 0) rslot[1] = slot[0];
+  }
+}
+
+__device__ __forceinline__ unsigned long long papr_key(float2 v, int n)
+{
+  const float p2 = v.x * v.x + v.y * v.y;
+  return ((unsigned long long)__float_as_uint(p2) << 32) | (0xFFFFFFFFu - (uint32_t)n);
+}
+
+template <int CL, int FMT>
+__global__ void __launch_bounds__(PAPR_MAX_THREADS) k_papr_tr(const PaprArgs a)
+{
+  extern __shared__ __align__(16) uint8_t smem_raw[];
+  const int N = a.fft_n, H = N / CL, S = a.tones, T = blockDim.x, tid = threadIdx.x;
+  float2 *c = reinterpret_cast<float2 *>(smem_raw);
+  float2 *R = c + H;
+  unsigned long long *keys = reinterpret_cast<unsigned long long *>(R + S);
+  const uint32_t rank = CL == 2 ? cluster_rank() : 0u;
+  unsigned long long *rkeys = CL == 2 ? cluster_map(keys, rank ^ 1u) : keys;      // [3][2], see papr_key_max
+  const int unit = blockIdx.x / CL, f = unit / a.num_symbols, l = unit - f * a.num_symbols;
+  const int set = __ldg(a.sym_set + l);
+  BND(set >= 0 && set < a.sets);
+  const float2 *kern = a.kernel + (long long)set * N;
+  const int32_t *bins = a.bins + (long long)set * S;
+  const long long sym0 = (long long)f * a.spf + 2048 + (long long)l * (N + a.gi);      // first CP sample
+  BND(a.in_len == 0 || sym0 + a.gi + N <= a.in_len);
+  const float2 *xin = a.in + sym0 + a.gi + (long long)rank * H;
+  const float V = a.vclip, A2 = a.tone_max * a.tone_max;
+
+  if (tid < 6) keys[tid] = 0ull;
+  for (int t = tid; t < S; t += T) R[t] = make_float2(0.f, 0.f);
+  papr_sync<CL>();      // the keys are cleared in every CTA before any of them adds to them
+
+  // sweep 0: load the CTA's samples
+  unsigned long long key = 0ull;
+  for (int j = tid; j < H; j += T) {
+    const float2 v = __ldg(xin + j);
+    c[j] = v;
+    key = max(key, papr_key(v, (int)rank * H + j));
+  }
+  papr_key_max<CL>(key, keys, rkeys);
+  papr_sync<CL>();
+
+  int applied = 0, reason = PAPR_STOP_LIMIT;
+  for (int it = 0;; it++) {
+    const unsigned long long K = CL == 2 ? max(keys[2 * (it % 3)], keys[2 * (it % 3) + 1]) : keys[2 * (it % 3)];
+    if (tid == 0) keys[2 * ((it + 2) % 3)] = 0ull;      // slot of iteration it + 1's sweep: nobody reads or fills it now
+    if (it == a.iterations) break;
+    const int m = (int)(0xFFFFFFFFu - (uint32_t)K);
+    BND(K != 0ull && m >= 0 && m < N);
+    const float y = sqrtf(__uint_as_float((uint32_t)(K >> 32)));
+    if (!(y > V)) { reason = PAPR_STOP_CLIP; break; }
+    const int owner = m / H;
+    const float2 cm = (CL == 1 || owner == (int)rank) ? c[m - owner * H] : cluster_map(c, (uint32_t)owner)[m - owner * H];
+    if constexpr (CL == 2) cluster_arrive();      // c_m is read: the owner may update it once everyone has arrived
+    const float s = (y - V) / y;
+    const float bx = s * cm.x, by = s * cm.y;
+    // the update's reserved-carrier values, dR_b = -beta exp(-j 2 pi b m / N) / (g |S|), checked against tone_max
+    bool bad = false;
+    for (int t = tid; t < S; t += T) {
+      const int b = __ldg(bins + t);
+      BND(b >= 0 && b < N);
+      const float2 e = __ldg(a.tone_tw + (int)(((long long)b * m) & (N - 1)));
+      const float2 r = make_float2(R[t].x - (bx * e.x - by * e.y) * a.tone_scale, R[t].y - (bx * e.y + by * e.x) * a.tone_scale);
+      bad |= r.x * r.x + r.y * r.y > A2;
+    }
+    bad = __syncthreads_or(bad);
+    if (bad) {
+      if constexpr (CL == 2) cluster_wait();
+      reason = PAPR_STOP_TONE;
+      break;
+    }
+    for (int t = tid; t < S; t += T) {
+      const int b = __ldg(bins + t);
+      const float2 e = __ldg(a.tone_tw + (int)(((long long)b * m) & (N - 1)));
+      R[t] = make_float2(R[t].x - (bx * e.x - by * e.y) * a.tone_scale, R[t].y - (bx * e.y + by * e.x) * a.tone_scale);
+    }
+    if constexpr (CL == 2) cluster_wait();
+    // sweep: c_n -= beta p[(n - m) mod N] -- the kernel table streams from L2 in order, wrapping once
+    key = 0ull;
+    const int k0 = (int)rank * H - m;
+    for (int j = tid; j < H; j += T) {
+      const float2 q = __ldg(kern + ((k0 + j) & (N - 1)));
+      float2 v = c[j];
+      v.x -= bx * q.x - by * q.y;
+      v.y -= bx * q.y + by * q.x;
+      c[j] = v;
+      key = max(key, papr_key(v, (int)rank * H + j));
+    }
+    papr_key_max<CL>(key, keys + 2 * ((it + 1) % 3), rkeys + 2 * ((it + 1) % 3));
+    applied++;
+    papr_sync<CL>();
+  }
+  if (rank == 0 && tid == 0) a.stats[unit] = (int16_t)(applied | reason << 8);
+
+  typedef typename SinkT<FMT>::type sample_t;
+  sample_t *sym = reinterpret_cast<sample_t *>(a.out) + sym0;
+  const float gain = a.gain;
+  if (!a.inplace || applied > 0) {
+    BND(a.out_len == 0 || sym0 + a.gi + N <= a.out_len);
+    const int cp_from = N - a.gi;
+    for (int j = tid; j < H; j += T) {
+      const int n = (int)rank * H + j;
+      float2 v = c[j];
+      if (!a.inplace) { v.x *= gain; v.y *= gain; }
+      store_sample(sym, a.gi + n, v);
+      if (n >= cp_from) store_sample(sym, n - cp_from, v);
+    }
+  }
+  if (!a.inplace && l == 0 && rank == 0) {
+    const float2 *p1 = a.in + (long long)f * a.spf;
+    sample_t *o = reinterpret_cast<sample_t *>(a.out) + (long long)f * a.spf;
+    for (int i = tid; i < 2048; i += T) {
+      float2 v = __ldg(p1 + i);
+      v.x *= gain; v.y *= gain;
+      store_sample(o, i, v);
+    }
+  }
+  if constexpr (CL == 2) papr_sync<CL>();      // no CTA leaves while its partner may still address its shared memory
+}
+
+template <int CL, int FMT>
+static void launch_papr_t(const PaprArgs &a, cudaStream_t s)
+{
+  const int H = a.fft_n / CL;
+  const int T = H >= 4096 ? PAPR_MAX_THREADS : (H / 4 < 256 ? 256 : H / 4);
+  const size_t smem = (size_t)H * sizeof(float2) + (size_t)a.tones * sizeof(float2) + 6 * sizeof(unsigned long long);
+  static bool attr[MAX_DEVICES];
+  allow_smem(k_papr_tr<CL, FMT>, 227 * 1024, attr);
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)(a.frames * a.num_symbols * CL));
+  cfg.blockDim = dim3((unsigned)T);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  cudaLaunchKernelEx(&cfg, k_papr_tr<CL, FMT>, a);
+  count_launch();
+}
+
+void launch_papr_tr(const PaprArgs &a, cudaStream_t s)
+{
+  if (a.frames * a.num_symbols < 1) return;
+  if (a.fft_n > 16384) {
+    if (a.out_fmt) launch_papr_t<2, 1>(a, s);
+    else launch_papr_t<2, 0>(a, s);
+  }
+  else {
+    if (a.out_fmt) launch_papr_t<1, 1>(a, s);
+    else launch_papr_t<1, 0>(a, s);
+  }
+}
+
 } // namespace t2k

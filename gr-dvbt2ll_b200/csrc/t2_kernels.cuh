@@ -173,6 +173,34 @@ int ofdm_position_of_bin(int m, int log2_m);
 // index inside the per-(symbol, phase) tables at which the entry of position p is kept
 int ofdm_table_index(int p, int log2_m);
 
+// ---- K6: tone-reservation PAPR reduction on the reserved carriers (chain, opt-in) ------------------------------------
+// Per OFDM symbol (P1 untouched), with x = the symbol's useful samples, p = the kernel of its reserved set S:
+//   c = x; repeat up to `iterations` times: m = argmax |c_m|^2 (lowest index on ties); y = |c_m|; stop if y <= vclip;
+//   beta = (y - vclip) c_m / y; stop if a reserved carrier would exceed tone_max; c_n -= beta p[(n - m) mod N].
+// Output: [last gi samples of c | c] in the sink format.
+struct PaprArgs {
+  const float2 *in;          // complex64 samples at gain 1 (k_ofdm's output), T2 frames spf samples apart
+  void *out;                 // the same layout in the sink format; == in for the in-place form
+  int out_fmt;               // 0 = complex64, 1 = interleaved int16 I/Q (round(gain * c * 32767), saturated)
+  float gain;                // sink gain (1 in the in-place form)
+  int inplace;               // 1: out == in, complex64, gain 1: symbols without an update and P1 are not rewritten
+  long long spf;             // samples per T2 frame
+  int fft_n, gi, num_symbols, frames;
+  int iterations;            // 1..64
+  float vclip, tone_max;     // clip magnitude (units of x), bound of a reserved carrier (bin units)
+  float tone_scale;          // 1 / (normalization * tones)
+  int tones;                 // |S|
+  const int32_t *sym_set;    // [num_symbols] set of each symbol
+  const int32_t *bins;       // [sets][tones]
+  const float2 *kernel;      // [sets][fft_n]
+  const float2 *tone_tw;     // [fft_n] exp(-j 2 pi i / N)
+  int16_t *stats;            // [frames][num_symbols]: updates applied | stop reason << 8 (PAPR_STOP_*)
+  int sets;
+  long long in_len, out_len; // samples behind in / out (debug build bounds checks; 0 = not checked)
+};
+enum { PAPR_STOP_CLIP = 1, PAPR_STOP_TONE = 2, PAPR_STOP_LIMIT = 3 };
+void launch_papr_tr(const PaprArgs &a, cudaStream_t s);
+
 long long kernel_launch_count();
 
 } // namespace t2k

@@ -221,6 +221,18 @@ struct OfdmPlan {
 };
 bool build_ofdm_plan(const OfdmParams &prm, OfdmPlan *p, std::string *err);
 
+// Tone-reservation PAPR reduction (beyond the reference, which leaves the reserved carriers at zero): the reserved
+// carriers of each symbol (P2PAPR_CARRIER / TRPAPR_CARRIER of carrier_type) as FFT bins, one entry per distinct set
+// (P2 and frame-closing symbols share one, the data symbols' are one base set shifted by dx * s: at most dy + 1).
+struct PaprTrPlan {
+  int sets, tones;                     // distinct sets, reserved carriers per set
+  std::vector<int32_t> sym_set;        // [num_symbols] set of each symbol
+  std::vector<int32_t> bins;           // [sets][tones] FFT bins (k + left_nulls + N/2) mod N, carrier order
+  std::vector<cfloat> kernel;          // [sets][N] p_n = (1/tones) sum_b exp(+j 2 pi b n / N), p_0 = 1
+  std::vector<cfloat> tone_tw;         // [N] exp(-j 2 pi i / N)
+};
+bool build_papr_tr_plan(const OfdmPlan &op, PaprTrPlan *p, std::string *err);
+
 // Chain mode: compose frame plan and OFDM plan into one per-carrier code table whose non-negative
 // entries index the natural-order cells produced by the mapper kernel, and merge the pools.
 struct ChainTables {

@@ -39,6 +39,7 @@ EXPORTED_SYMBOLS = [
     "dvbt2ll_stream_create", "dvbt2ll_stream_destroy", "dvbt2ll_stream_synchronize",
     "dvbt2ll_chain_create_multiplp", "dvbt2ll_chain_num_plp", "dvbt2ll_chain_plp_ts_bytes",
     "dvbt2ll_chain_history_bytes", "dvbt2ll_ts_sync", "dvbt2ll_ts_fill", "dvbt2ll_chain_create_plps",
+    "dvbt2ll_chain_set_papr_tr",
 ]
 GATHER_BLOB_BYTES = 256
 
@@ -105,6 +106,7 @@ def lib():
         L.dvbt2ll_chain_stage_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.dvbt2ll_chain_enable_timing.argtypes = [vp, ci]
         L.dvbt2ll_chain_set_sink.argtypes = [vp, ci, C.c_float]
+        L.dvbt2ll_chain_set_papr_tr.argtypes = [vp, ci, C.c_float, C.c_float]
         L.dvbt2ll_set_overfull_policy.argtypes = [ci]
         L.dvbt2ll_set_overfull_policy.restype = None
         L.dvbt2ll_set_host_register.argtypes = [vp, ci]
@@ -442,6 +444,15 @@ class Chain(_Block):
             raise ValueError(last_error())
         self.sink_format = int(fmt)
 
+    def set_papr_tr(self, iterations, vclip, tone_max):
+        """Tone-reservation PAPR reduction on the reserved carriers (paprmode TR or BOTH): up to `iterations` (1..64)
+        peak cancellations per OFDM symbol down to the sample magnitude `vclip` (units of the complex64 output at gain
+        1), no reserved carrier above `tone_max` (data cells have unit mean power); iterations = 0 switches it off.
+        The "papr" tap then holds updates applied | stop reason << 8 per (channel, frame, symbol)."""
+        r = lib().dvbt2ll_chain_set_papr_tr(self._h, int(iterations), float(vclip), float(tone_max))
+        if r < 0:
+            raise ValueError(last_error())
+
     def history_bytes(self, first_frame):
         """Stream bytes that must precede the first TS byte of `first_frame` in every row handed to run_host():
         187 in normal input mode once the stream has started (CRC-8 of the packet in flight), else 0."""
@@ -477,7 +488,8 @@ class Chain(_Block):
         return r
 
     def tap(self, stage, dtype=np.uint8):
-        """Stage output of the most recent run: "bch", "fec", "cells", or one PLP's codewords "bch.<p>" / "fec.<p>"."""
+        """Stage output of the most recent run: "bch", "fec", "cells", one PLP's codewords "bch.<p>" / "fec.<p>", or the
+        tone-reservation counts "papr" (int16)."""
         n = lib().dvbt2ll_chain_tap(self._h, stage.encode(), None, 0)
         if n < 0:
             raise RuntimeError(last_error())

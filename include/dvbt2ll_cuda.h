@@ -162,8 +162,23 @@ DVBT2LL_API_EXPORT int dvbt2ll_chain_set_sink(dvbt2ll_handle *h, int format, flo
  * first cell in the frame, first cell in this memory).  Copies to HOST; returns
  * bytes or negative error. */
 DVBT2LL_API_EXPORT long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, long long cap);
+/* Tone-reservation PAPR reduction (EN 302 755 9.6.2, peak-cancellation form; beyond the reference, which sends the
+ * reserved carriers as zeros).  Needs paprmode PAPR_TR or PAPR_BOTH.  iterations = 0 switches the stage off (the
+ * default), 1..64 switches it on; vclip (a sample magnitude in the units of the complex64 output at gain 1) and tone_max
+ * (the largest magnitude of a reserved carrier, in the units where data cells have unit mean power) must be finite and
+ * > 0.  Per OFDM symbol (P1 untouched), with x the useful samples and p_n = (1/|S|) sum_{b in S} exp(+j 2 pi b n / N)
+ * the kernel of its reserved bins S: c = x; up to `iterations` times: m = argmax |c_m| (lowest m on equal float
+ * values), y = |c_m|, stop if y <= vclip; beta = (y - vclip) c_m / y; stop, without this update, if a reserved carrier
+ * R_b - beta exp(-j 2 pi b m / N) / (normalization |S|) would exceed tone_max; c_n -= beta p_{(n - m) mod N}.  Only
+ * the reserved carriers change.  The symbol is then [last GI samples of c | c], through the sink.  Builds the tables
+ * on the host (dvbt2ll_plan_get "ofdm.tr_set": int32 set per symbol, "ofdm.tr_bins": int32 [sets][|S|] FFT bins,
+ * "ofdm.tr_kernel": complex64 [sets][N]); may be called between runs.  Tap "papr": one int16 per (channel, frame,
+ * symbol) of the last run, updates applied | stop reason << 8 (1 = clip reached, 2 = tone_max, 3 = iteration limit);
+ * refused while the stage is off. */
+DVBT2LL_API_EXPORT int dvbt2ll_chain_set_papr_tr(dvbt2ll_handle *h, int iterations, float vclip, float tone_max);
 /* Device time in ms of each stage kernel (bb_bch, ldpc, map, ofdm, total), averaged over the chain runs issued since
- * timing was enabled (at most the last 64); events are recorded per run, so the caller's timed loop needs no sync. */
+ * timing was enabled (at most the last 64); events are recorded per run, so the caller's timed loop needs no sync.
+ * With tone reservation on, "ofdm" covers k_ofdm and the tone-reservation kernel after it. */
 DVBT2LL_API_EXPORT int dvbt2ll_chain_stage_ms(dvbt2ll_handle *h, float *ms5);
 DVBT2LL_API_EXPORT void dvbt2ll_chain_enable_timing(dvbt2ll_handle *h, int on);
 
