@@ -8,12 +8,15 @@
 // of `batch` T2 frames per call (stream position carried by first_frame + the 187 history bytes in front of a batch).
 //
 // usage: t2_file_modulator [--config c1|c2|c3|c4] [--plp-blocks a,b,..] [--plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]]...
-//                          [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] --out FILE  TS_FILE [TS_FILE ...]
+//                          [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] [--miso 1|2|both [--out2 FILE2]]
+//                          --out FILE  TS_FILE [TS_FILE ...]
 // --plp, once per PLP: its FEC blocks per T2 frame and, optionally, its own FEC type, code rate, constellation and
 // rotation (enum values of dvbt2ll_config.h; the config's where omitted).
 // --papr-tr: paprmode = PAPR_TR and tone-reservation PAPR reduction on the reserved carriers (dvbt2ll_chain_set_papr_tr).
 // The reserved carriers take cells away: a config whose FEC blocks no longer fit is refused as over-full; lower its
 // block count with --plp BLOCKS (c1: 7, c3: 200, c4: 119; c2 fits as it is).
+// --miso: preamble = T2_MISO; 1 or 2 emits that transmitter group (2 with MISO processing, dvbt2ll_chain_set_miso);
+// both writes group 1 to --out and group 2 to --out2 from one FEC pass (dvbt2ll_chain_run_host_miso).
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -55,7 +58,7 @@ std::vector<unsigned char> read_file(const char *path)
 
 int main(int argc, char **argv)
 {
-  std::string cfg = "c1", out_path;
+  std::string cfg = "c1", out_path, out2_path, miso;
   std::vector<int> plp_blocks;
   std::vector<dvbt2ll_plp_params> plps;
   std::vector<int> plp_own;          // --plp entries that name their own parameters
@@ -68,6 +71,8 @@ int main(int argc, char **argv)
     std::string a = argv[i];
     if (a == "--config" && i + 1 < argc) cfg = argv[++i];
     else if (a == "--out" && i + 1 < argc) out_path = argv[++i];
+    else if (a == "--out2" && i + 1 < argc) out2_path = argv[++i];
+    else if (a == "--miso" && i + 1 < argc) miso = argv[++i];
     else if (a == "--frames" && i + 1 < argc) frames = std::atoi(argv[++i]);
     else if (a == "--batch" && i + 1 < argc) batch = std::atoi(argv[++i]);
     else if (a == "--sc16" && i + 1 < argc) { sc16 = 1; gain = (float)std::atof(argv[++i]); }
@@ -91,8 +96,9 @@ int main(int argc, char **argv)
     else inputs.push_back(argv[i]);
   }
   dvbt2ll_chain_params prm;
-  if (!named_config(cfg, &prm) || out_path.empty() || inputs.empty() || batch < 1 || (!plps.empty() && !plp_blocks.empty())) {
-    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] --out FILE TS_FILE...\n", argv[0]);
+  const bool miso_ok = miso.empty() ? out2_path.empty() : (miso == "both") == !out2_path.empty() && (miso == "1" || miso == "2" || miso == "both");
+  if (!named_config(cfg, &prm) || out_path.empty() || inputs.empty() || batch < 1 || (!plps.empty() && !plp_blocks.empty()) || !miso_ok) {
+    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] [--miso 1|2|both [--out2 FILE2]] --out FILE TS_FILE...\n", argv[0]);
     return 2;
   }
   bool own = false;
@@ -106,11 +112,13 @@ int main(int argc, char **argv)
   if ((int)inputs.size() != P) { std::fprintf(stderr, "one TS file per PLP expected (%d)\n", P); return 2; }
   if (P == 1 && !own && !plps.empty()) prm.fecblocks = plps[0].fecblocks;
   if (tr_iter) prm.paprmode = 2;      // PAPR_TR
+  if (!miso.empty()) { prm.preamble = 1; prm.misogroup = miso == "2" ? 1 : 0; }      // PREAMBLE_T2_MISO, MISO_TX1 / TX2
   dvbt2ll_handle *h = own ? dvbt2ll_chain_create_plps(&prm, P, plps.data(), batch, -1)
                     : P == 1 ? dvbt2ll_chain_create(&prm, batch, -1) : dvbt2ll_chain_create_multiplp(&prm, P, plp_blocks.data(), batch, -1);
   if (!h) { std::fprintf(stderr, "chain: %s\n", dvbt2ll_last_error()); return 1; }
   if (sc16 && dvbt2ll_chain_set_sink(h, 1, gain) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }
   if (tr_iter && dvbt2ll_chain_set_papr_tr(h, tr_iter, tr_vclip, tr_tone_max) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }
+  if (!miso.empty() && dvbt2ll_chain_set_miso(h, 1) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }
 
   // ---- ingest: sync acquisition per file; whole T2 frames available = limited by the shortest PLP (then null filled)
   std::vector<std::vector<unsigned char> > ts(P);
@@ -131,7 +139,9 @@ int main(int argc, char **argv)
   const size_t ssz = sc16 ? 4 : 8;
   FILE *fo = std::fopen(out_path.c_str(), "wb");
   if (!fo) { std::fprintf(stderr, "cannot write %s\n", out_path.c_str()); return 1; }
-  std::vector<unsigned char> out((size_t)batch * S * ssz), rows;
+  FILE *fo2 = 0;
+  if (!out2_path.empty() && !(fo2 = std::fopen(out2_path.c_str(), "wb"))) { std::fprintf(stderr, "cannot write %s\n", out2_path.c_str()); return 1; }
+  std::vector<unsigned char> out((size_t)batch * S * ssz), out2(fo2 ? out.size() : 0), rows;
   long long nulls = 0;
   for (int f0 = 0; f0 < frames; f0 += batch) {
     const int n = frames - f0 < batch ? frames - f0 : batch;
@@ -145,11 +155,14 @@ int main(int argc, char **argv)
       // [pos - hist, pos + len) of the aligned stream, null packets where the file has ended
       nulls += dvbt2ll_ts_fill(rows.data() + pitch * p, (size_t)(hist + len), ts[p].data() + start[p], ts[p].size() - start[p], pos - hist);
     }
-    const int r = dvbt2ll_chain_run_host(h, rows.data() + hist, (long long)pitch, 1, n, f0, out.data());
+    const int r = fo2 ? dvbt2ll_chain_run_host_miso(h, rows.data() + hist, (long long)pitch, 1, n, f0, out.data(), out2.data())
+                      : dvbt2ll_chain_run_host(h, rows.data() + hist, (long long)pitch, 1, n, f0, out.data());
     if (r < 0) { std::fprintf(stderr, "chain: %s\n", dvbt2ll_last_error()); return 1; }
     std::fwrite(out.data(), ssz, (size_t)n * S, fo);
+    if (fo2) std::fwrite(out2.data(), ssz, (size_t)n * S, fo2);
   }
   std::fclose(fo);
+  if (fo2) std::fclose(fo2);
   std::printf("%d T2 frame(s), %lld samples, %lld null-packet bytes inserted, %lld kernel launches\n", frames, (long long)frames * S, nulls,
               dvbt2ll_kernel_launches());
   dvbt2ll_destroy(h);

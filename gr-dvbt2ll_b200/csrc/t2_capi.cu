@@ -664,9 +664,10 @@ struct OfdmDevice {
   // c16: `code` holds staging slots (chain mode, 16-bit cells) and is re-encoded as the chain-mode carrier codes of
   // t2_kernels.cuh (2 * slot | (small pool cell + 1) << 17 | 0x80000000 + pool cell) for the kernel's branch-free fill;
   // with tab_base (several constellation tables) a data carrier's code also carries the first table entry of its cell's
-  // PLP, tab_base[plp[carrier]] << OFDM_CODE_TAB_SHIFT
+  // PLP, tab_base[plp[carrier]] << OFDM_CODE_TAB_SHIFT; with miso (MISO group-2 codes, t2::compose_miso) a data carrier
+  // whose cell sits at an odd place i of its symbol (op.code - op.sym_data_start) also carries OFDM_CODE_MISO_IM
   int init(const std::vector<int32_t> &code, const t2::CellPool &pool, const t2::OfdmPlan &op, bool c16 = false,
-           const std::vector<uint8_t> *plp = 0, const int *tab_base = 0)
+           const std::vector<uint8_t> *plp = 0, const int *tab_base = 0, bool miso = false)
   {
     // one copy of the pool per L1-post variant: in copy v the L1-post slot holds variant v, so the kernel
     // selects a pool base per frame instead of patching indices per cell
@@ -706,6 +707,7 @@ struct OfdmDevice {
               if (v >= 65536) return fail(DVBT2LL_ERR_INVALID, "chain: staging slot out of range");
               v = 2 * v;
               if (tab_base) v |= tab_base[(*plp)[(size_t)l * cps + k]] << t2k::OFDM_CODE_TAB_SHIFT;
+              if (miso && ((op.code[(size_t)l * cps + k] - op.sym_data_start[l]) & 1)) v |= t2k::OFDM_CODE_MISO_IM;
             }
             else if (~v < 8) v = (~v + 1) << 17;
             else { v = (int32_t)(0x80000000u | (uint32_t)(~v)); sym_flags[l] = 1; }
@@ -738,6 +740,7 @@ struct OfdmDevice {
     a.out_fmt = 0; a.sink_gain = 1.0f;
     a.cells_len = 0; a.out_len = 0; a.pool_len = pool_stride;
     a.lut_tables = 1;
+    a.miso = 0;
   }
 };
 
@@ -838,13 +841,18 @@ struct ChainHandle : dvbt2ll_handle {
   t2::PaprTrPlan tr;
   DevBuf d_tr_set, d_tr_bins, d_tr_kernel, d_tr_tw, d_tr_stats, d_tr_scratch;
   int tr_frames;         // frames whose counts the last run left in d_tr_stats (the "papr" tap)
+  // MISO processing (dvbt2ll_chain_set_miso, dvbt2ll_chain_run_*_miso), built at first use: the pilot plan, carrier
+  // tables and device tables of group g (0: TX1, 1: TX2 with MISO processing) over the chain's staging
+  struct MisoGroup { t2::OfdmPlan op; t2::MisoTables tab; OfdmDevice dev; bool uploaded = false; };
+  std::unique_ptr<MisoGroup> miso_g[2];
+  bool miso_on;
   int last_frames;
   long long next_frame;  // stream position of the generic work() / work_device() path (T2 frames consumed so far)
   bool timing;
   enum { TIMING_SLOTS = 64 };
   cudaEvent_t ev[TIMING_SLOTS][5];     // per-run event sets so the timed loop never has to synchronise
   long long n_timed;
-  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), tr_iter(0), tr_vclip(0.f), tr_tone_max(0.f), tr_built(false), tr_uploaded(false), tr_frames(0), last_frames(0), next_frame(0), timing(false)
+  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), tr_iter(0), tr_vclip(0.f), tr_tone_max(0.f), tr_built(false), tr_uploaded(false), tr_frames(0), miso_on(false), last_frames(0), next_frame(0), timing(false)
   {
     n_timed = 0;
     for (int s = 0; s < TIMING_SLOTS; s++) for (int i = 0; i < 5; i++) ev[s][i] = 0;
@@ -947,12 +955,25 @@ struct ChainHandle : dvbt2ll_handle {
   }
   // buf_frame: first T2-frame slot of the intermediate buffers to use; hist_valid < 0: history is present iff
   // first_frame > 0; tr_frame0: position of the batch's first frame in the tone-reservation counts (d_tr_stats)
+  // d_out2 != NULL: MISO group 1 to d_out and group 2 with MISO processing to d_out2, from one pass of the front end
   int run(const void *d_ts, long long ts_pitch, int n_channels, int n_frames, long long first_frame, void *d_out, cudaStream_t s,
-          int buf_frame = 0, int hist_valid = -1, int tr_frame0 = 0)
+          int buf_frame = 0, int hist_valid = -1, int tr_frame0 = 0, void *d_out2 = 0)
   {
     const int frames = n_channels * n_frames;
     if (frames < 1) return 0;
     if (buf_frame + frames > max_frames) return fail(DVBT2LL_ERR_INVALID, "chain: batch larger than max_frames given at create");
+    // the OFDM carrier tables of each output: the chain's own, or a MISO group's
+    const MisoGroup *g1 = 0, *g2 = 0;
+    if (d_out2 || miso_group2_out()) {
+      int r = miso_upload(1);
+      if (r) return r;
+      g2 = miso_g[1].get();
+      if (d_out2 && oplan.prm.misogroup != t2::MISO_TX1) {
+        if ((r = miso_upload(0))) return r;
+        g1 = miso_g[0].get();
+      }
+      if (!d_out2) { g1 = g2; g2 = 0; }
+    }
     const int nfec = frames * F();
     const int bp = align16(bb.plan.fec.nbch / 8), fp = align16(bb.plan.fec.nldpc / 8);
     cudaEvent_t *tev = ev[n_timed % TIMING_SLOTS];
@@ -1009,7 +1030,8 @@ struct ChainHandle : dvbt2ll_handle {
       }
     }
     t2k::OfdmArgs oa;
-    odev.fill(oa, oplan, tables.pool);
+    if (g1) { g1->dev.fill(oa, g1->op, g1->tab.pool); oa.miso = g1 == miso_g[1].get(); }
+    else odev.fill(oa, oplan, tables.pool);
     oa.cells = 0; oa.cells_stride = cells16_stride();
     oa.cells16 = cell_buf; oa.run_desc = d_run_desc.as<int2>(); oa.run_ptr = d_run_ptr.as<int32_t>();
     oa.run_cnt = d_run_cnt.as<int32_t>(); oa.desc_cap = (tables.max_runs + 2) & ~1;
@@ -1023,6 +1045,14 @@ struct ChainHandle : dvbt2ll_handle {
     oa.frames = frames; oa.frames_per_channel = n_frames;
     oa.frame_idx0 = (int)(first_frame % (tables.pool.l1post_variants > 0 ? tables.pool.l1post_variants : 1));
     lut_copies = t2k::launch_ofdm(oa, s);
+    if (g2) {
+      // group 2: the same cells, its own pilots and pool, the MISO form of the fill
+      t2k::OfdmArgs o2 = oa;
+      o2.code_pos = g2->dev.d_code.as<int32_t>(); o2.pool = g2->dev.d_pool.as<float2>(); o2.sym_flags = g2->dev.d_sym_flags.as<int32_t>();
+      o2.out = d_out2;
+      o2.miso = 1;
+      t2k::launch_ofdm(o2, s);
+    }
     if (tr_on) {
       t2k::PaprArgs pa;
       pa.in = (const float2 *)ofdm_out; pa.out = d_out;
@@ -1042,6 +1072,32 @@ struct ChainHandle : dvbt2ll_handle {
     CK(cudaGetLastError());
     if (buf_frame == 0) last_frames = frames;
     return frames;
+  }
+  bool miso_preamble() const { return oplan.prm.preamble == t2::PREAMBLE_T2_MISO || oplan.prm.preamble == t2::PREAMBLE_T2_LITE_MISO; }
+  // set_miso(1) on a group-2 chain: run() emits group 2 with MISO processing
+  bool miso_group2_out() const { return miso_on && oplan.prm.misogroup == t2::MISO_TX2; }
+  // host tables of MISO group g (refused for a symbol with an odd cell count)
+  int miso_build(int g)
+  {
+    if (miso_g[g]) return 0;
+    std::unique_ptr<MisoGroup> m(new MisoGroup());
+    t2::OfdmParams op = oplan.prm;
+    op.misogroup = g ? t2::MISO_TX2 : t2::MISO_TX1;
+    std::string err;
+    if (!t2::build_ofdm_plan(op, &m->op, &err) || !t2::compose_miso(oplan, tables, m->op, g == 1, &m->tab, &err))
+      return fail(DVBT2LL_ERR_INVALID, err);
+    miso_g[g] = std::move(m);
+    return 0;
+  }
+  int miso_upload(int g)
+  {
+    int r = miso_build(g);
+    if (r) return r;
+    MisoGroup &m = *miso_g[g];
+    if (m.uploaded) return 0;
+    if ((r = m.dev.init(m.tab.code, m.tab.pool, m.op, true, &m.tab.plp, lut_tables > 1 ? lut_base : 0, g == 1))) return r;
+    m.uploaded = true;
+    return 0;
   }
   int tr_upload()
   {
@@ -1131,6 +1187,8 @@ struct ChainHandle : dvbt2ll_handle {
       return copy_out(v, sizeof(int) * (3 + fplan.num_plp), out, cap);
     }
     if (n == "frame.fi_src") return copy_vec(fplan.fi_src, out, cap);
+    if (miso_g[1] && n == "chain.miso_code") return copy_vec(miso_g[1]->tab.code, out, cap);
+    if (miso_g[1] && n == "chain.miso_pool") return copy_vec(miso_g[1]->tab.pool.cells, out, cap);
     if (tr_built && n == "ofdm.tr_set") return copy_vec(tr.sym_set, out, cap);
     if (tr_built && n == "ofdm.tr_bins") return copy_vec(tr.bins, out, cap);
     if (tr_built && n == "ofdm.tr_kernel") return copy_vec(tr.kernel, out, cap);
@@ -1671,27 +1729,32 @@ long long dvbt2ll_chain_plp_ts_bytes(const dvbt2ll_handle *h, int plp, long long
 long long dvbt2ll_chain_samples_per_frame(const dvbt2ll_handle *h) { ChainHandle *c = as_chain(h); return c ? c->oplan.samples_per_frame : -1; }
 int dvbt2ll_chain_fecframes_per_frame(const dvbt2ll_handle *h) { ChainHandle *c = as_chain(h); return c ? c->F() : -1; }
 
-int dvbt2ll_chain_run_device(dvbt2ll_handle *h, const void *d_ts, long long ts_pitch, int n_channels, int n_frames,
-                             long long first_frame, void *d_out, void *stream)
+// d_out2 != NULL: MISO group 1 to d_out and group 2 to d_out2 (dvbt2ll_chain_run_device_miso)
+static int chain_run_device(ChainHandle *c, const void *d_ts, long long ts_pitch, int n_channels, int n_frames,
+                            long long first_frame, void *d_out, void *d_out2, void *stream)
 {
-  ChainHandle *c = as_chain(h);
-  if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
   int r = c->enter();
   if (r) return r;
   if (n_channels < 0 || n_frames < 0) return fail(DVBT2LL_ERR_INVALID, "chain: negative batch size");
   if (n_channels == 0 || n_frames == 0) return 0;
   if (c->P() > 1 && ts_pitch < c->ts_bytes_max(first_frame, n_frames))
     return fail(DVBT2LL_ERR_INVALID, "chain: with several PLPs the TS rows (channel * num_plp + plp) need a pitch of at least the longest PLP's bytes");
-  return c->run(d_ts, ts_pitch, n_channels, n_frames, first_frame, d_out, stream ? (cudaStream_t)stream : c->stream);
+  return c->run(d_ts, ts_pitch, n_channels, n_frames, first_frame, d_out, stream ? (cudaStream_t)stream : c->stream, 0, -1, 0, d_out2);
 }
 
-int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch, int n_channels, int n_frames,
-                           long long first_frame, void *out)
+int dvbt2ll_chain_run_device(dvbt2ll_handle *h, const void *d_ts, long long ts_pitch, int n_channels, int n_frames,
+                             long long first_frame, void *d_out, void *stream)
 {
   ChainHandle *c = as_chain(h);
   if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
-  int r = c->enter();
-  if (r) return r;
+  return chain_run_device(c, d_ts, ts_pitch, n_channels, n_frames, first_frame, d_out, 0, stream);
+}
+
+// out2 != NULL: MISO group 1 to out and group 2 to out2 (dvbt2ll_chain_run_host_miso)
+static int chain_run_host(ChainHandle *c, const void *ts, long long ts_pitch, int n_channels, int n_frames,
+                          long long first_frame, void *out, void *out2)
+{
+  int r;
   if (n_channels < 0 || n_frames < 0) return fail(DVBT2LL_ERR_INVALID, "chain: negative batch size");
   if (n_channels == 0 || n_frames == 0) return 0;
   const int P = c->P();                      // TS rows per channel (row = channel * P + plp)
@@ -1705,9 +1768,9 @@ int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch
   const size_t ssz = c->sink_fmt ? 4 : 8;                                        // bytes per output sample
   const size_t out_bytes = (size_t)n_channels * n_frames * c->oplan.samples_per_frame * ssz;
   CK(c->d_ts_stage.ensure((size_t)n_channels * P * dpitch + 512));
-  CK(c->d_out_stage.ensure(out_bytes));
+  CK(c->d_out_stage.ensure(out2 ? 2 * out_bytes : out_bytes));
   uint8_t *base = c->d_ts_stage.as<uint8_t>() + 256;
-  uint8_t *dout = c->d_out_stage.as<uint8_t>();
+  uint8_t *dout = c->d_out_stage.as<uint8_t>(), *dout2 = dout + out_bytes;
   const size_t ch_out = (size_t)n_frames * c->oplan.samples_per_frame;          // samples per channel
   // host layout: channel-major with pitch ts_pitch; when first_frame > 0 each channel pointer must be preceded
   // by 187 history bytes.  Channels are processed in groups on two streams so that the H2D copy and the
@@ -1726,14 +1789,56 @@ int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch
     CK(cudaMemcpy2DAsync(base + (size_t)c0 * P * dpitch - hist, (size_t)dpitch, (const uint8_t *)ts + (size_t)c0 * P * ts_pitch - hist,
                          (size_t)ts_pitch, (size_t)(per_ch + hist), (size_t)nc * P, cudaMemcpyHostToDevice, s));
     r = c->run(base + (size_t)c0 * P * dpitch, dpitch, nc, n_frames, first_frame, dout + (size_t)c0 * ch_out * ssz, s,
-               groups == 1 ? 0 : (gi & 1) * per * n_frames, -1, c0 * n_frames);
+               groups == 1 ? 0 : (gi & 1) * per * n_frames, -1, c0 * n_frames, out2 ? dout2 + (size_t)c0 * ch_out * ssz : 0);
     if (r < 0) return r;
     CK(cudaMemcpyAsync((uint8_t *)out + (size_t)c0 * ch_out * ssz, dout + (size_t)c0 * ch_out * ssz, (size_t)nc * ch_out * ssz,
                        cudaMemcpyDeviceToHost, s));
+    if (out2)
+      CK(cudaMemcpyAsync((uint8_t *)out2 + (size_t)c0 * ch_out * ssz, dout2 + (size_t)c0 * ch_out * ssz, (size_t)nc * ch_out * ssz,
+                         cudaMemcpyDeviceToHost, s));
   }
   CK(cudaStreamSynchronize(c->stream));
   CK(cudaStreamSynchronize(c->stream2));
   return n_channels * n_frames;
+}
+
+int dvbt2ll_chain_run_host(dvbt2ll_handle *h, const void *ts, long long ts_pitch, int n_channels, int n_frames,
+                           long long first_frame, void *out)
+{
+  ChainHandle *c = as_chain(h);
+  if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
+  int r = c->enter();
+  if (r) return r;
+  return chain_run_host(c, ts, ts_pitch, n_channels, n_frames, first_frame, out, 0);
+}
+
+// the dual MISO calls: a MISO preamble, tone reservation off, both outputs given
+static int miso_dual_check(ChainHandle *c, const void *out1, const void *out2)
+{
+  if (!c->miso_preamble()) return fail(DVBT2LL_ERR_INVALID, "chain: MISO outputs need preamble T2_MISO or T2_LITE_MISO");
+  if (c->tr_iter > 0) return fail(DVBT2LL_ERR_INVALID, "chain: the MISO dual call does not apply tone reservation; switch it off");
+  if (!out1 || !out2) return fail(DVBT2LL_ERR_INVALID, "chain: the MISO dual call needs both outputs");
+  return c->miso_build(1);
+}
+
+int dvbt2ll_chain_run_device_miso(dvbt2ll_handle *h, const void *d_ts, long long ts_pitch, int n_channels, int n_frames,
+                                  long long first_frame, void *d_out1, void *d_out2, void *stream)
+{
+  ChainHandle *c = as_chain(h);
+  if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
+  const int r = miso_dual_check(c, d_out1, d_out2);
+  return r ? r : chain_run_device(c, d_ts, ts_pitch, n_channels, n_frames, first_frame, d_out1, d_out2, stream);
+}
+
+int dvbt2ll_chain_run_host_miso(dvbt2ll_handle *h, const void *ts, long long ts_pitch, int n_channels, int n_frames,
+                                long long first_frame, void *out1, void *out2)
+{
+  ChainHandle *c = as_chain(h);
+  if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
+  int r = miso_dual_check(c, out1, out2);
+  if (r) return r;
+  if ((r = c->enter())) return r;
+  return chain_run_host(c, ts, ts_pitch, n_channels, n_frames, first_frame, out1, out2);
 }
 
 long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, long long cap)
@@ -1806,6 +1911,19 @@ int dvbt2ll_chain_set_papr_tr(dvbt2ll_handle *h, int iterations, float vclip, fl
     c->tr_built = true;
   }
   c->tr_iter = iterations; c->tr_vclip = vclip; c->tr_tone_max = tone_max;
+  return 0;
+}
+
+int dvbt2ll_chain_set_miso(dvbt2ll_handle *h, int on)
+{
+  ChainHandle *c = as_chain(h);
+  if (!c) return fail(DVBT2LL_ERR_INVALID, "not a chain handle");
+  if (!c->miso_preamble()) return fail(DVBT2LL_ERR_INVALID, "chain: MISO processing needs preamble T2_MISO or T2_LITE_MISO");
+  if (on) {
+    const int r = c->miso_build(1);
+    if (r) return r;
+  }
+  c->miso_on = on != 0;
   return 0;
 }
 

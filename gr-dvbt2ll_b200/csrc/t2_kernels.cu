@@ -1611,7 +1611,8 @@ struct FillSmem {
 // `c` holds the codes of the thread's first batch (loaded by the caller ahead of the barrier that precedes the fill);
 // the codes of batch n + 1 are fetched while batch n is processed.
 // MT: the carrier codes carry the first entry of their constellation table (several tables, see OFDM_CODE_TAB_SHIFT).
-template <int LOG2M, int T, bool C16, bool POOL, bool SINC, bool MT = false>
+// MISO: MISO group-2 carrier codes, bit 0 of a data code selects the component whose sign flips (OFDM_CODE_MISO_IM).
+template <int LOG2M, int T, bool C16, bool POOL, bool SINC, bool MT = false, bool MISO = false>
 __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__ code, const float *__restrict__ sinc,
                                           int (&c)[FillGeom<LOG2M, T>::GPB][FillGeom<LOG2M, T>::R0], const float2 *__restrict__ cells,
                                           const float2 *__restrict__ pool, const FillSmem fs, int stage_cap_dbg = 0, int lut_n_dbg = 0)
@@ -1629,7 +1630,7 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
         if (C16) {
           // data cell: 16-bit code from the staging area through the LUT (a dummy read of offset 0 for the others);
           // small pool cell (null, pilots): (p + 1) << 17 -> spool[p]; big pool cell: sign bit set (POOL symbols only)
-          const unsigned off = POOL && cc < 0 ? 0u : (unsigned)cc & 0x1FFFFu;
+          const unsigned off = POOL && cc < 0 ? 0u : (unsigned)cc & (MISO ? 0x1FFFEu : 0x1FFFFu);
           // small pool cell: bits 17..20 only (with table bits a data code can exceed 0x20000 as well)
           BND(cc < 0 || (MT ? (unsigned)cc - 0x20000u < OFDM_CODE_SMALL_POOL : cc >= 0x20000) || off + 2 <= 2u * (unsigned)stage_cap_dbg);
           // explicit 32-bit shared-window addresses (one base register + the lane's table column): the generic-pointer
@@ -1649,6 +1650,13 @@ __device__ __forceinline__ void ofdm_fill(float2 *x, const int32_t *__restrict__
           else {
             asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.x) : "r"(fs.lut_lane_s + ((sc & 255u) << fs.esh)));
             asm volatile("ld.shared.f32 %0, [%1];" : "=f"(val.y) : "r"(fs.lut_lane_s + fs.im_ofs + ((sc >> 8) << fs.esh)));
+          }
+          if constexpr (MISO) {
+            // -conj(g) (bit 0 clear: negate Re) or conj(g) (bit 0 set: negate Im) of the paired cell; pool and pilot
+            // carriers are overwritten below (their pool values are already transformed)
+            const unsigned neg_im = (unsigned)cc << 31;
+            val.x = __uint_as_float(__float_as_uint(val.x) ^ neg_im ^ 0x80000000u);
+            val.y = __uint_as_float(__float_as_uint(val.y) ^ neg_im);
           }
           if (MT ? (unsigned)cc - 0x20000u < OFDM_CODE_SMALL_POOL : cc >= 0x20000) asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(val.x), "=f"(val.y) : "r"(fs.spool_m8_s + ((unsigned)cc >> 14)));
           if (POOL && cc < 0) val = __ldg(pool + (cc & 0x7FFFFFFF));
@@ -1718,13 +1726,16 @@ __device__ __forceinline__ void tmem_wait_ld4(float2 (&v)[4])
 }
 
 // FMT: sink format (bit 0, SinkT) | OFDM_FMT_MT: chain mode with several constellation tables, the carrier codes carry
-// their table's first entry (OFDM_CODE_TAB_SHIFT)
+// their table's first entry (OFDM_CODE_TAB_SHIFT) | OFDM_FMT_MISO: MISO group-2 carrier codes (OFDM_CODE_MISO_IM)
 constexpr int OFDM_FMT_MT = 2;
+constexpr int OFDM_FMT_MISO = 4;
 template <int LOG2M, int T, bool C16, int FMT, int SPLIT>
 __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const OfdmArgs a)
 {
   constexpr bool MT = (FMT & OFDM_FMT_MT) != 0;
+  constexpr bool MISO = (FMT & OFDM_FMT_MISO) != 0;
   static_assert(!MT || C16, "several constellation tables only in chain mode");
+  static_assert(!MISO || C16, "MISO processing only in chain mode");
   extern __shared__ __align__(16) uint8_t smem_raw[];
   float2 *x = reinterpret_cast<float2 *>(smem_raw);
   constexpr int M = 1 << LOG2M;
@@ -1914,12 +1925,12 @@ __global__ void __launch_bounds__(T, (LOG2M == 14 ? 1 : 1024 / T)) k_ofdm(const 
       if (C16 && phase == 0 && threadIdx.x == 0 && unit + (int)gridDim.x < units) desc_issue(cp1);
       // ---- 1. carrier fill (+ first pass)
       if (sinc) {
-        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, true, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
-        else ofdm_fill<LOG2M, T, C16, false, true, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
+        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, true, MT, MISO>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
+        else ofdm_fill<LOG2M, T, C16, false, true, MT, MISO>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
       }
       else {
-        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, false, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
-        else ofdm_fill<LOG2M, T, C16, false, false, MT>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
+        if (pool_sym) ofdm_fill<LOG2M, T, C16, true, false, MT, MISO>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
+        else ofdm_fill<LOG2M, T, C16, false, false, MT, MISO>(x, code, sinc, c, cells, pool, fs, a.stage_cap, a.lut_n);
       }
       __syncthreads();
       // every fill of the symbol has read its cells: the next symbol's cells may replace them (under the passes)
@@ -2083,13 +2094,17 @@ int launch_ofdm(const OfdmArgs &a0, cudaStream_t s)
     for (int sh = 5; sh > 0; sh--)
       if (base + (one << sh) + 1024 <= sm_bytes / ctas) { a.lut_rep_shift = sh; break; }
   }
-  if (a.cells16 && a.lut_tables > 1) {
-    if (a.out_fmt) launch_ofdm_c<true, 1 | OFDM_FMT_MT>(a, s);
-    else launch_ofdm_c<true, 0 | OFDM_FMT_MT>(a, s);
-  }
-  else if (a.cells16) {
-    if (a.out_fmt) launch_ofdm_c<true, 1>(a, s);
-    else launch_ofdm_c<true, 0>(a, s);
+  if (a.cells16) {
+    switch ((a.out_fmt ? 1 : 0) | (a.lut_tables > 1 ? OFDM_FMT_MT : 0) | (a.miso ? OFDM_FMT_MISO : 0)) {
+      case 0: launch_ofdm_c<true, 0>(a, s); break;
+      case 1: launch_ofdm_c<true, 1>(a, s); break;
+      case 2: launch_ofdm_c<true, 2>(a, s); break;
+      case 3: launch_ofdm_c<true, 3>(a, s); break;
+      case 4: launch_ofdm_c<true, 4>(a, s); break;
+      case 5: launch_ofdm_c<true, 5>(a, s); break;
+      case 6: launch_ofdm_c<true, 6>(a, s); break;
+      case 7: launch_ofdm_c<true, 7>(a, s); break;
+    }
   }
   else launch_ofdm_c<false, 0>(a, s);      // the drop-in block always emits complex64
   return 1 << a.lut_rep_shift;

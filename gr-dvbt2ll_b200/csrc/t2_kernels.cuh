@@ -154,15 +154,22 @@ struct OfdmArgs {
   // > 1: `lut` holds that many constellation tables back to back (lut_n entries in all, the largest table first) and the
   // data carrier codes carry their table's first entry (OFDM_CODE_TAB_SHIFT); the k_ofdm instantiations with OFDM_FMT_MT run
   int lut_tables;
+  // 1: MISO group-2 carrier codes (OFDM_CODE_MISO_IM); the k_ofdm instantiations with OFDM_FMT_MISO run
+  int miso;
 };
 // Chain-mode carrier codes of k_ofdm (code_pos), one 32-bit word per carrier:
 //   data carrier         -> 2 * staging slot                       bits 1..16 (byte offset into the staging area)
 //                           | first table entry << 21              bits 21..30, only with several tables (lut_tables > 1)
+//                           | OFDM_CODE_MISO_IM                    bit 0, only in the MISO group-2 codes (miso = 1)
 //   small pool cell p<8  -> (p + 1) << 17                          bits 17..20 (zero / pilot amplitudes, in shared memory)
 //   other pool cell      -> 0x80000000 | pool index                (L1 signalling, dummy cells; their symbols are flagged)
 // Non-data carriers look up entry (staging slot 0's code) of the first table, which is the largest: any cell code
 // stays inside it.
 constexpr int OFDM_CODE_TAB_SHIFT = 21;
+// MISO group 2 (EN 302 755 9.1, modified Alamouti): a data carrier's code names the staging slot of the other cell of
+// its pair, and the looked-up value has its real part negated (bit 0 clear: -conj) or its imaginary part (bit 0 set:
+// conj).  Pool cells come from a pool whose values are already transformed.
+constexpr unsigned OFDM_CODE_MISO_IM = 1u;
 constexpr unsigned OFDM_CODE_TAB_MAX = 1023;      // largest first-entry index the table bits hold
 constexpr unsigned OFDM_CODE_SMALL_POOL = 0x1E0000u;   // bits of a small pool cell
 // returns the number of constellation-table copies kept in shared memory (chain mode; 1 otherwise)

@@ -265,6 +265,24 @@ struct Chain16Tables {
 };
 bool compose_chain16(const FramePlan &fp, const OfdmPlan &op, Chain16Tables *out, std::string *err);
 
+// MISO processing (EN 302 755 9.1, modified Alamouti; beyond the reference, which sends group 1's cells from both
+// transmitter groups).  With g_{l,i} the cells of OFDM symbol l in the order the frequency interleaver emits them
+// (i < C_l, L1 / dummy / unmodulated cells included): group 1 sends e = g, group 2 sends e_{l,2i} = -conj(g_{l,2i+1}),
+// e_{l,2i+1} = conj(g_{l,2i}) in every P2, data and frame-closing symbol; pilots, nulls and reserved carriers are the
+// group's own.  The carrier tables of one group's output over the staging of `t` (whose runs, staging slots and copy
+// sizes every group shares): non-data carriers from `og` (the group's pilot plan), data carriers from t.code at the
+// carrier of cell i (group 1) or i ^ 1 (group 2, refused if a symbol has an odd cell count).  Group 2's kernel negates
+// Re (i even) or Im (i odd) of a data cell; a pool cell (L1, dummy) lands at one position per frame, so the group-2 pool
+// holds its transformed value instead (the shared zero cell stays as it is).
+struct MisoTables {
+  std::vector<int32_t> code;   // [num_symbols * c_ps], Chain16Tables::code's convention
+  std::vector<uint8_t> plp;    // [num_symbols * c_ps]
+  CellPool pool;
+};
+// op: the pilot plan `t` was composed with
+bool compose_miso(const OfdmPlan &op, const Chain16Tables &t, const OfdmPlan &og, bool group2, MisoTables *out,
+                  std::string *err);
+
 // small utilities
 void bb_prbs_bits(int n, uint8_t *out);          // 1 bit per byte; reference :357-369
 uint32_t crc32_bits(const uint8_t *bits, int n); // CRC-32 MSB first, init all ones (reference framemapper :1205-1224)

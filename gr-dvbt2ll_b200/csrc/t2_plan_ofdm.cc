@@ -399,4 +399,72 @@ bool compose_chain16(const FramePlan &fp, const OfdmPlan &op, Chain16Tables *out
   return true;
 }
 
+bool compose_miso(const OfdmPlan &op, const Chain16Tables &t, const OfdmPlan &og, bool group2, MisoTables *out,
+                  std::string *err)
+{
+  const int L = op.dims.num_symbols, cps = op.dims.c_ps;
+  bool same = og.dims.num_symbols == L && og.dims.c_ps == cps && og.pool.cells.size() == op.pool.cells.size();
+  for (size_t i = 0; same && i < og.pool.cells.size(); i++)      // pilot amplitudes (the pool part og's codes index)
+    same = og.pool.cells[i].re == t.pool.cells[i].re && og.pool.cells[i].im == t.pool.cells[i].im;
+  if (!same) {
+    if (err) *err = "chain: the MISO groups' pilot plans do not describe the same frame";
+    return false;
+  }
+  out->code.assign((size_t)L * cps, 0);
+  out->plp.assign((size_t)L * cps, 0);
+  out->pool = t.pool;
+  // per pool cell: 0 = not yet placed, 1 = lands at an even position of group 2 (-conj), 2 = at an odd one (conj)
+  std::vector<uint8_t> placed(t.pool.cells.size(), 0);
+  std::vector<int32_t> carrier_of;
+  for (int l = 0; l < L; l++) {
+    const int s = op.sym_data_start[l], n = op.sym_data_start[l + 1] - s;
+    if (group2 && (n & 1)) {
+      if (err) *err = "chain: MISO processing needs an even number of cells in every symbol; symbol " + std::to_string(l) +
+                      " has " + std::to_string(n);
+      return false;
+    }
+    carrier_of.assign(n, -1);
+    for (int k = 0; k < cps; k++) {
+      const int32_t c = op.code[(size_t)l * cps + k];
+      if ((c >= 0) != (og.code[(size_t)l * cps + k] >= 0) || (c >= 0 && c != og.code[(size_t)l * cps + k])) {
+        if (err) *err = "chain: the MISO groups' data carriers differ";
+        return false;
+      }
+      if (c >= 0) carrier_of[c - s] = k;
+    }
+    for (int k = 0; k < cps; k++) {
+      const size_t ck = (size_t)l * cps + k;
+      const int32_t c = og.code[ck];
+      if (c < 0) { out->code[ck] = c; continue; }
+      const int i = c - s;
+      const size_t src = (size_t)l * cps + carrier_of[group2 ? i ^ 1 : i];
+      const int32_t v = t.code[src];
+      out->code[ck] = v;
+      out->plp[ck] = t.plp[src];
+      if (!group2 || v >= 0) continue;
+      const int32_t p = ~v;
+      const cfloat z = t.pool.cells[p];
+      if (z.re == 0.0f && z.im == 0.0f) continue;      // the shared zero cell: -conj(0) = conj(0) = 0
+      const uint8_t want = (uint8_t)(1 + (i & 1));
+      if (placed[p] && placed[p] != want) {
+        if (err) *err = "chain: a pool cell lands at an even and at an odd position of a symbol";
+        return false;
+      }
+      placed[p] = want;
+    }
+  }
+  // a placed L1-post cell of variant 0 stands for the same cell of every variant (same position in every frame)
+  const CellPool &q = t.pool;
+  for (size_t p = 0; p < placed.size(); p++) {
+    if (!placed[p]) continue;
+    const bool post = (int)p >= q.l1post_base && (int)p < q.l1post_base + q.l1post_cells;
+    for (int v = 0; v < (post ? q.l1post_variants : 1); v++) {
+      cfloat &z = out->pool.cells[p + (size_t)v * q.l1post_cells];
+      if (placed[p] == 1) z.re = -z.re;
+      else z.im = -z.im;
+    }
+  }
+  return true;
+}
+
 } // namespace t2

@@ -39,7 +39,7 @@ EXPORTED_SYMBOLS = [
     "dvbt2ll_stream_create", "dvbt2ll_stream_destroy", "dvbt2ll_stream_synchronize",
     "dvbt2ll_chain_create_multiplp", "dvbt2ll_chain_num_plp", "dvbt2ll_chain_plp_ts_bytes",
     "dvbt2ll_chain_history_bytes", "dvbt2ll_ts_sync", "dvbt2ll_ts_fill", "dvbt2ll_chain_create_plps",
-    "dvbt2ll_chain_set_papr_tr",
+    "dvbt2ll_chain_set_papr_tr", "dvbt2ll_chain_set_miso", "dvbt2ll_chain_run_device_miso", "dvbt2ll_chain_run_host_miso",
 ]
 GATHER_BLOB_BYTES = 256
 
@@ -107,6 +107,9 @@ def lib():
         L.dvbt2ll_chain_enable_timing.argtypes = [vp, ci]
         L.dvbt2ll_chain_set_sink.argtypes = [vp, ci, C.c_float]
         L.dvbt2ll_chain_set_papr_tr.argtypes = [vp, ci, C.c_float, C.c_float]
+        L.dvbt2ll_chain_set_miso.argtypes = [vp, ci]
+        L.dvbt2ll_chain_run_device_miso.argtypes = [vp, vp, cll, ci, ci, cll, vp, vp, vp]
+        L.dvbt2ll_chain_run_host_miso.argtypes = [vp, vp, cll, ci, ci, cll, vp, vp]
         L.dvbt2ll_set_overfull_policy.argtypes = [ci]
         L.dvbt2ll_set_overfull_policy.restype = None
         L.dvbt2ll_set_host_register.argtypes = [vp, ci]
@@ -453,6 +456,14 @@ class Chain(_Block):
         if r < 0:
             raise ValueError(last_error())
 
+    def set_miso(self, on):
+        """MISO processing (EN 302 755 9.1, modified Alamouti; preamble T2_MISO or T2_LITE_MISO): with on = 1 a chain
+        with misogroup TX2 emits group 2, whose cells of each OFDM symbol are the pairs (-conj(g_2i+1), conj(g_2i)) of
+        group 1's; with misogroup TX1 the output is unchanged.  Off by default."""
+        r = lib().dvbt2ll_chain_set_miso(self._h, int(on))
+        if r < 0:
+            raise ValueError(last_error())
+
     def history_bytes(self, first_frame):
         """Stream bytes that must precede the first TS byte of `first_frame` in every row handed to run_host():
         187 in normal input mode once the stream has started (CRC-8 of the packet in flight), else 0."""
@@ -463,28 +474,55 @@ class Chain(_Block):
         starts with the history bytes (the 187 stream bytes before the first frame; none for first_frame = 0 or in
         high-efficiency mode), followed by the TS bytes of the frames.  Returns complex64 [n_channels, n_frames*samples]
         (int16 [n_channels, n_frames*samples, 2] with sink format 1)."""
-        P = self.num_plp
-        ts = np.ascontiguousarray(ts, dtype=np.uint8).reshape(n_channels * P, -1)      # row = channel * num_plp + plp
-        hist = self.history_bytes(first_frame)
-        need = max(self.plp_ts_bytes(p, first_frame, n_frames) for p in range(P))
-        if ts.shape[1] < hist + need:
-            raise ValueError("run_host: each TS row needs %d history bytes + %d TS bytes, got %d" % (hist, need, ts.shape[1]))
+        ts, hist = self._host_ts(ts, n_channels, n_frames, first_frame)
         if out is None:
-            if self.sink_format:
-                out = np.empty((n_channels, n_frames * self.samples_per_frame, 2), dtype=np.int16)
-            else:
-                out = np.empty((n_channels, n_frames * self.samples_per_frame), dtype=np.complex64)
+            out = self._host_out(n_channels, n_frames)
         r = lib().dvbt2ll_chain_run_host(self._h, ts.ctypes.data + hist, ts.shape[1], n_channels, n_frames, first_frame,
                                          out.ctypes.data)
         if r < 0:
             raise RuntimeError("dvbt2ll_chain_run_host failed (%d): %s" % (r, last_error()))
         return out
 
+    def run_host_miso(self, ts, n_channels, n_frames, first_frame=0):
+        """Both MISO transmitter groups from one pass of BB/BCH, LDPC and mapper (preamble T2_MISO or T2_LITE_MISO, tone
+        reservation off): returns (out1, out2), group 1 and group 2 with MISO processing, each laid out as run_host's
+        output.  ts as for run_host; misogroup does not matter."""
+        ts, hist = self._host_ts(ts, n_channels, n_frames, first_frame)
+        out1, out2 = self._host_out(n_channels, n_frames), self._host_out(n_channels, n_frames)
+        r = lib().dvbt2ll_chain_run_host_miso(self._h, ts.ctypes.data + hist, ts.shape[1], n_channels, n_frames,
+                                              first_frame, out1.ctypes.data, out2.ctypes.data)
+        if r < 0:
+            raise RuntimeError("dvbt2ll_chain_run_host_miso failed (%d): %s" % (r, last_error()))
+        return out1, out2
+
+    def _host_ts(self, ts, n_channels, n_frames, first_frame):
+        P = self.num_plp
+        ts = np.ascontiguousarray(ts, dtype=np.uint8).reshape(n_channels * P, -1)      # row = channel * num_plp + plp
+        hist = self.history_bytes(first_frame)
+        need = max(self.plp_ts_bytes(p, first_frame, n_frames) for p in range(P))
+        if ts.shape[1] < hist + need:
+            raise ValueError("run_host: each TS row needs %d history bytes + %d TS bytes, got %d" % (hist, need, ts.shape[1]))
+        return ts, hist
+
+    def _host_out(self, n_channels, n_frames):
+        if self.sink_format:
+            return np.empty((n_channels, n_frames * self.samples_per_frame, 2), dtype=np.int16)
+        return np.empty((n_channels, n_frames * self.samples_per_frame), dtype=np.complex64)
+
     def run_device(self, d_ts_ptr, ts_pitch, n_channels, n_frames, first_frame, d_out_ptr, stream_ptr):
         r = lib().dvbt2ll_chain_run_device(self._h, d_ts_ptr, ts_pitch, n_channels, n_frames, first_frame, d_out_ptr,
                                            stream_ptr)
         if r < 0:
             raise RuntimeError("dvbt2ll_chain_run_device failed (%d): %s" % (r, last_error()))
+        return r
+
+    def run_device_miso(self, d_ts_ptr, ts_pitch, n_channels, n_frames, first_frame, d_out1_ptr, d_out2_ptr, stream_ptr):
+        """run_device with both MISO groups from one front-end pass: group 1 to d_out1_ptr, group 2 with MISO processing
+        to d_out2_ptr (see run_host_miso)."""
+        r = lib().dvbt2ll_chain_run_device_miso(self._h, d_ts_ptr, ts_pitch, n_channels, n_frames, first_frame,
+                                                d_out1_ptr, d_out2_ptr, stream_ptr)
+        if r < 0:
+            raise RuntimeError("dvbt2ll_chain_run_device_miso failed (%d): %s" % (r, last_error()))
         return r
 
     def tap(self, stage, dtype=np.uint8):

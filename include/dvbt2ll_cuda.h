@@ -176,6 +176,27 @@ DVBT2LL_API_EXPORT long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *st
  * symbol) of the last run, updates applied | stop reason << 8 (1 = clip reached, 2 = tone_max, 3 = iteration limit);
  * refused while the stage is off. */
 DVBT2LL_API_EXPORT int dvbt2ll_chain_set_papr_tr(dvbt2ll_handle *h, int iterations, float vclip, float tone_max);
+/* MISO processing (EN 302 755 9.1, modified Alamouti; beyond the reference, whose group-2 output carries group 1's
+ * cells with only the pilots changed).  Let g_{l,0..C_l-1} be the cells of OFDM symbol l in the order the frequency
+ * interleaver emits them (the order of the data carriers, k rising; L1-pre / L1-post, dummy and the unmodulated cells of
+ * the frame-closing symbol included).  Group 1 sends e = g; group 2 sends e_{l,2i} = -conj(g_{l,2i+1}) and
+ * e_{l,2i+1} = conj(g_{l,2i}), i < C_l / 2, in every P2, data and frame-closing symbol.  Pilots, nulls, reserved
+ * carriers and P1 are not touched: each group keeps its own pilots (misogroup).
+ * dvbt2ll_chain_set_miso: needs preamble T2_MISO or T2_LITE_MISO (refused otherwise, and for a frame with an odd cell
+ * count in a symbol, naming it); with on = 1 a chain with misogroup TX2 emits group 2 with MISO processing from
+ * dvbt2ll_chain_run_* and dvbt2ll_work*, tone reservation still applying after it; with misogroup TX1 the output is
+ * unchanged.  Default off.  Once on, dvbt2ll_plan_get "chain.miso_code" (int32 carrier codes of group 2, "chain.code"'s
+ * convention) and "chain.miso_pool" (complex64, its pool with the L1 / dummy cells transformed) can be read.
+ * dvbt2ll_chain_run_{device,host}_miso: both groups from one pass of BB/BCH, LDPC and mapper -- group 1 to out1, group 2
+ * with MISO processing to out2, whatever misogroup says; the arguments are those of dvbt2ll_chain_run_{device,host}, both
+ * outputs take the sink, the stage time "ofdm" covers both k_ofdm launches.  Refused without a MISO preamble, with tone
+ * reservation on, or with a NULL output. */
+DVBT2LL_API_EXPORT int dvbt2ll_chain_set_miso(dvbt2ll_handle *h, int on);
+DVBT2LL_API_EXPORT int dvbt2ll_chain_run_device_miso(dvbt2ll_handle *h, const void *d_ts, long long ts_pitch, int n_channels,
+                                                     int n_frames, long long first_frame, void *d_out1, void *d_out2,
+                                                     void *stream);
+DVBT2LL_API_EXPORT int dvbt2ll_chain_run_host_miso(dvbt2ll_handle *h, const void *ts, long long ts_pitch, int n_channels,
+                                                   int n_frames, long long first_frame, void *out1, void *out2);
 /* Device time in ms of each stage kernel (bb_bch, ldpc, map, ofdm, total), averaged over the chain runs issued since
  * timing was enabled (at most the last 64); events are recorded per run, so the caller's timed loop needs no sync.
  * With tone reservation on, "ofdm" covers k_ofdm and the tone-reservation kernel after it. */
