@@ -806,20 +806,25 @@ std::vector<uint16_t> make_ci_inv4(const std::vector<uint16_t> &ci_inv, int *str
 }
 
 struct ChainHandle : dvbt2ll_handle {
-  // the stages of PLP parameter set 0 (every PLP's, unless the PLPs have their own parameters)
-  BbHandle bb;
-  LdpcHandle ldpc;
-  MapHandle map;
-  // PLPs with their own parameters (dvbt2ll_chain_create_plps) and more than one set of them (fplan.plp_sets > 1): the
-  // stages of sets 1.., one launch per PLP and stage; the BCH / FEC buffers are PLP-major (PLP p's region holds its
-  // codewords [channel][frame][block] at its own pitch), the 16-bit cells of PLP p start at fplan.plp_chain_off[p]
-  struct Set { BbHandle bb; LdpcHandle ldpc; MapHandle map; };
-  std::unique_ptr<Set> xset[t2::MAX_PLP];
-  DevBuf d_ci_inv_p[t2::MAX_PLP], d_ci_inv4_p[t2::MAX_PLP];
-  int ci4_stride_p[t2::MAX_PLP];
-  size_t bch_off[t2::MAX_PLP + 1], fec_off[t2::MAX_PLP + 1];   // byte offsets of the PLP regions
+  // the stages of each PLP parameter set (fplan.plp_set: a distinct framesize, rate, constellation and rotation), built
+  // from the set's first PLP, with that PLP's inverse cell permutation; set 0 also carries the chain-wide BB fields
+  // (input mode, in-band signalling, sync-error counter)
+  struct Set {
+    BbHandle bb;
+    LdpcHandle ldpc;
+    MapHandle map;
+    DevBuf d_ci_inv, d_ci_inv4;
+    int ci4_stride;
+    int bch_pitch() const { return align16(bb.plan.fec.nbch / 8); }
+    int fec_pitch() const { return align16(bb.plan.fec.nldpc / 8); }
+  };
+  std::unique_ptr<Set[]> sets;     // [fplan.plp_sets]
+  // FEC groups (see group_of): PLPs [p0, p1) with `blocks` FEC blocks per T2 frame, and their regions of the BCH / FEC
+  // buffers, which hold the codewords [frame slot][block of the group] at the set's pitch
+  struct Group { int p0, p1, blocks; size_t bch_off, fec_off; };
+  std::vector<Group> grp;
   // constellation tables of the OFDM fill: one per distinct (constellation, rotation), the largest first; PLP p's
-  // starts at entry lut_base[p].  One table: the set-0 mapper's.
+  // starts at entry lut_base[p]
   std::vector<t2::cfloat> luts;
   int lut_tables, lut_base[t2::MAX_PLP], lut_single;
   int lut_copies;      // copies of the table(s) k_ofdm kept in shared memory in the last run
@@ -828,8 +833,8 @@ struct ChainHandle : dvbt2ll_handle {
   t2::OfdmPlan oplan;
   t2::Chain16Tables tables;
   OfdmDevice odev;
-  DevBuf d_bch, d_fec, d_cells, d_ts_stage, d_out_stage, d_ci_inv, d_ci_inv4, d_fec_shift, d_run_desc, d_run_ptr, d_run_cnt, d_stage_bytes;
-  int stage_cap, ci4_stride;
+  DevBuf d_bch, d_fec, d_cells, d_ts_stage, d_out_stage, d_fec_shift, d_run_desc, d_run_ptr, d_run_cnt, d_stage_bytes;
+  int stage_cap;
   int max_frames, device;
   int sink_fmt;          // 0 complex64 (what pilotgenp1insert_cc emits), 1 interleaved int16 I/Q
   float sink_gain;       // the flowgraph's multiply_const stage folded into the last kernel
@@ -869,13 +874,12 @@ struct ChainHandle : dvbt2ll_handle {
     if (device >= 0) CK(cudaSetDevice(device));
     return ensure_device();
   }
-  bool mixed() const { return fplan.plp_sets > 1; }
-  BbHandle &bb_of(int plp) { const int s = fplan.plp_set[plp]; return s ? xset[s]->bb : bb; }
-  const BbHandle &bb_of(int plp) const { const int s = fplan.plp_set[plp]; return s ? xset[s]->bb : bb; }
-  LdpcHandle &ldpc_of(int plp) { const int s = fplan.plp_set[plp]; return s ? xset[s]->ldpc : ldpc; }
-  MapHandle &map_of(int plp) { const int s = fplan.plp_set[plp]; return s ? xset[s]->map : map; }
-  int bch_pitch(int plp) const { return align16(bb_of(plp).plan.fec.nbch / 8); }
-  int fec_pitch(int plp) const { return align16(bb_of(plp).plan.fec.nldpc / 8); }
+  Set &set_of(int plp) const { return sets[fplan.plp_set[plp]]; }
+  int first_plp(int set) const { int p = 0; while (fplan.plp_set[p] != set) p++; return p; }
+  // The FEC group of a PLP: one LDPC and one mapper launch per group.  PLPs of a single parameter set form one group,
+  // their codewords in the frame's block list, so a create_multiplp chain runs each stage once; with several sets
+  // every PLP is a group of its own, whose cells FramePlan::plp_chain_off starts on a 16-byte boundary by the same rule.
+  int group_of(int plp) const { return fplan.plp_sets > 1 ? plp : 0; }
   int F() const { return fplan.prm.fecblocks; }
   int P() const { return fplan.num_plp; }
   int Fp(int plp) const { return fplan.plp_first_block[plp + 1] - fplan.plp_first_block[plp]; }
@@ -887,9 +891,9 @@ struct ChainHandle : dvbt2ll_handle {
     const int fpl = Fp(plp);            // the PLP's FEC blocks per T2 frame = its in-band signalling cycle
     const long long j0 = frame * fpl;
     long long nb0 = 0;
-    if (bb.plan.inband) nb0 = (j0 + fpl - 1) / fpl;
-    const long long P = j0 * bb_of(plp).plan.payload_bytes - 13 * nb0;  // payload bytes before the frame
-    if (bb.plan.mode == t2::INPUTMODE_NORMAL || P == 0) return P;
+    if (sets[0].bb.plan.inband) nb0 = (j0 + fpl - 1) / fpl;
+    const long long P = j0 * set_of(plp).bb.plan.payload_bytes - 13 * nb0;  // payload bytes before the frame
+    if (sets[0].bb.plan.mode == t2::INPUTMODE_NORMAL || P == 0) return P;
     const long long last = P - 1;                                       // high efficiency mode: sync bytes are skipped,
     return 1 + last + last / 187 + 1;                                   // packets = 1 sync + 187 payload bytes
   }
@@ -907,26 +911,16 @@ struct ChainHandle : dvbt2ll_handle {
   int forecast(int noutput) const { return (int)(ts_per_frame() * (noutput / oplan.samples_per_frame)); }
   int dev_init()
   {
-    bb.stream = 0; ldpc.stream = 0; map.stream = 0;
     int r;
-    if ((r = bb.dev_init())) return r;
-    if ((r = ldpc.dev_init())) return r;
-    if ((r = map.dev_init())) return r;
-    for (int s = 1; s < fplan.plp_sets; s++) {
-      Set &x = *xset[s];
-      x.bb.stream = 0; x.ldpc.stream = 0; x.map.stream = 0;
+    for (int s = 0; s < fplan.plp_sets; s++) {
+      Set &x = sets[s];
       if ((r = x.bb.dev_init()) || (r = x.ldpc.dev_init()) || (r = x.map.dev_init())) return r;
+      const std::vector<uint16_t> &ci_inv = fplan.plp_cell_perm_inv[first_plp(s)];
+      CK(upload(x.d_ci_inv, ci_inv));
+      CK(upload(x.d_ci_inv4, make_ci_inv4(ci_inv, &x.ci4_stride)));
     }
     if ((r = odev.init(tables.code, tables.pool, oplan, true, &tables.plp, lut_tables > 1 ? lut_base : 0))) return r;
-    CK(upload(d_ci_inv, fplan.cell_perm_inv));
-    CK(upload(d_ci_inv4, make_ci_inv4(fplan.cell_perm_inv, &ci4_stride)));
-    if (mixed()) {
-      for (int pl = 0; pl < P(); pl++) {
-        CK(upload(d_ci_inv_p[pl], fplan.plp_cell_perm_inv[pl]));
-        CK(upload(d_ci_inv4_p[pl], make_ci_inv4(fplan.plp_cell_perm_inv[pl], &ci4_stride_p[pl])));
-      }
-      CK(upload(d_luts, luts));
-    }
+    CK(upload(d_luts, luts));
     CK(upload(d_fec_shift, fplan.fec_shift));
     CK(upload(d_run_desc, tables.run_desc));
     CK(upload(d_run_ptr, tables.run_ptr));
@@ -935,17 +929,18 @@ struct ChainHandle : dvbt2ll_handle {
     stage_cap = (tables.max_slots + 7) & ~7;
     if ((size_t)(1 << odev.log2_m) * 8 * 17 / 16 + (size_t)stage_cap * 2 + 2048 + 96 + (size_t)(tables.max_runs + 2) * 8 > 227 * 1024)
       return fail(DVBT2LL_ERR_INVALID, "chain: the cells of one OFDM symbol do not fit the shared-memory staging area");
-    const size_t nfec = (size_t)max_frames * F();
-    bch_off[0] = fec_off[0] = 0;
+    grp.clear();
+    size_t bch_end = 0, fec_end = 0;
     for (int pl = 0; pl < P(); pl++) {
-      bch_off[pl + 1] = bch_off[pl] + (size_t)max_frames * Fp(pl) * bch_pitch(pl);
-      fec_off[pl + 1] = fec_off[pl] + (size_t)max_frames * Fp(pl) * fec_pitch(pl);
+      if (group_of(pl) == (int)grp.size()) grp.push_back(Group{ pl, pl, 0, bch_end, fec_end });
+      Group &G = grp.back();
+      G.p1 = pl + 1;
+      G.blocks += Fp(pl);
+      bch_end += (size_t)max_frames * Fp(pl) * set_of(pl).bch_pitch();
+      fec_end += (size_t)max_frames * Fp(pl) * set_of(pl).fec_pitch();
     }
-    if (mixed()) {
-      CK(d_bch.ensure(bch_off[P()] + 64));
-      CK(d_fec.ensure(fec_off[P()] + 64));
-    }
-    else CK(d_bch.ensure(nfec * align16(bb.plan.fec.nbch / 8) + 64));
+    CK(d_bch.ensure(bch_end + 64));
+    CK(d_fec.ensure(fec_end + 64));
     CK(d_cells.ensure((size_t)max_frames * cells16_stride() * sizeof(uint16_t) + 64));   // 16-bit cell codes
     // the padding cells between frames and the slack behind the last one are never written by the mapper but travel
     // with the aligned bulk copies: give them a valid code once
@@ -974,47 +969,56 @@ struct ChainHandle : dvbt2ll_handle {
       }
       if (!d_out2) { g1 = g2; g2 = 0; }
     }
-    const int nfec = frames * F();
-    const int bp = align16(bb.plan.fec.nbch / 8), fp = align16(bb.plan.fec.nldpc / 8);
     cudaEvent_t *tev = ev[n_timed % TIMING_SLOTS];
     if (timing) cudaEventRecord(tev[0], s);
-    uint8_t *bch_buf = d_bch.as<uint8_t>() + (size_t)buf_frame * F() * bp;
-    if (!mixed()) CK(d_fec.ensure((size_t)max_frames * F() * fp + 64));      // (PLP-major buffers: sized at dev_init)
-    uint8_t *fec_buf = d_fec.as<uint8_t>() + (size_t)buf_frame * F() * fp;
+    // a group's codewords of the batch: slot buf_frame onwards of its regions
+    auto bch_buf = [&](const Group &G) { return d_bch.as<uint8_t>() + G.bch_off + (size_t)buf_frame * G.blocks * set_of(G.p0).bch_pitch(); };
+    auto fec_buf = [&](const Group &G) { return d_fec.as<uint8_t>() + G.fec_off + (size_t)buf_frame * G.blocks * set_of(G.p0).fec_pitch(); };
     uint16_t *cell_buf = d_cells.as<uint16_t>() + (size_t)buf_frame * cells16_stride();
-    if (mixed()) run_plps(d_ts, ts_pitch, n_channels, n_frames, first_frame, cell_buf, s, buf_frame, hist_valid, tev);
-    else {
     // BB framing + BCH, PLP by PLP: row c * P + p of the TS holds PLP p of channel c; every PLP has its own stream
     // position (packet phase, in-band cycle = its FEC blocks per frame), and its codewords go to their place inside
-    // the frame's block list (streams begin on a packet boundary at frame 0)
+    // its group's block list (streams begin on a packet boundary at frame 0)
     for (int pl = 0; pl < P(); pl++) {
-      const int fpl = Fp(pl);
+      const Group &G = grp[group_of(pl)];
+      Set &x = set_of(pl);
+      const int fpl = Fp(pl), bp = x.bch_pitch();
       const long long j0 = first_frame * fpl;
-      const int fb0 = bb.plan.inband ? (int)(j0 % fpl) : 0;
+      const int fb0 = sets[0].bb.plan.inband ? (int)(j0 % fpl) : 0;
       const int count0 = (int)(stream_pos(first_frame, pl) % 188);
       t2k::BbArgs ba;
-      bb.fill_args(ba, (const uint8_t *)d_ts + (long long)pl * ts_pitch, ts_pitch * P(), n_channels, n_frames * fpl, count0, fb0,
-                   hist_valid >= 0 ? hist_valid : (first_frame > 0 ? 1 : 0), bch_buf, bp);
+      x.bb.fill_args(ba, (const uint8_t *)d_ts + (long long)pl * ts_pitch, ts_pitch * P(), n_channels, n_frames * fpl, count0, fb0,
+                     hist_valid >= 0 ? hist_valid : (first_frame > 0 ? 1 : 0), bch_buf(G), bp);
       ba.fecblocks = fpl;
       ba.ts_len = ts_bytes(first_frame, n_frames, pl);
-      ba.out_len = (long long)frames * F() * bp;
-      if (P() > 1) { ba.out_group = fpl; ba.out_group_stride = F(); ba.out_group_off = fplan.plp_first_block[pl]; }
+      ba.out_len = (long long)frames * G.blocks * bp;
+      if (G.p1 - G.p0 > 1) {
+        ba.out_group = fpl; ba.out_group_stride = G.blocks;
+        ba.out_group_off = fplan.plp_first_block[pl] - fplan.plp_first_block[G.p0];
+      }
       t2k::launch_bb_bch(ba, s);
     }
     if (timing) cudaEventRecord(tev[1], s);
-    t2k::LdpcArgs la;
-    ldpc.fill_args(la, bch_buf, bp, fec_buf, fp, nfec);
-    t2k::MapArgs ma;
-    map.fill_args(ma, fec_buf, fp, 0, nfec);
-    ma.out16 = cell_buf; ma.out16_frame_stride = cells16_stride();                                        // 16-bit cell codes,
-    ma.ci_inv = d_ci_inv.as<uint16_t>(); ma.fec_shift = d_fec_shift.as<int32_t>(); ma.fecblocks = F();   // cell-interleaved
-    ma.ci_inv4 = d_ci_inv4.as<uint16_t>(); ma.ci_inv4_stride = ci4_stride;
-    ma.out_len = (long long)frames * cells16_stride();
-    t2k::launch_ldpc(la, s);
-    if (timing) cudaEventRecord(tev[2], s);
-    t2k::launch_map(ma, s);
-    if (timing) cudaEventRecord(tev[3], s);
+    for (const Group &G : grp) {
+      Set &x = set_of(G.p0);
+      t2k::LdpcArgs la;
+      x.ldpc.fill_args(la, bch_buf(G), x.bch_pitch(), fec_buf(G), x.fec_pitch(), frames * G.blocks);
+      t2k::launch_ldpc(la, s);
     }
+    if (timing) cudaEventRecord(tev[2], s);
+    // the mapper writes the group's 16-bit cell codes, cell-interleaved, to its place in each frame's cell memory
+    for (const Group &G : grp) {
+      Set &x = set_of(G.p0);
+      t2k::MapArgs ma;
+      x.map.fill_args(ma, fec_buf(G), x.fec_pitch(), 0, frames * G.blocks);
+      ma.out16 = cell_buf + fplan.plp_chain_off[G.p0]; ma.out16_frame_stride = cells16_stride();
+      ma.ci_inv = x.d_ci_inv.as<uint16_t>(); ma.fec_shift = d_fec_shift.as<int32_t>() + fplan.plp_first_block[G.p0];
+      ma.fecblocks = G.blocks;
+      ma.ci_inv4 = x.d_ci_inv4.as<uint16_t>(); ma.ci_inv4_stride = x.ci4_stride;
+      ma.im_from_re = lut_single;      // the w~ codes only when the OFDM fill keeps the single-table form for every PLP
+      ma.out_len = (long long)frames * cells16_stride() - fplan.plp_chain_off[G.p0];
+      t2k::launch_map(ma, s);
+    }
+    if (timing) cudaEventRecord(tev[3], s);
     // tone reservation: in place on d_out when the sink is complex64 at gain 1; otherwise k_ofdm writes complex64 at
     // gain 1 to a scratch (the buffer slots of buf_frame) and k_papr_tr applies the sink
     const bool tr_on = tr_iter > 0, tr_inplace = tr_on && sink_fmt == 0 && sink_gain == 1.0f;
@@ -1035,9 +1039,8 @@ struct ChainHandle : dvbt2ll_handle {
     oa.cells = 0; oa.cells_stride = cells16_stride();
     oa.cells16 = cell_buf; oa.run_desc = d_run_desc.as<int2>(); oa.run_ptr = d_run_ptr.as<int32_t>();
     oa.run_cnt = d_run_cnt.as<int32_t>(); oa.desc_cap = (tables.max_runs + 2) & ~1;
-    oa.stage_bytes = d_stage_bytes.as<int32_t>(); oa.stage_cap = stage_cap; oa.lut_single = map.plan.im_from_re;
-    oa.lut = map.d_lut.as<float2>(); oa.lut_n = 1 << map.plan.mod;
-    if (mixed()) { oa.lut_single = lut_single; oa.lut = d_luts.as<float2>(); oa.lut_n = (int)luts.size(); oa.lut_tables = lut_tables; }
+    oa.stage_bytes = d_stage_bytes.as<int32_t>(); oa.stage_cap = stage_cap;
+    oa.lut = d_luts.as<float2>(); oa.lut_n = (int)luts.size(); oa.lut_tables = lut_tables; oa.lut_single = lut_single;
     oa.out = ofdm_out; oa.out_stride = oplan.samples_per_frame;
     oa.cells_len = (long long)frames * cells16_stride(); oa.out_len = (long long)frames * oplan.samples_per_frame;
     oa.out_fmt = sink_fmt; oa.sink_gain = sink_gain; oa.norm = oplan.normalization * sink_gain;
@@ -1109,45 +1112,6 @@ struct ChainHandle : dvbt2ll_handle {
     tr_uploaded = true;
     return 0;
   }
-  // BB + BCH, LDPC and mapper of a chain whose PLPs have more than one parameter set: a launch per PLP and stage, each
-  // on the PLP's own contiguous regions of the BCH / FEC buffers and of the cell memory
-  void run_plps(const void *d_ts, long long ts_pitch, int n_channels, int n_frames, long long first_frame, uint16_t *cell_buf,
-                cudaStream_t s, int buf_frame, int hist_valid, cudaEvent_t *tev)
-  {
-    const int frames = n_channels * n_frames;
-    auto bch_buf = [&](int pl) { return d_bch.as<uint8_t>() + bch_off[pl] + (size_t)buf_frame * Fp(pl) * bch_pitch(pl); };
-    auto fec_buf = [&](int pl) { return d_fec.as<uint8_t>() + fec_off[pl] + (size_t)buf_frame * Fp(pl) * fec_pitch(pl); };
-    for (int pl = 0; pl < P(); pl++) {
-      const int fpl = Fp(pl);
-      const long long j0 = first_frame * fpl;
-      t2k::BbArgs ba;
-      bb_of(pl).fill_args(ba, (const uint8_t *)d_ts + (long long)pl * ts_pitch, ts_pitch * P(), n_channels, n_frames * fpl,
-                          (int)(stream_pos(first_frame, pl) % 188), bb.plan.inband ? (int)(j0 % fpl) : 0,
-                          hist_valid >= 0 ? hist_valid : (first_frame > 0 ? 1 : 0), bch_buf(pl), bch_pitch(pl));
-      ba.fecblocks = fpl;
-      ba.ts_len = ts_bytes(first_frame, n_frames, pl);
-      t2k::launch_bb_bch(ba, s);
-    }
-    if (timing) cudaEventRecord(tev[1], s);
-    for (int pl = 0; pl < P(); pl++) {
-      t2k::LdpcArgs la;
-      ldpc_of(pl).fill_args(la, bch_buf(pl), bch_pitch(pl), fec_buf(pl), fec_pitch(pl), frames * Fp(pl));
-      t2k::launch_ldpc(la, s);
-    }
-    if (timing) cudaEventRecord(tev[2], s);
-    for (int pl = 0; pl < P(); pl++) {
-      t2k::MapArgs ma;
-      map_of(pl).fill_args(ma, fec_buf(pl), fec_pitch(pl), 0, frames * Fp(pl));
-      ma.out16 = cell_buf + fplan.plp_chain_off[pl]; ma.out16_frame_stride = cells16_stride();
-      ma.ci_inv = d_ci_inv_p[pl].as<uint16_t>(); ma.fec_shift = d_fec_shift.as<int32_t>() + fplan.plp_first_block[pl];
-      ma.fecblocks = Fp(pl);
-      ma.ci_inv4 = d_ci_inv4_p[pl].as<uint16_t>(); ma.ci_inv4_stride = ci4_stride_p[pl];
-      ma.im_from_re = lut_single;      // the w~ codes only when the OFDM fill keeps the single-table form for every PLP
-      ma.out_len = (long long)frames * cells16_stride() - fplan.plp_chain_off[pl];
-      t2k::launch_map(ma, s);
-    }
-    if (timing) cudaEventRecord(tev[3], s);
-  }
   int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
   {
     const int frames = noutput / oplan.samples_per_frame;
@@ -1202,14 +1166,14 @@ struct ChainHandle : dvbt2ll_handle {
     if (n == "chain.luts") {
       // constellation tables of the OFDM fill: { tables, single-table form, copies in shared memory in the last run
       // (0 before any), first entry of each PLP's table }
-      int v[3 + t2::MAX_PLP] = { lut_tables, mixed() ? lut_single : map.plan.im_from_re, lut_copies };
-      for (int i = 0; i < P(); i++) v[3 + i] = mixed() ? lut_base[i] : 0;
+      int v[3 + t2::MAX_PLP] = { lut_tables, lut_single, lut_copies };
+      for (int i = 0; i < P(); i++) v[3 + i] = lut_base[i];
       return copy_out(v, sizeof(int) * (3 + P()), out, cap);
     }
     long long r;
-    if ((r = bb.plan_get(name, out, cap)) >= 0) return r;
-    if ((r = ldpc.plan_get(name, out, cap)) >= 0) return r;
-    if ((r = map.plan_get(name, out, cap)) >= 0) return r;
+    if ((r = sets[0].bb.plan_get(name, out, cap)) >= 0) return r;
+    if ((r = sets[0].ldpc.plan_get(name, out, cap)) >= 0) return r;
+    if ((r = sets[0].map.plan_get(name, out, cap)) >= 0) return r;
     if (n == "frame.code") return copy_vec(fplan.code, out, cap);
     if (n == "frame.ci_dst") return copy_vec(fplan.ci_dst, out, cap);
     if (n == "ofdm.code") return copy_vec(oplan.code, out, cap);
@@ -1279,7 +1243,7 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
   BbHandle *b = h->kind == dvbt2ll_handle::BB ? static_cast<BbHandle *>(h) : 0;
   ChainHandle *ch = h->kind == dvbt2ll_handle::CHAIN ? static_cast<ChainHandle *>(h) : 0;
   if (ch && ch->P() > 1) return fail(DVBT2LL_ERR_INVALID, "chain: a multi-PLP chain takes one TS per PLP: use dvbt2ll_chain_run_host / _run_device");
-  if (ch) b = &ch->bb;          // the chain streams like its first stage: history + frame counter carried across calls
+  if (ch) b = &ch->sets[0].bb;  // the chain streams like its first stage: history + frame counter carried across calls
   // items to stage in
   long long need;
   if (ch) need = ch->ts_bytes(ch->next_frame, frames);
@@ -1592,57 +1556,23 @@ dvbt2ll_handle *dvbt2ll_pilotgenp1insert_create(int carriermode, int fftsize, in
   return h;
 }
 
-static dvbt2ll_handle *chain_create(const dvbt2ll_chain_params *c, int num_plp, const int *plp_fecblocks, int max_frames, int device)
+// own_modcod: every PLP has its own framesize / rate / constellation / rotation (dvbt2ll_chain_create_plps); otherwise
+// they are the chain's, and an over-full frame follows the over-full policy like the reference's frame mapper
+static dvbt2ll_handle *chain_create(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, bool own_modcod,
+                                    int max_frames, int device)
 {
-  if (!c || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
-  if (num_plp < 1 || num_plp > t2::MAX_PLP || (num_plp > 1 && !plp_fecblocks)) { fail(DVBT2LL_ERR_INVALID, "chain: number of PLPs out of range"); return 0; }
-  ChainHandle *h = new ChainHandle();
-  std::string err;
-  h->max_frames = max_frames; h->device = device;
-  int fecblocks = c->fecblocks;
-  if (num_plp > 1) {
-    fecblocks = 0;
-    for (int p = 0; p < num_plp; p++) fecblocks += plp_fecblocks[p];
-  }
-  t2::FrameParams fp = { c->framesize, c->rate, c->constellation, c->rotation, fecblocks, c->tiblocks, c->carriermode,
-                         c->fftsize, c->guardinterval, c->l1constellation, c->pilotpattern, c->t2frames, c->numdatasyms,
-                         c->paprmode, c->version, c->preamble, c->inputmode, c->reservedbiasbits, c->l1scrambled, c->inband };
-  fp.num_plp = num_plp;
-  for (int p = 0; p < num_plp && num_plp > 1; p++) fp.plp_fecblocks[p] = plp_fecblocks[p];
-  t2::OfdmParams op = { c->carriermode, c->fftsize, c->pilotpattern, c->guardinterval, c->numdatasyms, c->paprmode,
-                        c->version, c->preamble, c->misogroup, c->equalization, c->bandwidth, c->vlength };
-  bool ok = true;
-  ok = ok && t2::build_bb_plan(c->framesize, c->rate, c->inputmode, c->inband, fecblocks, c->tsrate, &h->bb.plan, &err);
-  ok = ok && t2::build_ldpc_plan(c->framesize, c->rate, &h->ldpc.plan, &err);
-  ok = ok && t2::build_map_plan(c->framesize, c->rate, c->constellation, c->rotation, &h->map.plan, &err);
-  ok = ok && t2::build_frame_plan(fp, &h->fplan, &err);
-  ok = ok && t2::build_ofdm_plan(op, &h->oplan, &err);
-  ok = ok && t2::compose_chain16(h->fplan, h->oplan, &h->tables, &err);
-  if (!ok) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
-  if (h->fplan.overfull) { h->warnings = 1; g_err = "Frame Mapper, too many FEC blocks in T2 frame."; }
-  return h;
-}
-
-dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, int max_frames,
-                                          int device)
-{
-  if (!c || !plp || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
-  if (num_plp < 1 || num_plp > t2::MAX_PLP) { fail(DVBT2LL_ERR_INVALID, "chain: number of PLPs out of range"); return 0; }
-  int fecblocks = 0;
-  for (int p = 0; p < num_plp; p++) {
-    if (plp[p].fecblocks < 1 || plp[p].fecblocks > 1023) { fail(DVBT2LL_ERR_INVALID, "chain: FEC blocks of a PLP out of range"); return 0; }
-    fecblocks += plp[p].fecblocks;
-  }
   std::unique_ptr<ChainHandle> h(new ChainHandle());
   std::string err;
   h->max_frames = max_frames; h->device = device;
-  // the frame's own FEC / modulation fields are PLP 0's (they name the parameter set of the stages bb / ldpc / map)
+  int fecblocks = 0;
+  for (int p = 0; p < num_plp; p++) fecblocks += plp[p].fecblocks;
+  // the frame's own FEC / modulation fields are PLP 0's
   t2::FrameParams fp = { plp[0].framesize, plp[0].rate, plp[0].constellation, plp[0].rotation, fecblocks, c->tiblocks,
                          c->carriermode, c->fftsize, c->guardinterval, c->l1constellation, c->pilotpattern, c->t2frames,
                          c->numdatasyms, c->paprmode, c->version, c->preamble, c->inputmode, c->reservedbiasbits,
                          c->l1scrambled, c->inband };
   fp.num_plp = num_plp;
-  fp.plp_modcod = 1;
+  fp.plp_modcod = own_modcod ? 1 : 0;
   for (int p = 0; p < num_plp; p++) {
     fp.plp_fecblocks[p] = plp[p].fecblocks;
     fp.plp_framesize[p] = plp[p].framesize; fp.plp_rate[p] = plp[p].rate;
@@ -1652,53 +1582,68 @@ dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *c, int num
                         c->version, c->preamble, c->misogroup, c->equalization, c->bandwidth, c->vlength };
   bool ok = t2::build_frame_plan(fp, &h->fplan, &err);
   // the stages of every parameter set, built from its first PLP: the same checks as a single-PLP chain's
+  if (ok) h->sets.reset(new ChainHandle::Set[h->fplan.plp_sets]);
   for (int s = 0; ok && s < h->fplan.plp_sets; s++) {
-    int p = 0;
-    while (h->fplan.plp_set[p] != s) p++;
-    if (s) h->xset[s].reset(new ChainHandle::Set());
-    BbHandle &bb = s ? h->xset[s]->bb : h->bb;
-    LdpcHandle &ldpc = s ? h->xset[s]->ldpc : h->ldpc;
-    MapHandle &map = s ? h->xset[s]->map : h->map;
-    ok = ok && t2::build_bb_plan(plp[p].framesize, plp[p].rate, c->inputmode, c->inband, fecblocks, c->tsrate, &bb.plan, &err);
-    ok = ok && t2::build_ldpc_plan(plp[p].framesize, plp[p].rate, &ldpc.plan, &err);
-    ok = ok && t2::build_map_plan(plp[p].framesize, plp[p].rate, plp[p].constellation, plp[p].rotation, &map.plan, &err);
+    const dvbt2ll_plp_params &q = plp[h->first_plp(s)];
+    ChainHandle::Set &x = h->sets[s];
+    ok = ok && t2::build_bb_plan(q.framesize, q.rate, c->inputmode, c->inband, fecblocks, c->tsrate, &x.bb.plan, &err);
+    ok = ok && t2::build_ldpc_plan(q.framesize, q.rate, &x.ldpc.plan, &err);
+    ok = ok && t2::build_map_plan(q.framesize, q.rate, q.constellation, q.rotation, &x.map.plan, &err);
   }
   ok = ok && t2::build_ofdm_plan(op, &h->oplan, &err);
   ok = ok && t2::compose_chain16(h->fplan, h->oplan, &h->tables, &err);
   if (!ok) { fail(DVBT2LL_ERR_INVALID, err); return 0; }
-  if (h->mixed()) {
-    // one table per distinct (constellation, rotation), the largest first: the non-data carriers' look-ups (entry =
-    // any cell code, see OFDM_CODE_TAB_SHIFT) stay inside it
-    std::vector<int> order;
-    for (int p = 0; p < num_plp; p++) order.push_back(p);
-    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return plp[x].constellation > plp[y].constellation; });
-    h->lut_tables = 0;
-    h->lut_single = 1;
-    for (size_t i = 0; i < order.size(); i++) {
-      const int p = order[i];
-      const t2::MapPlan &mp = h->map_of(p).plan;
-      h->lut_single &= mp.im_from_re;
-      size_t j = 0;
-      while (j < i && !(plp[order[j]].constellation == plp[p].constellation && plp[order[j]].rotation == plp[p].rotation)) j++;
-      if (j < i) { h->lut_base[p] = h->lut_base[order[j]]; continue; }
-      h->lut_base[p] = (int)h->luts.size();
-      h->luts.insert(h->luts.end(), mp.lut.begin(), mp.lut.end());
-      h->lut_tables++;
-    }
-    h->luts.resize((h->luts.size() + 15) & ~(size_t)15);      // the small pool behind the tables stays 64-byte aligned
-    if (h->luts.size() - 1 > t2k::OFDM_CODE_TAB_MAX) { fail(DVBT2LL_ERR_INVALID, "chain: constellation tables too large"); return 0; }
+  // one table per distinct (constellation, rotation), the largest first: the non-data carriers' look-ups (entry =
+  // any cell code, see OFDM_CODE_TAB_SHIFT) stay inside it
+  std::vector<int> order;
+  for (int p = 0; p < num_plp; p++) order.push_back(p);
+  std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return plp[x].constellation > plp[y].constellation; });
+  h->lut_tables = 0;
+  h->lut_single = 1;
+  for (size_t i = 0; i < order.size(); i++) {
+    const int p = order[i];
+    const t2::MapPlan &mp = h->set_of(p).map.plan;
+    h->lut_single &= mp.im_from_re;
+    size_t j = 0;
+    while (j < i && !(plp[order[j]].constellation == plp[p].constellation && plp[order[j]].rotation == plp[p].rotation)) j++;
+    if (j < i) { h->lut_base[p] = h->lut_base[order[j]]; continue; }
+    h->lut_base[p] = (int)h->luts.size();
+    h->luts.insert(h->luts.end(), mp.lut.begin(), mp.lut.end());
+    h->lut_tables++;
   }
+  // several tables: a multiple of 16 entries, so the small pool behind them in shared memory stays 64-byte aligned
+  // (k_ofdm rounds a lone 4-entry table up to 16 itself)
+  if (h->lut_tables > 1) h->luts.resize((h->luts.size() + 15) & ~(size_t)15);
+  if (h->luts.size() - 1 > t2k::OFDM_CODE_TAB_MAX) { fail(DVBT2LL_ERR_INVALID, "chain: constellation tables too large"); return 0; }
+  if (h->fplan.overfull) { h->warnings = 1; g_err = "Frame Mapper, too many FEC blocks in T2 frame."; }
   return h.release();
 }
 
-dvbt2ll_handle *dvbt2ll_chain_create(const dvbt2ll_chain_params *c, int max_frames, int device)
+dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, int max_frames,
+                                          int device)
 {
-  return chain_create(c, 1, 0, max_frames, device);
+  if (!c || !plp || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
+  if (num_plp < 1 || num_plp > t2::MAX_PLP) { fail(DVBT2LL_ERR_INVALID, "chain: number of PLPs out of range"); return 0; }
+  for (int p = 0; p < num_plp; p++)
+    if (plp[p].fecblocks < 1 || plp[p].fecblocks > 1023) { fail(DVBT2LL_ERR_INVALID, "chain: FEC blocks of a PLP out of range"); return 0; }
+  return chain_create(c, num_plp, plp, true, max_frames, device);
 }
 
 dvbt2ll_handle *dvbt2ll_chain_create_multiplp(const dvbt2ll_chain_params *c, int num_plp, const int *plp_fecblocks, int max_frames, int device)
 {
-  return chain_create(c, num_plp, plp_fecblocks, max_frames, device);
+  if (!c || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
+  if (num_plp < 1 || num_plp > t2::MAX_PLP || (num_plp > 1 && !plp_fecblocks)) { fail(DVBT2LL_ERR_INVALID, "chain: number of PLPs out of range"); return 0; }
+  dvbt2ll_plp_params plp[t2::MAX_PLP];
+  for (int p = 0; p < num_plp; p++) {
+    const dvbt2ll_plp_params q = { num_plp > 1 ? plp_fecblocks[p] : c->fecblocks, c->framesize, c->rate, c->constellation, c->rotation };
+    plp[p] = q;
+  }
+  return chain_create(c, num_plp, plp, false, max_frames, device);
+}
+
+dvbt2ll_handle *dvbt2ll_chain_create(const dvbt2ll_chain_params *c, int max_frames, int device)
+{
+  return dvbt2ll_chain_create_multiplp(c, 1, 0, max_frames, device);
 }
 
 static ChainHandle *as_chain(const dvbt2ll_handle *h)
@@ -1717,7 +1662,7 @@ long long dvbt2ll_chain_history_bytes(const dvbt2ll_handle *h, long long first_f
 {
   ChainHandle *c = as_chain(h);
   if (!c) return -1;
-  return (first_frame > 0 && c->bb.plan.mode == t2::INPUTMODE_NORMAL) ? 187 : 0;
+  return (first_frame > 0 && c->sets[0].bb.plan.mode == t2::INPUTMODE_NORMAL) ? 187 : 0;
 }
 int dvbt2ll_chain_num_plp(const dvbt2ll_handle *h) { ChainHandle *c = as_chain(h); return c ? c->P() : -1; }
 long long dvbt2ll_chain_plp_ts_bytes(const dvbt2ll_handle *h, int plp, long long first_frame, int n_frames)
@@ -1760,7 +1705,7 @@ static int chain_run_host(ChainHandle *c, const void *ts, long long ts_pitch, in
   const int P = c->P();                      // TS rows per channel (row = channel * P + plp)
   const long long per_ch = c->ts_bytes_max(first_frame, n_frames);
   // normal input mode: the CRC-8 that replaces the first sync byte covers the 187 bytes before the pointer
-  const long long hist = (first_frame > 0 && c->bb.plan.mode == t2::INPUTMODE_NORMAL) ? 187 : 0;
+  const long long hist = (first_frame > 0 && c->sets[0].bb.plan.mode == t2::INPUTMODE_NORMAL) ? 187 : 0;
   if (n_channels * P == 1 && ts_pitch < per_ch + hist) ts_pitch = per_ch + hist;      // a single row: the pitch is never used to step
   if (ts_pitch < per_ch + hist)
     return fail(DVBT2LL_ERR_INVALID, "chain: ts_pitch smaller than the TS bytes (+ 187 history bytes) of one channel");
@@ -1850,30 +1795,28 @@ long long dvbt2ll_chain_tap(dvbt2ll_handle *h, const char *stage, void *out, lon
   const void *src; size_t bytes;
   std::string n(stage);
   if ((n.compare(0, 4, "bch.") == 0 || n.compare(0, 4, "fec.") == 0) && n.size() > 4) {
-    // PLP p's codewords [channel][frame][block] at its own pitch: its region of the PLP-major buffers, or gathered from
-    // the frame-major ones
+    // PLP p's codewords [channel][frame][block] at its own pitch, out of its group's region
     char *end = 0;
     const long p = std::strtol(n.c_str() + 4, &end, 10);
     if (*end || p < 0 || p >= c->P()) return fail(DVBT2LL_ERR_INVALID, "chain: unknown tap");
     const bool fec = n[0] == 'f';
-    const size_t pitch = fec ? c->fec_pitch((int)p) : c->bch_pitch((int)p), fp = c->Fp((int)p);
-    const DevBuf &buf = fec ? c->d_fec : c->d_bch;
-    bytes = (size_t)c->last_frames * fp * pitch;
+    const ChainHandle::Group &G = c->grp[c->group_of((int)p)];
+    const size_t pitch = fec ? c->set_of((int)p).fec_pitch() : c->set_of((int)p).bch_pitch(), row = c->Fp((int)p) * pitch;
+    bytes = (size_t)c->last_frames * row;
     CK(cudaStreamSynchronize(c->stream));
     CK(cudaDeviceSynchronize());
     if (!out || cap <= 0) return (long long)bytes;
     std::vector<uint8_t> h(bytes);
-    if (c->mixed()) CK(cudaMemcpy(h.data(), buf.as<uint8_t>() + (fec ? c->fec_off[p] : c->bch_off[p]), bytes, cudaMemcpyDeviceToHost));
-    else
-      for (int f = 0; f < c->last_frames; f++)
-        CK(cudaMemcpy(h.data() + (size_t)f * fp * pitch, buf.as<uint8_t>() + ((size_t)f * c->F() + c->fplan.plp_first_block[p]) * pitch,
-                      fp * pitch, cudaMemcpyDeviceToHost));
+    const uint8_t *region = fec ? c->d_fec.as<uint8_t>() + G.fec_off : c->d_bch.as<uint8_t>() + G.bch_off;
+    CK(cudaMemcpy2D(h.data(), row, region + (size_t)(c->fplan.plp_first_block[p] - c->fplan.plp_first_block[G.p0]) * pitch,
+                    G.blocks * pitch, row, c->last_frames, cudaMemcpyDeviceToHost));
     std::memcpy(out, h.data(), (size_t)cap < bytes ? (size_t)cap : bytes);
     return (long long)bytes;
   }
-  if ((n == "bch" || n == "fec") && c->mixed()) return fail(DVBT2LL_ERR_INVALID, "chain: the PLPs have their own FEC parameters: use the taps bch.<plp> / fec.<plp>");
-  if (n == "bch") { src = c->d_bch.p; bytes = nfec * align16(c->bb.plan.fec.nbch / 8); }
-  else if (n == "fec") { src = c->d_fec.p; bytes = nfec * align16(c->bb.plan.fec.nldpc / 8); }
+  if ((n == "bch" || n == "fec") && c->grp.size() != 1)
+    return fail(DVBT2LL_ERR_INVALID, "chain: the PLPs have their own FEC parameters: use the taps bch.<plp> / fec.<plp>");
+  if (n == "bch") { src = c->d_bch.p; bytes = nfec * c->sets[0].bch_pitch(); }
+  else if (n == "fec") { src = c->d_fec.p; bytes = nfec * c->sets[0].fec_pitch(); }
   else if (n == "cells") { src = c->d_cells.p; bytes = (size_t)c->last_frames * c->cells16_stride() * sizeof(uint16_t); }
   else if (n == "papr") {
     if (c->tr_iter < 1 || c->tr_frames < 1) return fail(DVBT2LL_ERR_INVALID, "chain: the tone-reservation stage is off");

@@ -108,3 +108,10 @@ def test_chain_multiplp_matches_oracle(name):
         assert np.array_equal(alone.view(np.uint32), out[c].view(np.uint32))
         bch = np.unpackbits(ch.tap("bch").reshape(nfr * F, -1)[:, :p_["nbch"] // 8], axis=1)
         assert bits_equal(bch.reshape(-1), want["bch"])
+        # one PLP's codewords: its blocks of every frame of the whole-frame taps
+        first = np.concatenate([[0], np.cumsum(cfg["plp_fecblocks"])])
+        for stage in ("bch", "fec"):
+            whole = ch.tap(stage).reshape(nfr, F, -1)
+            for p in range(P):
+                want_p = whole[:, first[p]:first[p + 1]].reshape(-1)
+                assert np.array_equal(ch.tap("%s.%d" % (stage, p)), want_p), (name, c, stage, p)

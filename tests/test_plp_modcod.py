@@ -30,6 +30,8 @@ CASES = {
     # three constellation tables, room for the longer L1-post
     "c1-3mix": dict(K.CONFIGS["c1"], plps=[plp(1, S, K.C3_5, K.MOD_64QAM, 1), plp(2, S, K.C3_4, K.MOD_16QAM, 1),
                                            plp(2, S, K.C4_5, K.MOD_256QAM, 1)]),
+    # two code rates, one 4-entry QPSK table: two parameter sets whose k_ofdm fill keeps the single-table form
+    "c1-qpsk-rates": dict(K.CONFIGS["c1"], plps=[plp(1, S, K.C1_2, K.MOD_QPSK, 0), plp(1, S, K.C3_5, K.MOD_QPSK, 0)]),
     # mixed PLP_FEC_TYPE, one constellation table (the first PLP takes the cfg's parameters)
     "c1-fectype": dict(K.CONFIGS["c1"], plps=[dict(fecblocks=4), plp(1, N, K.C2_3, K.MOD_256QAM, 1)]),
     # N_P2 = 8 (zig-zag), in-band type B signalling, high-efficiency input mode
