@@ -69,6 +69,43 @@ std::vector<t2::cfloat> make_twiddles(int n, int count)
   return w;
 }
 
+// TS byte index, in a stream that starts on a packet boundary, at which FECFRAME j begins: j FECFRAMEs of `payload`
+// bytes, 13 fewer for the first FECFRAME of every in-band signalling cycle of `cycle` FECFRAMEs (0: no in-band
+// signalling).  In high efficiency mode the sync byte in front of every 187 payload bytes is not carried, and FECFRAME
+// j starts right behind the last payload byte of FECFRAME j - 1.
+long long ts_stream_pos(long long j, int payload, int cycle, int mode)
+{
+  const long long P = j * payload - (cycle > 0 ? 13 * ((j + cycle - 1) / cycle) : 0);     // payload bytes before it
+  if (mode == t2::INPUTMODE_NORMAL || P == 0) return P;
+  return P + (P - 1) / 187 + 1;
+}
+
+// Stream state of a TS-consuming handle (the drop-in BB block, the chain's generic work path), carried across calls
+struct TsStream {
+  long long fecframes;            // FECFRAMEs consumed so far
+  uint8_t history[187];           // last 187 TS bytes consumed (CRC-8 of the packet in flight)
+  int *h_err;                     // sync-error counter in mapped pinned host memory: no copy back per call
+  TsStream() : fecframes(0), h_err(0) { std::memset(history, 0, sizeof(history)); }
+  ~TsStream() { if (h_err) cudaFreeHost(h_err); }
+  int init()
+  {
+    if (!h_err) {
+      CK(cudaHostAlloc((void **)&h_err, 16, cudaHostAllocMapped | cudaHostAllocPortable));
+      std::memset(h_err, 0, 16);
+    }
+    return 0;
+  }
+  // slide the 187-byte history window over `used` newly consumed bytes
+  void note_consumed(const uint8_t *in, long long used)
+  {
+    if (used >= 187) std::memcpy(history, in + used - 187, 187);
+    else if (used > 0) {
+      std::memmove(history, history + used, 187 - (size_t)used);
+      std::memcpy(history + 187 - used, in, (size_t)used);
+    }
+  }
+};
+
 } // namespace
 
 // Device-resident hand-off between two adjacent drop-in blocks (dvbt2ll_link): the producer's last NSLOT outputs, each
@@ -303,7 +340,13 @@ struct dvbt2ll_handle {
   virtual int dev_init() = 0;
   // device-resident work on the given stream
   virtual int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s) = 0;
-  // host-side staging hooks: items that must be copied in for noutput outputs (default = forecast)
+  // items work() must copy in for noutput outputs
+  virtual long long input_items(int noutput) const { return forecast(noutput); }
+  // TS-consuming handles (the BB block, the chain): their stream state, and work_device told whether the 187 bytes in
+  // front of d_in hold the stream's history (work() puts it there; device-resident callers keep it there once anything
+  // has been consumed)
+  virtual TsStream *ts_stream() { return 0; }
+  virtual int work_ts(const void *, int, void *, int, int *, cudaStream_t, int) { return fail(DVBT2LL_ERR_INVALID, "not a TS-consuming handle"); }
   virtual long long plan_get(const char *name, void *out, long long cap) const = 0;
 
   virtual int enter() { return ensure_device(); }
@@ -341,37 +384,13 @@ long long dims_get(const t2::OfdmDims &d, void *out, long long cap)
 }
 
 // ================================================================================================
-struct BbHandle : dvbt2ll_handle {
+// BB framing + BCH (k_bb_bch): the plan, its device tables and the kernel's launch arguments, shared by the drop-in
+// block and the chain's parameter sets
+struct BbStage {
   t2::BbPlan plan;
-  DevBuf d_scr, d_crc, d_tab, d_cols, d_ib, d_ts, d_packed;
-  // streaming state (reference: count, crc via history, fec_block)
-  int count, fec_block;
-  uint8_t history[187];           // last 187 TS bytes consumed (CRC-8 of the packet in flight)
-  long long total_consumed;       // TS bytes consumed so far through work() / work_device()
-  int *h_err;                     // sync-error counter in mapped pinned host memory: no copy back per call
-  BbHandle() : dvbt2ll_handle(BB), count(0), fec_block(0), total_consumed(0), h_err(0) { std::memset(history, 0, sizeof(history)); }
-  ~BbHandle() { if (h_err) cudaFreeHost(h_err); }
-  // slide the 187-byte history window over `used` newly consumed bytes
-  void note_consumed(const uint8_t *in, long long used)
-  {
-    if (used >= 187) std::memcpy(history, in + used - 187, 187);
-    else if (used > 0) {
-      std::memmove(history, history + used, 187 - (size_t)used);
-      std::memcpy(history + 187 - used, in, (size_t)used);
-    }
-  }
-
-  int output_multiple() const { return plan.fec.nbch; }
-  int in_item() const { return 1; }
-  int out_item() const { return 1; }
-  int forecast(int noutput) const
-  {
-    // reference :207-216
-    const int base = (noutput - 80 - (plan.fec.nbch - plan.fec.kbch)) / 8;
-    return plan.mode == t2::INPUTMODE_NORMAL ? base : base + ((plan.fec.kbch - 80) / 8) / 187 + 1;
-  }
+  DevBuf d_scr, d_crc, d_tab, d_cols, d_ib;
   uint32_t crc_pos_mask[47][8];
-  int dev_init()
+  int init()
   {
     std::vector<uint8_t> scr(plan.scramble);
     scr.resize((scr.size() + 7) & ~(size_t)3, 0);      // kernel XORs the scrambler word-wise
@@ -407,29 +426,11 @@ struct BbHandle : dvbt2ll_handle {
     CK(upload(d_tab, plan.bch_byte_tab));
     CK(upload(d_cols, plan.bch_shift_cols));
     CK(upload(d_ib, plan.inband_bytes));
-    if (!h_err) {
-      CK(cudaHostAlloc((void **)&h_err, 16, cudaHostAllocMapped | cudaHostAllocPortable));
-      std::memset(h_err, 0, 16);
-    }
     return 0;
   }
-  // payload bytes of `frames` FECFRAMEs starting at in-band phase fb0
-  long long payload_bytes(int frames, int fb0) const
-  {
-    long long nb = 0;
-    if (plan.inband) nb = (fb0 + frames + plan.fecblocks - 1) / plan.fecblocks - (fb0 + plan.fecblocks - 1) / plan.fecblocks;
-    return (long long)frames * plan.payload_bytes - 13 * nb;
-  }
-  long long ts_needed(int frames) const
-  {
-    const long long P = payload_bytes(frames, fec_block);
-    if (plan.mode == t2::INPUTMODE_NORMAL || P == 0) return P;
-    const int t0 = (188 - count) % 188;
-    const long long last = P - 1;
-    return (last < t0 ? last : t0 + 1 + (last - t0) + (last - t0) / 187) + 1;
-  }
+  // sync_errors: the caller's counter of payload sync bytes != 0x47 (device-visible)
   void fill_args(t2k::BbArgs &a, const uint8_t *d_ts_ptr, long long pitch, int channels, int frames, int count0,
-                 int fb0, int hist_valid, uint8_t *d_out, int out_pitch)
+                 int fb0, int hist_valid, uint8_t *d_out, int out_pitch, int *sync_errors) const
   {
     a.ts = d_ts_ptr; a.ts_pitch = pitch; a.hist_valid = hist_valid; a.n_channels = channels; a.frames = frames;
     a.count0 = count0; a.fec_block0 = fb0;
@@ -439,33 +440,10 @@ struct BbHandle : dvbt2ll_handle {
     a.scramble = d_scr.as<uint8_t>(); a.crc8_tab = d_crc.as<uint8_t>(); a.bch_tab = d_tab.as<uint32_t>();
     std::memcpy(a.crc8_pos_mask, crc_pos_mask, sizeof(crc_pos_mask));
     a.bch_cols = d_cols.as<uint32_t>(); a.inband_bytes = d_ib.as<uint8_t>();
-    a.out = d_out; a.out_pitch = out_pitch; a.sync_errors = h_err;
+    a.out = d_out; a.out_pitch = out_pitch; a.sync_errors = sync_errors;
     a.ts_len = 0; a.out_len = (long long)channels * frames * out_pitch;
     a.out_group = 0; a.out_group_stride = 0; a.out_group_off = 0;
   }
-  // d_in must be preceded by 187 bytes of valid history on the device (work() arranges that)
-  int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
-  {
-    const int frames = noutput / plan.fec.nbch;
-    if (consumed) *consumed = 0;
-    if (frames < 1) return 0;
-    const long long need = ts_needed(frames);
-    if (ninput < need) return fail(DVBT2LL_ERR_SHORT, "bbheaderbch_bb: not enough input items");
-    const int pitch = align16(plan.fec.nbch / 8);
-    CK(d_packed.ensure((size_t)frames * pitch));
-    t2k::BbArgs a;
-    fill_args(a, (const uint8_t *)d_in, 0, 1, frames, count, fec_block, hist_on_device, d_packed.as<uint8_t>(), pitch);
-    a.ts_len = ninput;
-    t2k::launch_bb_bch(a, s);
-    t2k::launch_unpack_bits(d_packed.as<uint8_t>(), pitch, plan.fec.nbch, (uint8_t *)d_out, frames, s);
-    CK(cudaGetLastError());
-    count = (int)((count + need) % 188);
-    if (plan.inband) fec_block = (fec_block + frames) % plan.fecblocks;
-    total_consumed += need;
-    if (consumed) *consumed = (int)need;
-    return frames * plan.fec.nbch;
-  }
-  int hist_on_device = 0;
   long long plan_get(const char *name, void *out, long long cap) const
   {
     std::string n(name);
@@ -483,17 +461,71 @@ struct BbHandle : dvbt2ll_handle {
   }
 };
 
-// ================================================================================================
-struct LdpcHandle : dvbt2ll_handle {
-  t2::LdpcPlan plan;
-  DevBuf d_rowptr, d_entries, d_in_packed, d_out_packed;
-  int lane_per_row;         // accumulation scheme of k_ldpc, chosen per code in dev_init (DVBT2LL_LDPC_MODE=0|1 overrides)
-  LdpcHandle() : dvbt2ll_handle(LDPC), lane_per_row(0) {}
-  int output_multiple() const { return plan.fec.nldpc; }
+// the drop-in block: the stage, its stream state and the conversion of its packed codewords to one bit per byte
+struct BbHandle : dvbt2ll_handle {
+  BbStage st;
+  TsStream ts;
+  DevBuf d_packed;
+  BbHandle() : dvbt2ll_handle(BB) {}
+  TsStream *ts_stream() override { return &ts; }
+  int output_multiple() const { return st.plan.fec.nbch; }
   int in_item() const { return 1; }
   int out_item() const { return 1; }
-  int forecast(int noutput) const { return (noutput / plan.fec.nldpc) * plan.fec.nbch; }
+  int forecast(int noutput) const
+  {
+    // reference :207-216
+    const t2::BbPlan &p = st.plan;
+    const int base = (noutput - 80 - (p.fec.nbch - p.fec.kbch)) / 8;
+    return p.mode == t2::INPUTMODE_NORMAL ? base : base + ((p.fec.kbch - 80) / 8) / 187 + 1;
+  }
   int dev_init()
+  {
+    int r = st.init();
+    return r ? r : ts.init();
+  }
+  // TS byte index at which FECFRAME j starts: one in-band signalling cycle per `fecblocks` FECFRAMEs
+  long long stream_pos(long long j) const { return ts_stream_pos(j, st.plan.payload_bytes, st.plan.inband ? st.plan.fecblocks : 0, st.plan.mode); }
+  long long input_items(int noutput) const override
+  {
+    return stream_pos(ts.fecframes + noutput / st.plan.fec.nbch) - stream_pos(ts.fecframes);
+  }
+  // the 187 bytes before d_in are read once anything has been consumed (see the header); at the very start of the
+  // stream the history is all zero by definition
+  int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
+  {
+    return work_ts(d_in, ninput, d_out, noutput, consumed, s, ts.fecframes > 0 ? 1 : 0);
+  }
+  int work_ts(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s, int hist_valid) override
+  {
+    const t2::BbPlan &p = st.plan;
+    const int frames = noutput / p.fec.nbch;
+    if (consumed) *consumed = 0;
+    if (frames < 1) return 0;
+    const long long need = input_items(noutput);
+    if (ninput < need) return fail(DVBT2LL_ERR_SHORT, "bbheaderbch_bb: not enough input items");
+    const int pitch = align16(p.fec.nbch / 8);
+    CK(d_packed.ensure((size_t)frames * pitch));
+    t2k::BbArgs a;
+    st.fill_args(a, (const uint8_t *)d_in, 0, 1, frames, (int)(stream_pos(ts.fecframes) % 188),
+                 p.inband ? (int)(ts.fecframes % p.fecblocks) : 0, hist_valid, d_packed.as<uint8_t>(), pitch, ts.h_err);
+    a.ts_len = ninput;
+    t2k::launch_bb_bch(a, s);
+    t2k::launch_unpack_bits(d_packed.as<uint8_t>(), pitch, p.fec.nbch, (uint8_t *)d_out, frames, s);
+    CK(cudaGetLastError());
+    ts.fecframes += frames;
+    if (consumed) *consumed = (int)need;
+    return frames * p.fec.nbch;
+  }
+  long long plan_get(const char *name, void *out, long long cap) const { return st.plan_get(name, out, cap); }
+};
+
+// ================================================================================================
+// LDPC encoding (k_ldpc), shared like BbStage
+struct LdpcStage {
+  t2::LdpcPlan plan;
+  DevBuf d_rowptr, d_entries;
+  int lane_per_row = 0;     // accumulation scheme of k_ldpc, chosen per code in init (DVBT2LL_LDPC_MODE=0|1 overrides)
+  int init()
   {
     CK(upload(d_rowptr, plan.row_ptr));
     CK(upload(d_entries, plan.entries));
@@ -509,31 +541,13 @@ struct LdpcHandle : dvbt2ll_handle {
     // a lane per (row, word) for the others (consecutive lanes read consecutive words: fewer bank conflicts)
     return nldpc == 64800 ? (q >= 90 ? 1 : 0) : (q >= 18 ? 1 : 0);
   }
-  void fill_args(t2k::LdpcArgs &a, const uint8_t *in, int in_pitch, uint8_t *out, int out_pitch, int frames)
+  void fill_args(t2k::LdpcArgs &a, const uint8_t *in, int in_pitch, uint8_t *out, int out_pitch, int frames) const
   {
     a.in = in; a.in_pitch = in_pitch; a.out = out; a.out_pitch = out_pitch; a.frames = frames;
     a.nbch = plan.fec.nbch; a.nldpc = plan.fec.nldpc; a.q = plan.fec.q; a.groups = plan.groups;
     a.row_ptr = d_rowptr.as<uint16_t>(); a.entries = d_entries.as<uint32_t>();
     a.lane_per_row = lane_per_row;
     a.in_len = (long long)frames * in_pitch + 64; a.out_len = (long long)frames * out_pitch;
-  }
-  int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
-  {
-    const int frames = noutput / plan.fec.nldpc;
-    if (consumed) *consumed = 0;
-    if (frames < 1) return 0;
-    if (ninput < frames * plan.fec.nbch) return fail(DVBT2LL_ERR_SHORT, "ldpc: not enough input items");
-    const int ip = align16(plan.fec.nbch / 8), op = align16(plan.fec.nldpc / 8);
-    CK(d_in_packed.ensure((size_t)frames * ip + 64));
-    CK(d_out_packed.ensure((size_t)frames * op + 16));
-    t2k::launch_pack_bits((const uint8_t *)d_in, plan.fec.nbch, d_in_packed.as<uint8_t>(), ip, frames, s);
-    t2k::LdpcArgs a;
-    fill_args(a, d_in_packed.as<uint8_t>(), ip, d_out_packed.as<uint8_t>(), op, frames);
-    t2k::launch_ldpc(a, s);
-    t2k::launch_unpack_ldpc(d_out_packed.as<uint8_t>(), op, plan.fec.nbch, plan.fec.nldpc, plan.fec.q, (uint8_t *)d_out, frames, s);
-    CK(cudaGetLastError());
-    if (consumed) *consumed = frames * plan.fec.nbch;
-    return frames * plan.fec.nldpc;
   }
   long long plan_get(const char *name, void *out, long long cap) const
   {
@@ -544,23 +558,51 @@ struct LdpcHandle : dvbt2ll_handle {
   }
 };
 
-// ================================================================================================
-struct MapHandle : dvbt2ll_handle {
-  t2::MapPlan plan;
-  DevBuf d_bitsrc, d_lut, d_packed, d_qlut;
-  MapHandle() : dvbt2ll_handle(MAP) {}
-  int output_multiple() const { return plan.cell_size; }
+// the drop-in block: the stage and the conversion between one bit per byte and packed codewords
+struct LdpcHandle : dvbt2ll_handle {
+  LdpcStage st;
+  DevBuf d_in_packed, d_out_packed;
+  LdpcHandle() : dvbt2ll_handle(LDPC) {}
+  int output_multiple() const { return st.plan.fec.nldpc; }
   int in_item() const { return 1; }
-  int out_item() const { return 8; }
-  int forecast(int noutput) const { return (noutput / plan.cell_size) * plan.fec.nldpc; }
-  int dev_init()
+  int out_item() const { return 1; }
+  int forecast(int noutput) const { return (noutput / st.plan.fec.nldpc) * st.plan.fec.nbch; }
+  int dev_init() { return st.init(); }
+  int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
+  {
+    const t2::FecSpec &f = st.plan.fec;
+    const int frames = noutput / f.nldpc;
+    if (consumed) *consumed = 0;
+    if (frames < 1) return 0;
+    if (ninput < frames * f.nbch) return fail(DVBT2LL_ERR_SHORT, "ldpc: not enough input items");
+    const int ip = align16(f.nbch / 8), op = align16(f.nldpc / 8);
+    CK(d_in_packed.ensure((size_t)frames * ip + 64));
+    CK(d_out_packed.ensure((size_t)frames * op + 16));
+    t2k::launch_pack_bits((const uint8_t *)d_in, f.nbch, d_in_packed.as<uint8_t>(), ip, frames, s);
+    t2k::LdpcArgs a;
+    st.fill_args(a, d_in_packed.as<uint8_t>(), ip, d_out_packed.as<uint8_t>(), op, frames);
+    t2k::launch_ldpc(a, s);
+    t2k::launch_unpack_ldpc(d_out_packed.as<uint8_t>(), op, f.nbch, f.nldpc, f.q, (uint8_t *)d_out, frames, s);
+    CK(cudaGetLastError());
+    if (consumed) *consumed = frames * f.nbch;
+    return frames * f.nldpc;
+  }
+  long long plan_get(const char *name, void *out, long long cap) const { return st.plan_get(name, out, cap); }
+};
+
+// ================================================================================================
+// bit interleaving + constellation mapping (k_map), shared like BbStage
+struct MapStage {
+  t2::MapPlan plan;
+  DevBuf d_bitsrc, d_lut, d_qlut;
+  int init()
   {
     CK(upload(d_bitsrc, plan.bit_src));
     CK(upload(d_lut, plan.lut));
     if (!plan.qpsk_lut.empty()) CK(upload(d_qlut, plan.qpsk_lut));
     return 0;
   }
-  void fill_args(t2k::MapArgs &a, const uint8_t *in, int in_pitch, float2 *out, int frames)
+  void fill_args(t2k::MapArgs &a, const uint8_t *in, int in_pitch, float2 *out, int frames) const
   {
     a.in = in; a.in_pitch = in_pitch; a.out = out; a.frames = frames;
     a.nldpc = plan.fec.nldpc; a.mod = plan.mod; a.cell_size = plan.cell_size; a.cyclic_delay = plan.cyclic_delay;
@@ -574,22 +616,6 @@ struct MapHandle : dvbt2ll_handle {
     std::memcpy(a.col_of_bit, plan.col_of_bit, 16);
     std::memcpy(a.twist_of_col, plan.twist_of_col, 16);
   }
-  int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
-  {
-    const int frames = noutput / plan.cell_size;
-    if (consumed) *consumed = 0;
-    if (frames < 1) return 0;
-    if (ninput < frames * plan.fec.nldpc) return fail(DVBT2LL_ERR_SHORT, "interleavermod_bc: not enough input items");
-    const int ip = align16(plan.fec.nldpc / 8);
-    CK(d_packed.ensure((size_t)frames * ip + 16));
-    t2k::launch_pack_ldpc((const uint8_t *)d_in, plan.fec.nbch, plan.fec.nldpc, plan.fec.q, d_packed.as<uint8_t>(), ip, frames, s);
-    t2k::MapArgs a;
-    fill_args(a, d_packed.as<uint8_t>(), ip, (float2 *)d_out, frames);
-    t2k::launch_map(a, s);
-    CK(cudaGetLastError());
-    if (consumed) *consumed = frames * plan.fec.nldpc;
-    return frames * plan.cell_size;
-  }
   long long plan_get(const char *name, void *out, long long cap) const
   {
     std::string n(name);
@@ -599,6 +625,36 @@ struct MapHandle : dvbt2ll_handle {
     if (n == "map.im_from_re") { const int v[4] = { plan.im_from_re, (int)plan.im_mask_i, (int)plan.im_mask_q, (int)plan.im_flip }; return copy_out(v, sizeof(v), out, cap); }
     return -1;
   }
+};
+
+// the drop-in block: the stage and the packing of the codeword items
+struct MapHandle : dvbt2ll_handle {
+  MapStage st;
+  DevBuf d_packed;
+  MapHandle() : dvbt2ll_handle(MAP) {}
+  int output_multiple() const { return st.plan.cell_size; }
+  int in_item() const { return 1; }
+  int out_item() const { return 8; }
+  int forecast(int noutput) const { return (noutput / st.plan.cell_size) * st.plan.fec.nldpc; }
+  int dev_init() { return st.init(); }
+  int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
+  {
+    const t2::MapPlan &p = st.plan;
+    const int frames = noutput / p.cell_size;
+    if (consumed) *consumed = 0;
+    if (frames < 1) return 0;
+    if (ninput < frames * p.fec.nldpc) return fail(DVBT2LL_ERR_SHORT, "interleavermod_bc: not enough input items");
+    const int ip = align16(p.fec.nldpc / 8);
+    CK(d_packed.ensure((size_t)frames * ip + 16));
+    t2k::launch_pack_ldpc((const uint8_t *)d_in, p.fec.nbch, p.fec.nldpc, p.fec.q, d_packed.as<uint8_t>(), ip, frames, s);
+    t2k::MapArgs a;
+    st.fill_args(a, d_packed.as<uint8_t>(), ip, (float2 *)d_out, frames);
+    t2k::launch_map(a, s);
+    CK(cudaGetLastError());
+    if (consumed) *consumed = frames * p.fec.nldpc;
+    return frames * p.cell_size;
+  }
+  long long plan_get(const char *name, void *out, long long cap) const { return st.plan_get(name, out, cap); }
 };
 
 // ================================================================================================
@@ -807,12 +863,12 @@ std::vector<uint16_t> make_ci_inv4(const std::vector<uint16_t> &ci_inv, int *str
 
 struct ChainHandle : dvbt2ll_handle {
   // the stages of each PLP parameter set (fplan.plp_set: a distinct framesize, rate, constellation and rotation), built
-  // from the set's first PLP, with that PLP's inverse cell permutation; set 0 also carries the chain-wide BB fields
-  // (input mode, in-band signalling, sync-error counter)
+  // from the set's first PLP, with that PLP's inverse cell permutation; the chain-wide BB fields (input mode, in-band
+  // signalling) are fplan.prm's, and every set's BB launch counts sync errors in the chain's stream state
   struct Set {
-    BbHandle bb;
-    LdpcHandle ldpc;
-    MapHandle map;
+    BbStage bb;
+    LdpcStage ldpc;
+    MapStage map;
     DevBuf d_ci_inv, d_ci_inv4;
     int ci4_stride;
     int bch_pitch() const { return align16(bb.plan.fec.nbch / 8); }
@@ -852,12 +908,12 @@ struct ChainHandle : dvbt2ll_handle {
   std::unique_ptr<MisoGroup> miso_g[2];
   bool miso_on;
   int last_frames;
-  long long next_frame;  // stream position of the generic work() / work_device() path (T2 frames consumed so far)
+  TsStream ts;           // stream state of the generic work() / work_device() path
   bool timing;
   enum { TIMING_SLOTS = 64 };
   cudaEvent_t ev[TIMING_SLOTS][5];     // per-run event sets so the timed loop never has to synchronise
   long long n_timed;
-  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), tr_iter(0), tr_vclip(0.f), tr_tone_max(0.f), tr_built(false), tr_uploaded(false), tr_frames(0), miso_on(false), last_frames(0), next_frame(0), timing(false)
+  ChainHandle() : dvbt2ll_handle(CHAIN), lut_tables(1), lut_single(0), lut_copies(0), max_frames(0), device(0), sink_fmt(0), sink_gain(1.0f), stream2(0), tr_iter(0), tr_vclip(0.f), tr_tone_max(0.f), tr_built(false), tr_uploaded(false), tr_frames(0), miso_on(false), last_frames(0), timing(false)
   {
     n_timed = 0;
     for (int s = 0; s < TIMING_SLOTS; s++) for (int i = 0; i < 5; i++) ev[s][i] = 0;
@@ -885,17 +941,11 @@ struct ChainHandle : dvbt2ll_handle {
   int Fp(int plp) const { return fplan.plp_first_block[plp + 1] - fplan.plp_first_block[plp]; }
   // cells per T2 frame in the 16-bit cell memory, padded so every frame starts on a 16-byte boundary (bulk copies)
   long long cells16_stride() const { return ((long long)fplan.plp_chain_off[P()] + 7) & ~7LL; }
-  // TS byte index (per channel, stream starts on a packet boundary) at which T2 frame `frame` begins
+  // TS byte index (per channel) at which T2 frame `frame` begins in PLP `plp`'s stream: the PLP's FEC blocks per T2
+  // frame are its in-band signalling cycle
   long long stream_pos(long long frame, int plp = 0) const
   {
-    const int fpl = Fp(plp);            // the PLP's FEC blocks per T2 frame = its in-band signalling cycle
-    const long long j0 = frame * fpl;
-    long long nb0 = 0;
-    if (sets[0].bb.plan.inband) nb0 = (j0 + fpl - 1) / fpl;
-    const long long P = j0 * set_of(plp).bb.plan.payload_bytes - 13 * nb0;  // payload bytes before the frame
-    if (sets[0].bb.plan.mode == t2::INPUTMODE_NORMAL || P == 0) return P;
-    const long long last = P - 1;                                       // high efficiency mode: sync bytes are skipped,
-    return 1 + last + last / 187 + 1;                                   // packets = 1 sync + 187 payload bytes
+    return ts_stream_pos(frame * Fp(plp), set_of(plp).bb.plan.payload_bytes, fplan.prm.inband ? Fp(plp) : 0, fplan.prm.inputmode);
   }
   long long ts_bytes(long long first_frame, int n_frames, int plp = 0) const { return stream_pos(first_frame + n_frames, plp) - stream_pos(first_frame, plp); }
   long long ts_bytes_max(long long first_frame, int n_frames) const
@@ -905,6 +955,11 @@ struct ChainHandle : dvbt2ll_handle {
     return m;
   }
   long long ts_per_frame() const { return ts_bytes(0, 1); }
+  // stream bytes that must precede the first TS byte of `first_frame` in every TS row: in normal input mode the CRC-8
+  // that replaces the first sync byte covers the 187 bytes before the pointer
+  long long history_bytes(long long first_frame) const { return (first_frame > 0 && fplan.prm.inputmode == t2::INPUTMODE_NORMAL) ? 187 : 0; }
+  // the generic work path's stream position in T2 frames
+  long long next_frame() const { return ts.fecframes / F(); }
   int output_multiple() const { return oplan.samples_per_frame; }
   int in_item() const { return 1; }
   int out_item() const { return sink_fmt ? 4 : 8; }
@@ -914,11 +969,12 @@ struct ChainHandle : dvbt2ll_handle {
     int r;
     for (int s = 0; s < fplan.plp_sets; s++) {
       Set &x = sets[s];
-      if ((r = x.bb.dev_init()) || (r = x.ldpc.dev_init()) || (r = x.map.dev_init())) return r;
+      if ((r = x.bb.init()) || (r = x.ldpc.init()) || (r = x.map.init())) return r;
       const std::vector<uint16_t> &ci_inv = fplan.plp_cell_perm_inv[first_plp(s)];
       CK(upload(x.d_ci_inv, ci_inv));
       CK(upload(x.d_ci_inv4, make_ci_inv4(ci_inv, &x.ci4_stride)));
     }
+    if ((r = ts.init())) return r;
     if ((r = odev.init(tables.code, tables.pool, oplan, true, &tables.plp, lut_tables > 1 ? lut_base : 0))) return r;
     CK(upload(d_luts, luts));
     CK(upload(d_fec_shift, fplan.fec_shift));
@@ -982,12 +1038,11 @@ struct ChainHandle : dvbt2ll_handle {
       const Group &G = grp[group_of(pl)];
       Set &x = set_of(pl);
       const int fpl = Fp(pl), bp = x.bch_pitch();
-      const long long j0 = first_frame * fpl;
-      const int fb0 = sets[0].bb.plan.inband ? (int)(j0 % fpl) : 0;
       const int count0 = (int)(stream_pos(first_frame, pl) % 188);
+      // every T2 frame begins an in-band signalling cycle (in-band phase 0)
       t2k::BbArgs ba;
-      x.bb.fill_args(ba, (const uint8_t *)d_ts + (long long)pl * ts_pitch, ts_pitch * P(), n_channels, n_frames * fpl, count0, fb0,
-                     hist_valid >= 0 ? hist_valid : (first_frame > 0 ? 1 : 0), bch_buf(G), bp);
+      x.bb.fill_args(ba, (const uint8_t *)d_ts + (long long)pl * ts_pitch, ts_pitch * P(), n_channels, n_frames * fpl, count0, 0,
+                     hist_valid >= 0 ? hist_valid : (first_frame > 0 ? 1 : 0), bch_buf(G), bp, ts.h_err);
       ba.fecblocks = fpl;
       ba.ts_len = ts_bytes(first_frame, n_frames, pl);
       ba.out_len = (long long)frames * G.blocks * bp;
@@ -1112,18 +1167,24 @@ struct ChainHandle : dvbt2ll_handle {
     tr_uploaded = true;
     return 0;
   }
+  // the generic work path streams like the drop-in BB block: stream state carried across calls, 187 history bytes in
+  // front of d_in once anything has been consumed (normal input mode)
+  TsStream *ts_stream() override { return &ts; }
+  long long input_items(int noutput) const override { return ts_bytes(next_frame(), noutput / oplan.samples_per_frame); }
   int work_device(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s)
+  {
+    return work_ts(d_in, ninput, d_out, noutput, consumed, s, ts.fecframes > 0 ? 1 : 0);
+  }
+  int work_ts(const void *d_in, int ninput, void *d_out, int noutput, int *consumed, cudaStream_t s, int hist_valid) override
   {
     const int frames = noutput / oplan.samples_per_frame;
     if (consumed) *consumed = 0;
     if (frames < 1) return 0;
-    // streams like the first stage: frame counter carried across calls, 187 history bytes in front of d_in once
-    // anything has been consumed (normal input mode)
-    const long long need = ts_bytes(next_frame, frames);
+    const long long need = input_items(noutput);
     if ((long long)ninput < need) return fail(DVBT2LL_ERR_SHORT, "chain: not enough input items");
-    int r = run(d_in, 0, 1, frames, next_frame, d_out, s);
+    int r = run(d_in, 0, 1, frames, next_frame(), d_out, s, 0, hist_valid);
     if (r < 0) return r;
-    next_frame += frames;
+    ts.fecframes += (long long)frames * F();
     if (consumed) *consumed = (int)need;
     return frames * oplan.samples_per_frame;
   }
@@ -1218,12 +1279,6 @@ int dvbt2ll_work_device(dvbt2ll_handle *h, const void *d_in, int ninput, void *d
   if (!h) return fail(DVBT2LL_ERR_INVALID, "null handle");
   int r = h->enter();
   if (r) return r;
-  if (h->kind == dvbt2ll_handle::BB) {
-    // device-resident callers keep the 187 stream bytes before d_in in front of it (see the header): they are read
-    // once anything has been consumed; at the very start of the stream the history is all zero by definition
-    BbHandle *b = static_cast<BbHandle *>(h);
-    b->hist_on_device = b->total_consumed > 0 ? 1 : 0;
-  }
   cudaStream_t s = stream ? (cudaStream_t)stream : h->stream;
   r = h->work_device(d_in, ninput, d_out, noutput, consumed, s);
   if (r >= 0 && !stream) CK(cudaStreamSynchronize(s));
@@ -1240,15 +1295,10 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
   const int frames = noutput / om;
   if (frames < 1) return 0;
   const int nout = frames * om;
-  BbHandle *b = h->kind == dvbt2ll_handle::BB ? static_cast<BbHandle *>(h) : 0;
+  TsStream *ts = h->ts_stream();    // TS-consuming handles: history + stream position carried across calls
   ChainHandle *ch = h->kind == dvbt2ll_handle::CHAIN ? static_cast<ChainHandle *>(h) : 0;
   if (ch && ch->P() > 1) return fail(DVBT2LL_ERR_INVALID, "chain: a multi-PLP chain takes one TS per PLP: use dvbt2ll_chain_run_host / _run_device");
-  if (ch) b = &ch->sets[0].bb;  // the chain streams like its first stage: history + frame counter carried across calls
-  // items to stage in
-  long long need;
-  if (ch) need = ch->ts_bytes(ch->next_frame, frames);
-  else if (b) need = b->ts_needed(frames);
-  else need = (long long)h->forecast(nout);
+  const long long need = h->input_items(nout);
   if (ninput < need) return fail(DVBT2LL_ERR_SHORT, "not enough input items for the requested output");
   if (ch && frames > ch->max_frames) return fail(DVBT2LL_ERR_INVALID, "chain: more frames requested than max_frames given at create");
   DevBuf &d_in = h->stage_in;
@@ -1263,7 +1313,7 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
     h->link_out->item = h->out_item();
     AutoLinks::get().add(h->link_out);
   }
-  if (!found_in && auto_link && !b) {
+  if (!found_in && auto_link && !ts) {
     // not linked explicitly: try the record that matched last time, then every other block's (one lock at a time)
     const uint8_t *ip = (const uint8_t *)in;
     std::vector<std::shared_ptr<LinkRec> > cand;
@@ -1298,7 +1348,7 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
   };
   const uint8_t *resident = 0;           // the input items, if the upstream block left them in HBM
   LinkRec::Slot *taken = 0;
-  if (found_in && !b) {
+  if (found_in && !ts) {
     LinkRec &L = *found_in;
     const uint8_t *ip = (const uint8_t *)in;
     for (int k = 1; k <= LinkRec::NSLOT && !taken; k++) {         // newest first
@@ -1354,16 +1404,10 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
   // call) turns the two copies into DMA transfers at full PCIe rate instead of staged pageable copies
   if (!resident) h->pin(in, in_bytes);
   h->pin(out, out_bytes);
-  if (b) {
-    CK(cudaMemcpyAsync(din - 187, b->history, 187, cudaMemcpyHostToDevice, s));
-    b->hist_on_device = 1;
-  }
+  if (ts) CK(cudaMemcpyAsync(din - 187, ts->history, 187, cudaMemcpyHostToDevice, s));
   if (!resident) CK(h->copy_host(din, in, in_bytes, cudaMemcpyHostToDevice, s));
   int used = 0;
-  if (ch) {
-    r = ch->run(din, 0, 1, frames, ch->next_frame, d_out.p, s, 0, 1);
-    if (r >= 0) { r = nout; used = (int)need; ch->next_frame += frames; }
-  }
+  if (ts) r = h->work_ts(din, (int)need, d_out.p, nout, &used, s, 1);     // the history uploaded above
   else r = h->work_device(din, (int)need, d_out.p, nout, &used, s);
   if (r < 0) return r;
   if (resident) {
@@ -1376,9 +1420,9 @@ int dvbt2ll_work(dvbt2ll_handle *h, const void *in, int ninput, void *out, int n
   const bool lazy_out = h->link_out && h->link_out->lazy;      // (only ever changed by this block's own thread)
   if (!lazy_out) CK(h->copy_host(out, d_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
-  if (b) {
-    h->warnings = *b->h_err;         // mapped host counter, complete after the synchronize
-    b->note_consumed((const uint8_t *)in, used);
+  if (ts) {
+    h->warnings = *ts->h_err;        // mapped host counter, complete after the synchronize
+    ts->note_consumed((const uint8_t *)in, used);
   }
   if (mine) {
     lk_out.lock();
@@ -1508,7 +1552,7 @@ dvbt2ll_handle *dvbt2ll_bbheaderbch_create(int framesize, int rate, int mode, in
   BbHandle *h = new BbHandle();
   std::string err;
   if (mode != t2::INPUTMODE_NORMAL && mode != t2::INPUTMODE_HIEFF) { delete h; fail(DVBT2LL_ERR_INVALID, "bbheaderbch_bb: unknown input mode"); return 0; }
-  if (!t2::build_bb_plan(framesize, rate, mode, inband, fecblocks, tsrate, &h->plan, &err)) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
+  if (!t2::build_bb_plan(framesize, rate, mode, inband, fecblocks, tsrate, &h->st.plan, &err)) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
   return h;
 }
 
@@ -1516,7 +1560,7 @@ dvbt2ll_handle *dvbt2ll_ldpc_create(int framesize, int rate)
 {
   LdpcHandle *h = new LdpcHandle();
   std::string err;
-  if (!t2::build_ldpc_plan(framesize, rate, &h->plan, &err)) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
+  if (!t2::build_ldpc_plan(framesize, rate, &h->st.plan, &err)) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
   return h;
 }
 
@@ -1524,7 +1568,7 @@ dvbt2ll_handle *dvbt2ll_interleavermod_create(int framesize, int rate, int const
 {
   MapHandle *h = new MapHandle();
   std::string err;
-  if (!t2::build_map_plan(framesize, rate, constellation, rotation, &h->plan, &err)) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
+  if (!t2::build_map_plan(framesize, rate, constellation, rotation, &h->st.plan, &err)) { delete h; fail(DVBT2LL_ERR_INVALID, err); return 0; }
   return h;
 }
 
@@ -1661,8 +1705,7 @@ long long dvbt2ll_chain_ts_bytes(const dvbt2ll_handle *h, long long first_frame,
 long long dvbt2ll_chain_history_bytes(const dvbt2ll_handle *h, long long first_frame)
 {
   ChainHandle *c = as_chain(h);
-  if (!c) return -1;
-  return (first_frame > 0 && c->sets[0].bb.plan.mode == t2::INPUTMODE_NORMAL) ? 187 : 0;
+  return c ? c->history_bytes(first_frame) : -1;
 }
 int dvbt2ll_chain_num_plp(const dvbt2ll_handle *h) { ChainHandle *c = as_chain(h); return c ? c->P() : -1; }
 long long dvbt2ll_chain_plp_ts_bytes(const dvbt2ll_handle *h, int plp, long long first_frame, int n_frames)
@@ -1704,8 +1747,7 @@ static int chain_run_host(ChainHandle *c, const void *ts, long long ts_pitch, in
   if (n_channels == 0 || n_frames == 0) return 0;
   const int P = c->P();                      // TS rows per channel (row = channel * P + plp)
   const long long per_ch = c->ts_bytes_max(first_frame, n_frames);
-  // normal input mode: the CRC-8 that replaces the first sync byte covers the 187 bytes before the pointer
-  const long long hist = (first_frame > 0 && c->sets[0].bb.plan.mode == t2::INPUTMODE_NORMAL) ? 187 : 0;
+  const long long hist = c->history_bytes(first_frame);
   if (n_channels * P == 1 && ts_pitch < per_ch + hist) ts_pitch = per_ch + hist;      // a single row: the pitch is never used to step
   if (ts_pitch < per_ch + hist)
     return fail(DVBT2LL_ERR_INVALID, "chain: ts_pitch smaller than the TS bytes (+ 187 history bytes) of one channel");

@@ -467,7 +467,7 @@ class Chain(_Block):
     def history_bytes(self, first_frame):
         """Stream bytes that must precede the first TS byte of `first_frame` in every row handed to run_host():
         187 in normal input mode once the stream has started (CRC-8 of the packet in flight), else 0."""
-        return 187 if (first_frame > 0 and self.cfg["inputmode"] == configs.INPUTMODE_NORMAL) else 0
+        return int(lib().dvbt2ll_chain_history_bytes(self._h, int(first_frame)))
 
     def run_host(self, ts, n_channels, n_frames, first_frame=0, out=None):
         """ts: uint8 array [n_channels, history_bytes(first_frame) + >= ts_bytes(first_frame, n_frames)] (host): each row

@@ -146,6 +146,23 @@ def test_chain_generic_work_streams():
     assert np.array_equal(np.concatenate(got).view(np.uint32), want.view(np.uint32))
 
 
+def test_chain_generic_work_counts_sync_errors():
+    """dvbt2ll_work on a chain handle counts a TS packet whose first byte is not 0x47 as a warning, like the drop-in
+    block (test_ts_sync_error_is_counted), and carries the count across calls; the baseband still follows the rule."""
+    cfg = K.resolve("c1")
+    ch = T.Chain(cfg, max_frames=2)
+    n0, n_all = ch.ts_bytes(0, 1), ch.ts_bytes(0, 2)
+    ts = K.make_ts(n_all, seed=11)
+    bad = (n0 // 188 + 3) * 188                 # a packet of the second frame
+    ts[bad] = 0x00
+    want = T.Chain(cfg, max_frames=2).run_host(ts, 1, 2)[0]
+    a, used = ch.work(ts, 1)
+    assert used == n0 and ch.warnings == 0
+    b, used = ch.work(ts[n0:], 1)
+    assert used == n_all - n0 and ch.warnings == 1
+    assert np.array_equal(np.concatenate([a, b]).view(np.uint32), want.view(np.uint32))
+
+
 def test_overfull_frame_warn_policy(compiled_ref):
     """An over-full T2 frame: refused by default, reproduced like the reference (warn, truncate) with the opt-in policy."""
     cfg = K.resolve(dict(K.CONFIGS["c1"], fecblocks=9))

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """k_ldpc accumulation scheme per code (run on the GPU box): times the LDPC stage of the fused chain for every T2 code
 with a lane per (row, word) [mode 0] and a lane per row [mode 1]; the faster one per code is what
-LdpcHandle::ldpc_lane_per_row_default encodes.  Output: profiles/r2_ldpc_modes.txt"""
+LdpcStage::ldpc_lane_per_row_default encodes.  Output: profiles/r2_ldpc_modes.txt"""
 import os
 import sys
 
