@@ -7,6 +7,7 @@ import pytest
 
 import dvbt2ll_b200 as T
 from dvbt2ll_b200 import configs as K
+import test_chain_modes
 import test_miso
 import test_papr_tr
 import test_plp_modcod
@@ -27,6 +28,8 @@ CASES = [
     ("c1-3plp-inband", K.resolve(test_plp_modcod.MULTIPLP["c1-3plp-inband"]), 3 + 2 + 1),
     ("c1-mix", test_plp_modcod.resolve("c1-mix"), 2 + 2 * 2 + 1),
     ("c1-qpsk-rates", test_plp_modcod.resolve("c1-qpsk-rates"), 2 + 2 * 2 + 1),
+    ("1k-16plp-modcod", test_chain_modes.MODE_CHAINS["1k"], 16 + 16 * 2 + 1),
+    ("4k-16plp-group", test_chain_modes.GROUP16, 16 + 2 + 1),
 ]
 
 

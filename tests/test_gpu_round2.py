@@ -438,10 +438,13 @@ def test_two_devices_in_one_process(reflib):
 
 
 def test_ldpc_both_accumulation_schemes(monkeypatch):
-    """k_ldpc picks a lane per (row, word) or a lane per row by code; both must give the oracle's codewords."""
+    """k_ldpc picks a lane per (row, word) or a lane per row by code; both must give the oracle's codewords, for each of
+    the 14 codes."""
     from oracle import t2oracle as O
     rng = np.random.default_rng(12)
-    for fs, rate in ((1, K.C1_2), (1, K.C2_3), (0, K.C1_3), (0, K.C4_5)):
+    codes = [(1, r) for r in (K.C1_2, K.C3_5, K.C2_3, K.C3_4, K.C4_5, K.C5_6)] + \
+            [(0, r) for r in (K.C1_3, K.C2_5, K.C1_2, K.C3_5, K.C2_3, K.C3_4, K.C4_5, K.C5_6)]
+    for fs, rate in codes:
         p = O.fec_params(fs, rate)
         info = rng.integers(0, 2, 3 * p["nbch"], dtype=np.uint8)
         want = O.ldpc_encode(info.reshape(3, p["nbch"]), fs, rate).reshape(-1)
