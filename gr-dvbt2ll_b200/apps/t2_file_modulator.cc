@@ -8,10 +8,13 @@
 // of `batch` T2 frames per call (stream position carried by first_frame + the 187 history bytes in front of a batch).
 //
 // usage: t2_file_modulator [--config c1|c2|c3|c4] [--plp-blocks a,b,..] [--plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]]...
-//                          [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] [--miso 1|2|both [--out2 FILE2]]
+//                          [--plp-types t0,t1,..] [--plp-groups g0,g1,..] [--subslices N] [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] [--miso 1|2|both [--out2 FILE2]]
 //                          --out FILE  TS_FILE [TS_FILE ...]
 // --plp, once per PLP: its FEC blocks per T2 frame and, optionally, its own FEC type, code rate, constellation and
 // rotation (enum values of dvbt2ll_config.h; the config's where omitted).
+// --plp-types / --plp-groups / --subslices: each PLP's PLP_TYPE (0 common, 1 data type 1, 2 data type 2; default 1) and
+// PLP_GROUP_ID (default 1), in the order of the PLPs, and the sub-slices per frame of the type-2 PLPs (default 1)
+// (dvbt2ll_chain_create_plp_layout); the PLPs must be listed common, then type 1, then type 2.
 // --papr-tr: paprmode = PAPR_TR and tone-reservation PAPR reduction on the reserved carriers (dvbt2ll_chain_set_papr_tr).
 // The reserved carriers take cells away: a config whose FEC blocks no longer fit is refused as over-full; lower its
 // block count with --plp BLOCKS (c1: 7, c3: 200, c4: 119; c2 fits as it is).
@@ -63,6 +66,8 @@ int main(int argc, char **argv)
   std::vector<dvbt2ll_plp_params> plps;
   std::vector<int> plp_own;          // --plp entries that name their own parameters
   std::vector<const char *> inputs;
+  std::vector<int> plp_types, plp_groups;
+  int subslices = 0;               // 0: not given
   int frames = -1, batch = 4, sc16 = 0;
   float gain = 1.0f;
   int tr_iter = 0;
@@ -85,6 +90,11 @@ int main(int argc, char **argv)
     else if (a == "--plp-blocks" && i + 1 < argc) {
       for (char *t = std::strtok(argv[++i], ","); t; t = std::strtok(0, ",")) plp_blocks.push_back(std::atoi(t));
     }
+    else if ((a == "--plp-types" || a == "--plp-groups") && i + 1 < argc) {
+      std::vector<int> &v = a == "--plp-types" ? plp_types : plp_groups;
+      for (char *t = std::strtok(argv[++i], ","); t; t = std::strtok(0, ",")) v.push_back(std::atoi(t));
+    }
+    else if (a == "--subslices" && i + 1 < argc) subslices = std::atoi(argv[++i]);
     else if (a == "--plp" && i + 1 < argc) {
       int v[5] = { 0, -1, -1, -1, -1 };
       const int n = std::sscanf(argv[++i], "%d:%d:%d:%d:%d", &v[0], &v[1], &v[2], &v[3], &v[4]);
@@ -98,7 +108,7 @@ int main(int argc, char **argv)
   dvbt2ll_chain_params prm;
   const bool miso_ok = miso.empty() ? out2_path.empty() : (miso == "both") == !out2_path.empty() && (miso == "1" || miso == "2" || miso == "both");
   if (!named_config(cfg, &prm) || out_path.empty() || inputs.empty() || batch < 1 || (!plps.empty() && !plp_blocks.empty()) || !miso_ok) {
-    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] [--miso 1|2|both [--out2 FILE2]] --out FILE TS_FILE...\n", argv[0]);
+    std::fprintf(stderr, "usage: %s [--config c1..c4] [--plp-blocks a,b,.. | --plp BLOCKS[:FRAMESIZE:RATE:CONSTELLATION:ROTATION]...] [--plp-types t0,t1,..] [--plp-groups g0,g1,..] [--subslices N] [--frames N] [--batch B] [--sc16 GAIN] [--papr-tr ITER:VCLIP:TONEMAX] [--miso 1|2|both [--out2 FILE2]] --out FILE TS_FILE...\n", argv[0]);
     return 2;
   }
   bool own = false;
@@ -110,10 +120,31 @@ int main(int argc, char **argv)
     for (size_t p = 0; p < plps.size(); p++) plp_blocks.push_back(plps[p].fecblocks);
   const int P = own ? (int)plps.size() : plp_blocks.empty() ? 1 : (int)plp_blocks.size();
   if ((int)inputs.size() != P) { std::fprintf(stderr, "one TS file per PLP expected (%d)\n", P); return 2; }
+  const bool layout = !plp_types.empty() || !plp_groups.empty() || subslices;
+  dvbt2ll_plp_layout lay;
+  if (layout) {
+    if ((!plp_types.empty() && (int)plp_types.size() != P) || (!plp_groups.empty() && (int)plp_groups.size() != P) || P > 16) {
+      std::fprintf(stderr, "--plp-types / --plp-groups: one value per PLP expected (%d)\n", P);
+      return 2;
+    }
+    if (plps.empty()) {        // --plp-blocks or the config's single PLP, with the config's parameters
+      if (plp_blocks.empty()) plp_blocks.push_back(prm.fecblocks);
+      for (int p = 0; p < P; p++) {
+        const dvbt2ll_plp_params q = { plp_blocks[p], prm.framesize, prm.rate, prm.constellation, prm.rotation };
+        plps.push_back(q);
+      }
+    }
+    lay.num_subslices = subslices ? subslices : 1;
+    for (int p = 0; p < 16; p++) {
+      lay.type[p] = p < (int)plp_types.size() ? plp_types[p] : 1;
+      lay.group[p] = p < (int)plp_groups.size() ? plp_groups[p] : 1;
+    }
+  }
   if (P == 1 && !own && !plps.empty()) prm.fecblocks = plps[0].fecblocks;
   if (tr_iter) prm.paprmode = 2;      // PAPR_TR
   if (!miso.empty()) { prm.preamble = 1; prm.misogroup = miso == "2" ? 1 : 0; }      // PREAMBLE_T2_MISO, MISO_TX1 / TX2
-  dvbt2ll_handle *h = own ? dvbt2ll_chain_create_plps(&prm, P, plps.data(), batch, -1)
+  dvbt2ll_handle *h = layout ? dvbt2ll_chain_create_plp_layout(&prm, P, plps.data(), &lay, batch, -1)
+                    : own ? dvbt2ll_chain_create_plps(&prm, P, plps.data(), batch, -1)
                     : P == 1 ? dvbt2ll_chain_create(&prm, batch, -1) : dvbt2ll_chain_create_multiplp(&prm, P, plp_blocks.data(), batch, -1);
   if (!h) { std::fprintf(stderr, "chain: %s\n", dvbt2ll_last_error()); return 1; }
   if (sc16 && dvbt2ll_chain_set_sink(h, 1, gain) < 0) { std::fprintf(stderr, "%s\n", dvbt2ll_last_error()); return 1; }

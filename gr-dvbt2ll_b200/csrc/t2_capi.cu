@@ -1221,8 +1221,15 @@ struct ChainHandle : dvbt2ll_handle {
     if (n == "frame.plp_cells") {
       // per PLP: cells per FECFRAME, first cell in the frame (PLP_START), first cell in the chain's cell memory
       int v[3 * t2::MAX_PLP];
-      for (int i = 0; i < P(); i++) { v[3 * i] = fplan.plp_cell_size[i]; v[3 * i + 1] = fplan.plp_first_cell[i]; v[3 * i + 2] = fplan.plp_chain_off[i]; }
+      for (int i = 0; i < P(); i++) { v[3 * i] = fplan.plp_cell_size[i]; v[3 * i + 1] = fplan.plp_start[i]; v[3 * i + 2] = fplan.plp_chain_off[i]; }
       return copy_out(v, sizeof(int) * 3 * P(), out, cap);
+    }
+    if (n == "frame.plp_layout") {
+      // per PLP: PLP_TYPE, PLP_GROUP_ID, cells per sub-slice; then SUB_SLICES_PER_FRAME, SUB_SLICE_INTERVAL, TYPE_2_START
+      int v[3 * t2::MAX_PLP + 3];
+      for (int i = 0; i < P(); i++) { v[3 * i] = fplan.plp_type[i]; v[3 * i + 1] = fplan.plp_group[i]; v[3 * i + 2] = fplan.plp_slice_cells[i]; }
+      v[3 * P()] = fplan.num_subslices; v[3 * P() + 1] = fplan.subslice_interval; v[3 * P() + 2] = fplan.type2_start;
+      return copy_out(v, sizeof(int) * (3 * P() + 3), out, cap);
     }
     if (n == "chain.luts") {
       // constellation tables of the OFDM fill: { tables, single-table form, copies in shared memory in the last run
@@ -1600,10 +1607,11 @@ dvbt2ll_handle *dvbt2ll_pilotgenp1insert_create(int carriermode, int fftsize, in
   return h;
 }
 
-// own_modcod: every PLP has its own framesize / rate / constellation / rotation (dvbt2ll_chain_create_plps); otherwise
-// they are the chain's, and an over-full frame follows the over-full policy like the reference's frame mapper
+// own_modcod: every PLP has its own framesize / rate / constellation / rotation (dvbt2ll_chain_create_plp_layout);
+// otherwise they are the chain's, and an over-full frame follows the over-full policy like the reference's frame mapper.
+// layout: PLP types, groups and sub-slices (NULL: type-1 PLPs of group 1, one sub-slice)
 static dvbt2ll_handle *chain_create(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, bool own_modcod,
-                                    int max_frames, int device)
+                                    const dvbt2ll_plp_layout *layout, int max_frames, int device)
 {
   std::unique_ptr<ChainHandle> h(new ChainHandle());
   std::string err;
@@ -1621,6 +1629,11 @@ static dvbt2ll_handle *chain_create(const dvbt2ll_chain_params *c, int num_plp, 
     fp.plp_fecblocks[p] = plp[p].fecblocks;
     fp.plp_framesize[p] = plp[p].framesize; fp.plp_rate[p] = plp[p].rate;
     fp.plp_constellation[p] = plp[p].constellation; fp.plp_rotation[p] = plp[p].rotation;
+  }
+  if (layout) {
+    fp.plp_layout = 1;
+    fp.num_subslices = layout->num_subslices;
+    for (int p = 0; p < num_plp; p++) { fp.plp_type[p] = layout->type[p]; fp.plp_group[p] = layout->group[p]; }
   }
   t2::OfdmParams op = { c->carriermode, c->fftsize, c->pilotpattern, c->guardinterval, c->numdatasyms, c->paprmode,
                         c->version, c->preamble, c->misogroup, c->equalization, c->bandwidth, c->vlength };
@@ -1663,14 +1676,23 @@ static dvbt2ll_handle *chain_create(const dvbt2ll_chain_params *c, int num_plp, 
   return h.release();
 }
 
-dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, int max_frames,
-                                          int device)
+dvbt2ll_handle *dvbt2ll_chain_create_plp_layout(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp,
+                                                const dvbt2ll_plp_layout *layout, int max_frames, int device)
 {
-  if (!c || !plp || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
+  if (!c || !plp || !layout || max_frames < 1) { fail(DVBT2LL_ERR_INVALID, "chain: bad arguments"); return 0; }
   if (num_plp < 1 || num_plp > t2::MAX_PLP) { fail(DVBT2LL_ERR_INVALID, "chain: number of PLPs out of range"); return 0; }
   for (int p = 0; p < num_plp; p++)
     if (plp[p].fecblocks < 1 || plp[p].fecblocks > 1023) { fail(DVBT2LL_ERR_INVALID, "chain: FEC blocks of a PLP out of range"); return 0; }
-  return chain_create(c, num_plp, plp, true, max_frames, device);
+  return chain_create(c, num_plp, plp, true, layout, max_frames, device);
+}
+
+dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *c, int num_plp, const dvbt2ll_plp_params *plp, int max_frames,
+                                          int device)
+{
+  dvbt2ll_plp_layout layout;
+  layout.num_subslices = 1;
+  for (int p = 0; p < t2::MAX_PLP; p++) { layout.type[p] = 1; layout.group[p] = 1; }
+  return dvbt2ll_chain_create_plp_layout(c, num_plp, plp, &layout, max_frames, device);
 }
 
 dvbt2ll_handle *dvbt2ll_chain_create_multiplp(const dvbt2ll_chain_params *c, int num_plp, const int *plp_fecblocks, int max_frames, int device)
@@ -1682,7 +1704,7 @@ dvbt2ll_handle *dvbt2ll_chain_create_multiplp(const dvbt2ll_chain_params *c, int
     const dvbt2ll_plp_params q = { num_plp > 1 ? plp_fecblocks[p] : c->fecblocks, c->framesize, c->rate, c->constellation, c->rotation };
     plp[p] = q;
   }
-  return chain_create(c, num_plp, plp, false, max_frames, device);
+  return chain_create(c, num_plp, plp, false, 0, max_frames, device);
 }
 
 dvbt2ll_handle *dvbt2ll_chain_create(const dvbt2ll_chain_params *c, int max_frames, int device)

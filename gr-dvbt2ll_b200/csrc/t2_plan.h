@@ -163,6 +163,15 @@ struct FrameParams {
   // PLPs do not fit is then always refused (there is no reference behaviour to reproduce).
   int plp_modcod;
   int plp_framesize[MAX_PLP], plp_rate[MAX_PLP], plp_constellation[MAX_PLP], plp_rotation[MAX_PLP];
+  // plp_layout = 1: PLP p has the L1-post PLP_TYPE plp_type[p] (0 common, 1 data type 1, 2 data type 2) and PLP_GROUP_ID
+  // plp_group[p], and the type-2 PLPs are split into num_subslices sub-slices; otherwise every PLP is a type-1 data PLP of
+  // group 1 and the frame has one sub-slice.  The PLPs are listed in mapping order: common, then type 1, then type 2.
+  // Common and type-1 PLPs each take one block of cells from data-cell address 0 on; TYPE_2_START is the cells they take.
+  // Type-2 PLP i with D_i cells per frame has sub-slices of L_i = D_i / N cells, SUB_SLICE_INTERVAL = sum_i L_i, and its
+  // cell k (time-interleaver output order) goes to address PLP_START_i + (k div L_i) SUB_SLICE_INTERVAL + k mod L_i,
+  // PLP_START_i = TYPE_2_START + sum_{j < i} L_j.
+  int plp_layout;
+  int plp_type[MAX_PLP], plp_group[MAX_PLP], num_subslices;
 };
 struct FramePlan {
   FrameParams prm;
@@ -173,7 +182,12 @@ struct FramePlan {
   int num_plp;                         // >= 1
   int plp_first_block[MAX_PLP + 1];    // first FEC block of each PLP inside the T2 frame's block list
   int plp_cell_size[MAX_PLP];          // cells per FECFRAME of each PLP
-  int plp_first_cell[MAX_PLP + 1];     // first cell of each PLP in the frame's data cells (L1-post PLP_START)
+  int plp_first_cell[MAX_PLP + 1];     // first cell of each PLP in the time-interleaved stream (PLP after PLP)
+  // L1-post layout (FrameParams::plp_layout): PLP_TYPE, PLP_GROUP_ID, PLP_START (data-cell address of the PLP's first cell;
+  // plp_first_cell except for type-2 PLPs), cells per sub-slice (the PLP's cells per frame unless type 2), and
+  // SUB_SLICES_PER_FRAME, SUB_SLICE_INTERVAL, TYPE_2_START
+  int plp_type[MAX_PLP], plp_group[MAX_PLP], plp_start[MAX_PLP], plp_slice_cells[MAX_PLP];
+  int num_subslices, subslice_interval, type2_start;
   // Chain mode: PLP p's 16-bit cells start at plp_chain_off[p] of the frame's cell memory.  PLPs of one parameter set
   // follow each other (plp_chain_off = plp_first_cell); with more than one set (plp_sets > 1, one mapper launch per
   // PLP) every PLP starts on an 8-cell (16-byte) boundary.  plp_chain_off[num_plp] = cells of a frame in that memory.

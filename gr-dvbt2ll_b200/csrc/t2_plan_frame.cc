@@ -205,7 +205,7 @@ void build_l1pre(const FrameParams &prm, int l1_post_size, int l1_post_info_size
 }
 
 // what L1-post signals of one PLP
-struct PlpL1 { int blocks, cell_size, framesize, rate, constellation, rotation; };
+struct PlpL1 { int blocks, cell_size, framesize, rate, constellation, rotation, type, group, start; };
 
 int plp_cod_of(int rate)
 {
@@ -216,13 +216,13 @@ int plp_cod_of(int rate)
   return 0;
 }
 
-void build_l1post(const FrameParams &prm, const PlpL1 *plps, int num_plp, int frame_idx, int n_post, int n_punc,
-                  int eta, std::vector<cfloat> &cells)
+void build_l1post(const FrameParams &prm, const PlpL1 *plps, int num_plp, int subslices, int subslice_interval,
+                  int type2_start, int frame_idx, int n_post, int n_punc, int eta, std::vector<cfloat> &cells)
 {
   const bool v131 = prm.version == VERSION_131;
   const bool bias = prm.reservedbiasbits && v131;
   BitWriter w;
-  w.put(1, 15);                                  // SUB_SLICES_PER_FRAME
+  w.put(subslices, 15);                          // SUB_SLICES_PER_FRAME
   w.put(num_plp, 8);                             // NUM_PLP
   w.put(0, 4);                                   // NUM_AUX
   w.put(0, 8);                                   // AUX_CONFIG_RFU
@@ -230,12 +230,12 @@ void build_l1post(const FrameParams &prm, const PlpL1 *plps, int num_plp, int fr
   w.put(729833333u, 32);                         // FREQUENCY
   for (int pl = 0; pl < num_plp; pl++) {         // configurable part, 89 bits per PLP
     w.put(pl, 8);                                // PLP_ID
-    w.put(1, 3);                                 // PLP_TYPE (data type 1)
+    w.put(plps[pl].type, 3);                     // PLP_TYPE
     w.put(3, 5);                                 // PLP_PAYLOAD_TYPE (TS)
     w.put(0, 1);                                 // FF_FLAG
     w.put(0, 3);                                 // FIRST_RF_IDX
     w.put(0, 8);                                 // FIRST_FRAME_IDX
-    w.put(1, 8);                                 // PLP_GROUP_ID
+    w.put(plps[pl].group, 8);                    // PLP_GROUP_ID
     w.put(plp_cod_of(plps[pl].rate), 3);         // PLP_COD
     w.put(plps[pl].constellation, 3);            // PLP_MOD
     w.put(plps[pl].rotation, 1);                 // PLP_ROTATION
@@ -254,20 +254,16 @@ void build_l1post(const FrameParams &prm, const PlpL1 *plps, int num_plp, int fr
   w.put(0, 2);                                   // FEF_LENGTH_MSB
   w.put(bias ? 0x3fffffff : 0, 30);              // RESERVED_2
   w.put(frame_idx, 8);                           // FRAME_IDX (dynamic)
-  w.put(0, 22);                                  // SUB_SLICE_INTERVAL
-  w.put(0, 22);                                  // TYPE_2_START
+  w.put(subslice_interval, 22);                  // SUB_SLICE_INTERVAL
+  w.put(type2_start, 22);                        // TYPE_2_START
   w.put(0, 8);                                   // L1_CHANGE_COUNTER
   w.put(0, 3);                                   // START_RF_IDX
   w.put(bias ? 0xff : 0, 8);                     // RESERVED_3
-  {
-    int start = 0;                               // type-1 PLPs follow each other from cell address 0 of the frame's data
-    for (int pl = 0; pl < num_plp; pl++) {       // dynamic part, 48 bits per PLP
-      w.put(pl, 8);                              // PLP_ID (dynamic; the reference leaves its single one uninitialised = 0)
-      w.put(start, 22);                          // PLP_START
-      w.put(plps[pl].blocks, 10);                // PLP_NUM_BLOCKS
-      w.put(bias ? 0xff : 0, 8);                 // RESERVED_4
-      start += plps[pl].blocks * plps[pl].cell_size;
-    }
+  for (int pl = 0; pl < num_plp; pl++) {         // dynamic part, 48 bits per PLP
+    w.put(pl, 8);                                // PLP_ID (dynamic; the reference leaves its single one uninitialised = 0)
+    w.put(plps[pl].start, 22);                   // PLP_START
+    w.put(plps[pl].blocks, 10);                  // PLP_NUM_BLOCKS
+    w.put(bias ? 0xff : 0, 8);                   // RESERVED_4
   }
   w.put(bias ? 0xff : 0, 8);                     // RESERVED_5
   append_crc32(w.b);                             // K_sig = 213 + 137 num_plp bits (350 for one PLP)
@@ -339,6 +335,58 @@ void build_l1post(const FrameParams &prm, const PlpL1 *plps, int num_plp, int fr
     cells.push_back(lut[pack >> eta]);
     cells.push_back(lut[pack & ((1u << eta) - 1)]);
   }
+}
+
+// PLP types, groups and sub-slicing (FrameParams::plp_layout): validates them and fills the plan's layout fields and each
+// PLP's type, group and PLP_START.  Without plp_layout: type-1 PLPs of group 1, one sub-slice, PLP_START = first cell.
+bool plp_layout(const FrameParams &prm, int P, FramePlan *p, PlpL1 *plps, std::string *err)
+{
+  auto refuse = [&](int pl, const char *why) {
+    if (err) *err = "framemapperfint_cc: PLP " + std::to_string(pl) + ": " + why;
+    return false;
+  };
+  const int N = prm.plp_layout ? prm.num_subslices : 1;
+  if (N < 1 || N > 32767) {
+    if (err) *err = "framemapperfint_cc: sub-slices per frame outside 1..32767";
+    return false;
+  }
+  bool type2 = false;
+  for (int pl = 0; pl < P; pl++) {
+    const int t = prm.plp_layout ? prm.plp_type[pl] : 1, g = prm.plp_layout ? prm.plp_group[pl] : 1;
+    if (t < 0 || t > 2) return refuse(pl, "PLP_TYPE outside 0..2 (common, data type 1, data type 2)");
+    if (pl > 0 && t < p->plp_type[pl - 1]) return refuse(pl, "listed out of mapping order (common, then type-1, then type-2 PLPs)");
+    if (g < 0 || g > 255) return refuse(pl, "PLP_GROUP_ID outside 0..255");
+    const int D = plps[pl].blocks * plps[pl].cell_size;
+    if (t == 2 && D % N) return refuse(pl, "type-2 cells per frame are not a multiple of the sub-slices per frame");
+    p->plp_type[pl] = plps[pl].type = t;
+    p->plp_group[pl] = plps[pl].group = g;
+    p->plp_slice_cells[pl] = t == 2 ? D / N : D;
+    type2 = type2 || t == 2;
+  }
+  if (N > 1 && !type2) {
+    if (err) *err = "framemapperfint_cc: more than one sub-slice per frame without a type-2 PLP";
+    return false;
+  }
+  for (int pl = 0; pl < P; pl++) {
+    if (p->plp_type[pl] != 0) continue;
+    int data = 0;
+    for (int o = 0; o < P; o++) {
+      if (o != pl && p->plp_group[o] == p->plp_group[pl] && p->plp_type[o] == 0) return refuse(pl, "common PLP of a group with another common PLP");
+      if (p->plp_group[o] == p->plp_group[pl] && p->plp_type[o] != 0) data++;
+    }
+    if (!data) return refuse(pl, "common PLP of a group without a data PLP");
+  }
+  // common and type-1 PLPs one after the other from address 0, then the type-2 PLPs' sub-slices
+  p->num_subslices = N;
+  p->type2_start = p->subslice_interval = 0;
+  int start = 0;
+  for (int pl = 0; pl < P; pl++) {
+    if (p->plp_type[pl] == 2 && (pl == 0 || p->plp_type[pl - 1] != 2)) p->type2_start = start;
+    p->plp_start[pl] = plps[pl].start = start;
+    start += p->plp_slice_cells[pl];
+    if (p->plp_type[pl] == 2) p->subslice_interval += p->plp_slice_cells[pl];
+  }
+  return true;
 }
 
 // frequency interleaver permutation function H (EN 302 755 8.5; reference :916-977)
@@ -418,6 +466,7 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
     p->plp_set[pl] = s < pl ? p->plp_set[s] : p->plp_sets++;
   }
   if (p->plp_first_block[P] != prm.fecblocks) { if (err) *err = "framemapperfint_cc: fecblocks is not the sum over the PLPs"; return false; }
+  if (!plp_layout(prm, P, p, plps, err)) return false;
   p->plp_chain_off[0] = 0;
   for (int pl = 0; pl < P; pl++) {
     const int end = p->plp_chain_off[pl] + plp_blocks[pl] * plps[pl].cell_size;
@@ -448,7 +497,7 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
   // own parameters have no reference behaviour to reproduce: such a frame is always refused.
   int linear_items = p->mapped_items;
   if (p->overfull) {
-    if (!overfull_warn_policy() || prm.plp_modcod) {
+    if (!overfull_warn_policy() || prm.plp_modcod || prm.plp_layout) {
       if (err) *err = "Frame Mapper, too many FEC blocks in T2 frame.";
       return false;
     }
@@ -567,7 +616,7 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
   pool.l1post_variants = prm.t2frames;
   for (int v = 0; v < prm.t2frames; v++) {
     std::vector<cfloat> c;
-    build_l1post(prm, plps, P, v, p->n_post, p->n_punc, eta, c);
+    build_l1post(prm, plps, P, p->num_subslices, p->subslice_interval, p->type2_start, v, p->n_post, p->n_punc, eta, c);
     if ((int)c.size() != l1post_cells) { if (err) *err = "internal: L1-post size"; return false; }
     pool.cells.insert(pool.cells.end(), c.begin(), c.end());
   }
@@ -586,7 +635,13 @@ bool build_frame_plan(const FrameParams &prm, FramePlan *p, std::string *err)
     size_t k = 0;
     for (int i = 0; i < 1840; i++) linear[k++] = -(1 + p->pool_l1pre + i);
     for (int i = 0; i < l1post_cells; i++) linear[k++] = -(1 + pool.l1post_base + i);
-    for (int i = 0; i < p->stream_items; i++) linear[k++] = p->ti_src[i];
+    // data cells in mapping order: each PLP's time-interleaver output at its data-cell addresses (FrameParams::plp_layout)
+    for (int pl = 0; pl < P; pl++) {
+      const int L = p->plp_slice_cells[pl], step = p->plp_type[pl] == 2 ? p->subslice_interval : L;
+      for (int i = 0; i < p->plp_first_cell[pl + 1] - p->plp_first_cell[pl]; i++)
+        linear[k + p->plp_start[pl] + (size_t)(i / L) * step + i % L] = p->ti_src[(size_t)p->plp_first_cell[pl] + i];
+    }
+    k += (size_t)p->stream_items;
     for (int i = 0; i < p->dummy_cells; i++) linear[k++] = -(1 + p->pool_dummy + i);
     for (int i = 0; i < d.n_fc - d.c_fc; i++) linear[k++] = -(1 + p->pool_zero);
   }

@@ -40,6 +40,7 @@ EXPORTED_SYMBOLS = [
     "dvbt2ll_chain_create_multiplp", "dvbt2ll_chain_num_plp", "dvbt2ll_chain_plp_ts_bytes",
     "dvbt2ll_chain_history_bytes", "dvbt2ll_ts_sync", "dvbt2ll_ts_fill", "dvbt2ll_chain_create_plps",
     "dvbt2ll_chain_set_papr_tr", "dvbt2ll_chain_set_miso", "dvbt2ll_chain_run_device_miso", "dvbt2ll_chain_run_host_miso",
+    "dvbt2ll_chain_create_plp_layout",
 ]
 GATHER_BLOB_BYTES = 256
 
@@ -56,12 +57,33 @@ class PlpParams(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("fecblocks", "framesize", "rate", "constellation", "rotation")]
 
 
+class PlpLayout(C.Structure):
+    _fields_ = [("num_subslices", C.c_int), ("type", C.c_int * 16), ("group", C.c_int * 16)]
+
+
 PLP_KEYS = ("framesize", "rate", "constellation", "rotation")
+LAYOUT_KEYS = ("type", "group")
 
 
 def plp_params(cfg):
     """cfg["plps"] with every PLP's missing framesize / rate / constellation / rotation taken from the cfg."""
-    return [dict({k: int(cfg[k]) for k in PLP_KEYS}, **{k: int(v) for k, v in p.items()}) for p in cfg["plps"]]
+    return [dict({k: int(cfg[k]) for k in PLP_KEYS}, **{k: int(v) for k, v in p.items() if k not in LAYOUT_KEYS})
+            for p in cfg["plps"]]
+
+
+def plp_layout(cfg):
+    """The PLP types, groups and sub-slices of cfg, or None when neither cfg["plps"] entries name a "type" or "group"
+    nor cfg names "subslices": PLP_TYPE (default 1, data type 1), PLP_GROUP_ID (default 1), SUB_SLICES_PER_FRAME
+    (default 1)."""
+    plps = cfg.get("plps") or []
+    if "subslices" not in cfg and not any(k in p for p in plps for k in LAYOUT_KEYS):
+        return None
+    if not plps:
+        raise ValueError('cfg["subslices"] needs the PLPs listed in cfg["plps"]')
+    lay = PlpLayout(num_subslices=int(cfg.get("subslices", 1)))
+    for i, p in enumerate(plps[:16]):
+        lay.type[i], lay.group[i] = int(p.get("type", 1)), int(p.get("group", 1))
+    return lay
 
 
 def lib():
@@ -152,6 +174,9 @@ def lib():
         L.dvbt2ll_chain_num_plp.argtypes = [vp]
         L.dvbt2ll_chain_create_plps.restype = vp
         L.dvbt2ll_chain_create_plps.argtypes = [C.POINTER(ChainParams), ci, C.POINTER(PlpParams), ci, ci]
+        L.dvbt2ll_chain_create_plp_layout.restype = vp
+        L.dvbt2ll_chain_create_plp_layout.argtypes = [C.POINTER(ChainParams), ci, C.POINTER(PlpParams), C.POINTER(PlpLayout),
+                                                      ci, ci]
         L.dvbt2ll_chain_plp_ts_bytes.restype = cll
         L.dvbt2ll_chain_plp_ts_bytes.argtypes = [vp, ci, cll, ci]
         L.dvbt2ll_chain_history_bytes.restype = cll
@@ -402,7 +427,12 @@ class Chain(_Block):
         self.cfg = cfg
         p = ChainParams(**{n: int(cfg[n]) for n, _ in ChainParams._fields_})
         plps = cfg.get("plp_fecblocks")
-        if cfg.get("plps"):                 # PLPs with their own FEC type, code rate, constellation and rotation
+        layout = plp_layout(cfg)
+        if layout is not None:              # PLP types, groups and sub-slices (and each PLP's own parameters)
+            pp = plp_params(cfg)
+            arr = (PlpParams * len(pp))(*[PlpParams(**q) for q in pp])
+            h = lib().dvbt2ll_chain_create_plp_layout(C.byref(p), len(pp), arr, C.byref(layout), int(max_frames), int(device))
+        elif cfg.get("plps"):               # PLPs with their own FEC type, code rate, constellation and rotation
             pp = plp_params(cfg)
             arr = (PlpParams * len(pp))(*[PlpParams(**q) for q in pp])
             h = lib().dvbt2ll_chain_create_plps(C.byref(p), len(pp), arr, int(max_frames), int(device))
@@ -417,6 +447,17 @@ class Chain(_Block):
     @property
     def num_plp(self):
         return int(lib().dvbt2ll_chain_num_plp(self._h))
+
+    @property
+    def plp_layout(self):
+        """The frame's PLP layout as L1-post signals it: per PLP "type" (PLP_TYPE), "group" (PLP_GROUP_ID), "start"
+        (PLP_START) and "slice_cells" (cells per sub-slice; the PLP's cells per frame unless type 2), and "subslices"
+        (SUB_SLICES_PER_FRAME), "subslice_interval" (SUB_SLICE_INTERVAL), "type2_start" (TYPE_2_START)."""
+        P = self.num_plp
+        v = [int(x) for x in self.plan("frame.plp_layout", np.int32)]
+        start = [int(x) for x in self.plan("frame.plp_cells", np.int32).reshape(P, 3)[:, 1]]
+        return dict(type=v[0:3 * P:3], group=v[1:3 * P:3], slice_cells=v[2:3 * P:3], start=start, subslices=v[3 * P],
+                    subslice_interval=v[3 * P + 1], type2_start=v[3 * P + 2])
 
     def plp_ts_bytes(self, plp, first_frame, n_frames):
         """TS bytes PLP `plp` of one channel consumes for T2 frames [first_frame, first_frame + n_frames)."""

@@ -125,6 +125,31 @@ typedef struct dvbt2ll_plp_params {
 } dvbt2ll_plp_params;
 DVBT2LL_API_EXPORT dvbt2ll_handle *dvbt2ll_chain_create_plps(const dvbt2ll_chain_params *p, int num_plp,
                                                              const dvbt2ll_plp_params *plp, int max_frames, int device);
+/* PLP types, groups and sub-slicing (EN 302 755 7.2.3.1 PLP_TYPE / PLP_GROUP_ID, 8.3.6.3; beyond the reference, whose
+ * single PLP is a type-1 data PLP).  As dvbt2ll_chain_create_plps, plus per PLP i the L1-post PLP_TYPE type[i] (0 =
+ * common, 1 = data type 1, 2 = data type 2) and PLP_GROUP_ID group[i] (0..255), and num_subslices = N (1..32767), the
+ * SUB_SLICES_PER_FRAME of the frame's type-2 PLPs.  The PLPs are listed in mapping order -- common PLPs, then type-1, then
+ * type-2 -- and PLP_ID is the list index.  In the frame's data cells (L1-post PLP_START addresses):
+ *   - common and type-1 PLPs each take one block of their D_i = PLP_NUM_BLOCKS x N_cells cells, one after the other
+ *     from address 0; TYPE_2_START is the sum of their cells (0 without type-2 PLPs);
+ *   - type-2 PLP i has sub-slices of L_i = D_i / N cells, SUB_SLICE_INTERVAL = sum of L_i over the type-2 PLPs, and
+ *     cell k of its time-interleaver output goes to PLP_START_i + (k div L_i) SUB_SLICE_INTERVAL + k mod L_i, with
+ *     PLP_START_i = TYPE_2_START + sum of L_j over the type-2 PLPs j before it;
+ *   - dummy cells and the frame-closing symbol's unmodulated cells follow the last data cell.
+ * BB framing, FEC, cell and time interleaving, FEC groups, taps and TS rows (channel * num_plp + plp) are those of
+ * dvbt2ll_chain_create_plps, which is this call with every type 1, every group 1 and N = 1.  Refused, naming the PLP: a
+ * type outside 0..2; PLPs out of mapping order; N outside 1..32767; N > 1 without a type-2 PLP; a type-2 PLP whose D_i is
+ * not a multiple of N; a group outside 0..255; two common PLPs in one group; a common PLP whose group has no data PLP.
+ * dvbt2ll_plan_get "frame.plp_layout": int32 per PLP { type, group, cells per sub-slice (D_i unless type 2) }, then N,
+ * SUB_SLICE_INTERVAL, TYPE_2_START; "frame.plp_cells" column 1 is each PLP's PLP_START. */
+typedef struct dvbt2ll_plp_layout {
+  int num_subslices;
+  int type[16], group[16];
+} dvbt2ll_plp_layout;
+DVBT2LL_API_EXPORT dvbt2ll_handle *dvbt2ll_chain_create_plp_layout(const dvbt2ll_chain_params *p, int num_plp,
+                                                                   const dvbt2ll_plp_params *plp,
+                                                                   const dvbt2ll_plp_layout *layout, int max_frames,
+                                                                   int device);
 DVBT2LL_API_EXPORT int dvbt2ll_chain_num_plp(const dvbt2ll_handle *h);
 /* Stream bytes that must precede the first TS byte of first_frame in every row handed to dvbt2ll_chain_run_*:
  * 187 in normal input mode once the stream has started (CRC-8 of the packet in flight), else 0. */
